@@ -32,6 +32,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 KERNEL = "rbf+stdperiodic"
 B_PER_GPU = 4096
@@ -274,6 +275,8 @@ def run_ours(args):
     var_ms, var_n = ctx.profile_read(L.PROF_VAR)
     ctx.set_profiling(False)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_dev)
 
     # ---- e2e: public API, pinned host buffers, copies inside the timed region ----
     hx, hy = torch.from_numpy(x).pin_memory(), torch.from_numpy(y).pin_memory()
@@ -390,6 +393,15 @@ def run_ours(args):
     return 0
 
 
+def dump_outputs(path, out_dev):
+    """What the last timed step returned to its caller - predictive mean and variance [B, M], LML [B] and status [B] of
+    rank 0's windows - as float64 .npy files (8 * (2 * B * M + 2 * B) bytes), so that two builds can be compared output
+    for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in zip(("mean", "var", "lml", "status"), out_dev):
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+
 def run_extra(ctx, torch, rank, world, dev_in, out_dev):
     """Numbers for the configs the headline does not carry, so that the driver's records hold them (every rank takes
     part: configs[3] is sharded over the ranks, configs[4] is factored block-cyclically over them):
@@ -477,7 +489,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "cpu_probe"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra.configs legs (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64; --impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "cpu_probe":      # bounded CPU-port sample for the cpu_baseline object of our arm
