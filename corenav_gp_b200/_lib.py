@@ -74,6 +74,16 @@ SIGNATURES = {
                                           c_dp, c_ip, c_i32]),
     "cngp_gp_slip_batch": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_i64, c_dp, c_dp, c_i64, c_i32, c_i32, c_i32,
                                      c_dp, c_dp, c_ip, c_ip]),
+    "cngp_predict_ragged": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_i64, c_dp, c_dp, c_ip, c_i32, c_dp, c_ip, c_i32,
+                                      c_i64, c_dp, c_dp, c_dp, c_ip, c_i32]),
+    "cngp_lml_grad_ragged": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_i64, c_dp, c_dp, c_ip, c_i32, c_i64, c_dp, c_dp,
+                                       c_ip, c_i32]),
+    "cngp_optimize_ragged": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_i64, c_dp, c_dp, c_ip, c_i32, c_i64, c_i32, c_dp,
+                                       c_dp, c_ip, c_i32]),
+    "cngp_gp_slip_ragged": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_i64, c_dp, c_dp, c_ip, c_i32, c_i64, c_i32, c_i32,
+                                      c_dp, c_dp, c_ip, c_ip, c_i32]),
+    "cngp_zupt_lookahead_ragged": (C.c_int, [c_vp, c_dp, c_dp, c_i64, c_ip, c_i32, c_dp, c_dp, c_dp, c_dp, c_dp, c_i32,
+                                             C.POINTER(StopConfig), c_ip, c_ip, c_ip, c_dp, c_dp, c_dp, c_dp, c_i32]),
     "cngp_default_stop_config": (None, [C.POINTER(StopConfig)]),
     "cngp_zupt_lookahead_batch": (C.c_int, [c_vp, c_dp, c_dp, c_i64, c_i32, c_dp, c_dp, c_dp, c_dp, c_dp, c_i32,
                                             C.POINTER(StopConfig), c_ip, c_ip, c_ip, c_dp, c_i32]),

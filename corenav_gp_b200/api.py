@@ -259,6 +259,106 @@ class GpContext:
             return mean, sigma, status
         return mean[:, :m].copy(), sigma[:, :m].copy(), status
 
+    # ---- ragged windows: window b has n[b] valid entries in its row of x / y, m[b] in its row of xstar / outputs ----
+    def _ragged_common(self, kernel, x, n):
+        k = parse_kernel(kernel)
+        dev = _is_cuda(x)
+        B, ld = (int(v) for v in tuple(x.shape))
+        if int(np.prod(tuple(n.shape))) != B:
+            raise CngpError(f"n has {int(np.prod(tuple(n.shape)))} entries for {B} windows")
+        return k, dev, B, ld, k.n_params + 1
+
+    @staticmethod
+    def _theta_stride(theta, P):
+        shape = tuple(theta.shape)
+        if shape[-1] != P:
+            raise CngpError(f"theta has {shape[-1]} entries, kernel needs {P} (noise last)")
+        return 0 if len(shape) == 1 else P
+
+    def predict_ragged(self, kernel, theta, x, y, n, xstar, m):
+        """predict() for windows of different sizes: x, y [B,ld] with n[b] valid entries in row b; xstar [B,ldm] with
+        m[b] valid test points.  theta [P] or [B,P].  Returns (mean [B,ldm], var [B,ldm], lml [B], status [B]) on the
+        device of the inputs; entries of mean / var beyond m[b] (and lml of windows with n[b] = 0) are left as allocated."""
+        k, dev, B, ld, P = self._ragged_common(kernel, x, n)
+        stride = self._theta_stride(theta, P)
+        ldm = int(tuple(xstar.shape)[-1])
+        mean = self._empty((B, ldm), np.float64, dev)
+        var = self._empty((B, ldm), np.float64, dev)
+        lml = self._empty((B,), np.float64, dev)
+        status = self._empty((B,), np.int32, dev)
+        a = [_Arg(theta, np.float64, dev), _Arg(x, np.float64, dev), _Arg(y, np.float64, dev), _Arg(n, np.int32, dev),
+             _Arg(xstar, np.float64, dev), _Arg(m, np.int32, dev), _Arg(mean, np.float64, dev, output=True),
+             _Arg(var, np.float64, dev, output=True), _Arg(lml, np.float64, dev, output=True),
+             _Arg(status, np.int32, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_predict_ragged(self.h, C.byref(k), a[0].ptr, stride, a[1].ptr, a[2].ptr, a[3].ptr, ld,
+                                          a[4].ptr, a[5].ptr, ldm, B, a[6].ptr, a[7].ptr, a[8].ptr, a[9].ptr,
+                                          L.MEM_DEVICE if dev else L.MEM_HOST)
+        self._check(rc, "cngp_predict_ragged")
+        return mean, var, lml, status
+
+    def lml_grad_ragged(self, kernel, theta, x, y, n, want_grad: bool = True):
+        """lml_grad() for windows of different sizes: theta [C,P]; x, y [B,ld] with n[b] valid entries.
+        Returns lml [C,B], grad [C,B,P] (or None), status [C,B]."""
+        k, dev, B, ld, P = self._ragged_common(kernel, x, n)
+        Cn = int(tuple(theta.shape)[0])
+        if tuple(theta.shape)[-1] != P:
+            raise CngpError(f"theta has {tuple(theta.shape)[-1]} entries, kernel needs {P} (noise last)")
+        lml = self._empty((Cn, B), np.float64, dev)
+        grad = self._empty((Cn, B, P), np.float64, dev) if want_grad else None
+        status = self._empty((Cn, B), np.int32, dev)
+        a = [_Arg(theta, np.float64, dev), _Arg(x, np.float64, dev), _Arg(y, np.float64, dev), _Arg(n, np.int32, dev),
+             _Arg(lml, np.float64, dev, output=True), _Arg(grad, np.float64, dev, True, output=True),
+             _Arg(status, np.int32, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_lml_grad_ragged(self.h, C.byref(k), a[0].ptr, Cn, a[1].ptr, a[2].ptr, a[3].ptr, ld, B,
+                                           a[4].ptr, a[5].ptr, a[6].ptr, L.MEM_DEVICE if dev else L.MEM_HOST)
+        self._check(rc, "cngp_lml_grad_ragged")
+        return lml, grad, status
+
+    def optimize_ragged(self, kernel, x, y, n, theta0=None, max_iters: int = 1000):
+        """optimize() for windows of different sizes: x, y [B,ld] with n[b] valid entries.  theta0 None (all ones),
+        [P] or [B,P].  Returns (theta [B,P], lml [B], iters [B]) on the device of the inputs."""
+        k, dev, B, ld, P = self._ragged_common(kernel, x, n)
+        stride = 0 if theta0 is None else self._theta_stride(theta0, P)
+        theta = self._empty((B, P), np.float64, dev)
+        lml = self._empty((B,), np.float64, dev)
+        iters = self._empty((B,), np.int32, dev)
+        a = [_Arg(theta0, np.float64, dev, True), _Arg(x, np.float64, dev), _Arg(y, np.float64, dev),
+             _Arg(n, np.int32, dev), _Arg(theta, np.float64, dev, output=True), _Arg(lml, np.float64, dev, output=True),
+             _Arg(iters, np.int32, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_optimize_ragged(self.h, C.byref(k), a[0].ptr, stride, a[1].ptr, a[2].ptr, a[3].ptr, ld, B,
+                                           max_iters, a[4].ptr, a[5].ptr, a[6].ptr, L.MEM_DEVICE if dev else L.MEM_HOST)
+        self._check(rc, "cngp_optimize_ragged")
+        return theta, lml, iters
+
+    def gp_slip_ragged(self, kernel, time_array, slip_array, n, theta=None, horizon: int = 600, ldm: Optional[int] = None):
+        """The node callback for windows of different sizes: time_array, slip_array [B,ld] with n[b] samples in row b
+        (e.g. slip_record's [B*max_windows, cap] rows with n = where(published, n_samples, 0)).  Returns (mean [B,ldm],
+        sigma [B,ldm], m_out [B], status [B]) on the device of the inputs; row b holds m_out[b] published points.
+        ldm defaults to the largest ld + horizon (every window of ld stamps fits)."""
+        k, dev, B, ld, P = self._ragged_common(kernel, time_array, n)
+        if ldm is None:
+            ldm = ld + int(horizon)
+        stride, targ = 0, _Arg(None, np.float64, dev, True)
+        if theta is not None:
+            stride = self._theta_stride(theta, P)
+            targ = _Arg(theta, np.float64, dev)
+        mean = self._empty((B, ldm), np.float64, dev)
+        sigma = self._empty((B, ldm), np.float64, dev)
+        m_out = self._empty((B,), np.int32, dev)
+        status = self._empty((B,), np.int32, dev)
+        a = [_Arg(time_array, np.float64, dev), _Arg(slip_array, np.float64, dev), _Arg(n, np.int32, dev),
+             _Arg(mean, np.float64, dev, output=True), _Arg(sigma, np.float64, dev, output=True),
+             _Arg(m_out, np.int32, dev, output=True), _Arg(status, np.int32, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_gp_slip_ragged(self.h, C.byref(k), targ.ptr, stride, a[0].ptr, a[1].ptr, a[2].ptr, ld, B,
+                                          int(horizon), ldm, a[3].ptr, a[4].ptr, a[5].ptr, a[6].ptr,
+                                          L.MEM_DEVICE if dev else L.MEM_HOST)
+        self._check(rc, "cngp_gp_slip_ragged")
+        return mean, sigma, m_out, status
+
     # ------------------------------------------------------------------------------------------------------
     @staticmethod
     def stop_config(**over) -> L.StopConfig:
@@ -273,11 +373,12 @@ class GpContext:
         return c
 
     def zupt_lookahead(self, mean, sigma, P, Q, STM, Hvec, pos, cfg: Optional[L.StopConfig] = None,
-                       want_state: bool = False):
+                       want_state: bool = False, m=None):
         """Batched GpPredictor look-ahead.  mean, sigma [B,M]; each of P,Q,STM ([225] or [B,225]), Hvec ([60] or
         [B,60]), pos ([3] or [B,3]) is shared or per window.  Returns dict(triggered, i_stop, step_stop, xy_err);
         want_state adds P_final [B,225], K_final [B,60], R_final [B,16] - what the reference leaves in the public
-        members P_pred, K_pred, R_IP after the callback (gp_predictor.h:36-43)."""
+        members P_pred, K_pred, R_IP after the callback (gp_predictor.h:36-43).  m [B] (optional): row b of mean / sigma
+        holds m[b] points (cngp_zupt_lookahead_ragged), e.g. the m_out of gp_slip_ragged."""
         dev = _is_cuda(mean)
         B, M = mean.shape
         cfg = cfg or self.stop_config()
@@ -298,6 +399,22 @@ class GpContext:
         a = [_Arg(mean, np.float64, dev), _Arg(sigma, np.float64, dev), _Arg(trig, np.int32, dev),
              _Arg(i_stop, np.int32, dev), _Arg(step, np.int32, dev), _Arg(xy, np.float64, dev)]
         self._bind_stream(dev)
+        if m is not None:
+            if int(np.prod(tuple(m.shape))) != B:
+                raise CngpError(f"m has {int(np.prod(tuple(m.shape)))} entries for {B} windows")
+            ma = _Arg(m, np.int32, dev)
+            st = [None, None, None]
+            if want_state:
+                st = [self._empty((B, n), np.float64, dev) for n in (225, 60, 16)]
+            s3 = [_Arg(v, np.float64, dev, True, output=True) for v in st]
+            rc = self.lib.cngp_zupt_lookahead_ragged(self.h, a[0].ptr, a[1].ptr, B, ma.ptr, M, *[c.ptr for c in ctx_args],
+                                                     mask, C.byref(cfg), a[2].ptr, a[3].ptr, a[4].ptr, a[5].ptr,
+                                                     s3[0].ptr, s3[1].ptr, s3[2].ptr, L.MEM_DEVICE if dev else L.MEM_HOST)
+            self._check(rc, "cngp_zupt_lookahead_ragged")
+            res = dict(triggered=trig, i_stop=i_stop, step_stop=step, xy_err=xy)
+            if want_state:
+                res.update(P_final=st[0], K_final=st[1], R_final=st[2])
+            return res
         if want_state:
             Pf, Kf, Rf = (self._empty((B, n), np.float64, dev) for n in (225, 60, 16))
             s3 = [_Arg(Pf, np.float64, dev, output=True), _Arg(Kf, np.float64, dev, output=True),

@@ -25,7 +25,7 @@ UNITS = {
     "cngp_api.cu": [],
     "zupt_lookahead.cu": ["-fmad=false"],   # explicit fma() only: same operation order as the C oracle
 }
-OPTIONAL_UNITS = {"chol_large.cu": [], "gp_slip.cu": [], "slip_record.cu": ["-fmad=false"], "ekf_context.cu": []}
+OPTIONAL_UNITS = {"chol_large.cu": [], "gp_slip.cu": [], "ragged.cu": [], "slip_record.cu": ["-fmad=false"], "ekf_context.cu": []}
 
 
 def _sources():

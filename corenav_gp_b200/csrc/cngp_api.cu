@@ -21,7 +21,7 @@
 extern "C" int cngp_launch_lookahead(const double*, const double*, long long, int, const double*, const double*,
                                      const double*, const double*, const double*, int, const cngp_stop_config*, int*,
                                      int*, int*, double*, unsigned long long*, double*, double*, double*, const double*, int,
-                                     cudaStream_t);
+                                     cudaStream_t, const int* m_win = nullptr);
 extern "C" int cngp_launch_llh_to_enu(const double*, long long, const cngp_stop_config*, double*, cudaStream_t);
 extern "C" int cngp_launch_ekf_context(const double*, const double*, const double*, const double*, long long, double, double,
                                        double*, double*, double*, cudaStream_t);
@@ -428,7 +428,7 @@ static int launch_var_k(cngp_ctx* ctx, VarArgs& va, long long nwin, cudaStream_t
     va.kstage = (double*)ctx->buf(12, (size_t)grid * G * WG * NT_MAX * 64 * sizeof(double));
     if (!va.kstage) return CNGP_ERR_NOMEM;
   }
-  const bool full = va.nt == NT_MAX && va.N == NT_MAX * 8;
+  const bool full = va.nt == NT_MAX && va.N == NT_MAX * 8 && !va.n_win;
   auto kfn = full ? gp_var_kernel<NT_MAX, G, WG, NSLOT, CT, KID, true, TAB> : gp_var_kernel<NT_MAX, G, WG, NSLOT, CT, KID, false, TAB>;
   cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   kfn<<<(unsigned)grid, G * WG * 32, smem, s>>>(va);
@@ -462,7 +462,7 @@ static int launch_var32(cngp_ctx* ctx, VarArgs& va, long long nwin, cudaStream_t
   const size_t smem = var32_smem_bytes(NSLOT, CT);
   va.kstage = (double*)ctx->buf(12, (size_t)grid * WG * NT_MAX * 32 * 16);
   if (!va.kstage) return CNGP_ERR_NOMEM;
-  const bool full = va.nt == NT_MAX && va.N == NT_MAX * 8;
+  const bool full = va.nt == NT_MAX && va.N == NT_MAX * 8 && !va.n_win;
   auto kfn = full ? gp_var32_kernel<NT_MAX, WG, NSLOT, CT, true> : gp_var32_kernel<NT_MAX, WG, NSLOT, CT, false>;
   cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   kfn<<<(unsigned)grid, WG * 32, smem, s>>>(va);
@@ -505,7 +505,8 @@ static bool lag_tables_enabled() {
 
 int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, int64_t theta_stride,
                       const double* x, const double* y, const double* xstar, int64_t xstar_stride, int64_t B, int32_t N,
-                      int32_t M, double* mean, double* var, double* lml, int32_t* status, int32_t mem, int sigma_mode) {
+                      int32_t M, double* mean, double* var, double* lml, int32_t* status, int32_t mem, int sigma_mode,
+                      const int32_t* n_win, const int32_t* m_win) {
   if (!ctx) return CNGP_ERR_INVALID;
   if (!kernel || !theta || !x || !y || B < 0 || N <= 0 || M < 0) return fail(ctx, CNGP_ERR_INVALID, "predict: bad argument");
   if (M > 0 && (!xstar || !mean || !var)) return fail(ctx, CNGP_ERR_INVALID, "predict: xstar/mean/var null");
@@ -613,6 +614,7 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
     fa.status = d_status;
     fa.jitter_retry = ctx->cfg.jitter_retry;
     fa.Asrc = nullptr; fa.a_col_stride = 0;
+    fa.n_win = n_win;
     ctx->begin(CNGP_PROF_FIT);
     launch_fit(kid, fa, nw, ctx->stream);
     ctx->end();
@@ -627,6 +629,7 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
       va.L = Lbuf; va.z = zbuf; va.feat = fbuf; va.status = d_status; va.mean = d_mean; va.var = d_var;
       va.sigma_mode = sigma_mode;
       va.kstage = nullptr;
+      va.n_win = n_win; va.m_win = m_win;
       ctx->begin(CNGP_PROF_VAR);
       int vrc;
       if (f32) {
@@ -685,7 +688,7 @@ extern "C" int cngp_predict_batch(cngp_ctx* ctx, const cngp_kernel* kernel, cons
                                   int64_t B, int32_t N, int32_t M, double* mean, double* var, double* lml,
                                   int32_t* status, int32_t mem) {
   return cngp_predict_impl(ctx, kernel, theta, theta_stride, x, y, xstar, xstar_stride, B, N, M, mean, var, lml, status,
-                           mem, 0);
+                           mem, 0, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -694,7 +697,7 @@ extern "C" int cngp_predict_batch(cngp_ctx* ctx, const cngp_kernel* kernel, cons
 // ------------------------------------------------------------------------------------------------------------
 int cngp_lml_grad_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, int64_t C, const double* x,
                        const double* y, int64_t B, int32_t N, double* lml, double* grad, int32_t* status, int32_t mem,
-                       const int32_t* win_map, const int32_t* skip) {
+                       const int32_t* win_map, const int32_t* skip, const int32_t* n_win) {
   if (!ctx) return CNGP_ERR_INVALID;
   if (!kernel || !theta || !x || !y || C < 0 || B < 0 || N <= 0) return fail(ctx, CNGP_ERR_INVALID, "lml_grad: bad argument");
   if (N > CNGP_MAX_N) return fail(ctx, CNGP_ERR_UNSUPPORTED, "lml_grad: N=%d > %d", N, CNGP_MAX_N);
@@ -746,6 +749,7 @@ int cngp_lml_grad_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
     fa.status = d_status;
     fa.jitter_retry = ctx->cfg.jitter_retry;
     fa.Asrc = nullptr; fa.a_col_stride = 0;
+    fa.n_win = n_win;
     ctx->begin(CNGP_PROF_FIT);
     launch_fit(match_fast_kernel(kp), fa, np, ctx->stream);
     ctx->end();
@@ -756,6 +760,7 @@ int cngp_lml_grad_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
       ga.x = d_x; ga.N = N; ga.nt = nt; ga.n_windows = (int)B; ga.problem0 = p0;
       ga.L = Lbuf; ga.W = Wbuf; ga.z = zbuf; ga.alpha = abuf; ga.status = d_status; ga.grad = d_grad;
       ga.skip = skip;
+      ga.n_win = n_win;
       // uniform-stamp contraction of gp_grad_kernel: stationary expressions, or few product terms with Brownian / Linear factors
       ga.lag_ok = fa.lag_ok ? 1 : ((lag_tables_enabled() && kp.n_terms <= GRAD_UNI_TERMS) ? 2 : 0);
       ctx->begin(CNGP_PROF_GRAD);
@@ -807,11 +812,20 @@ extern "C" int cngp_zupt_lookahead_batch(cngp_ctx* ctx, const double* mean, cons
                                       step_stop, xy_err, nullptr, nullptr, nullptr, mem);
 }
 
-extern "C" int cngp_zupt_lookahead_batch_ex(cngp_ctx* ctx, const double* mean, const double* sigma, int64_t B, int32_t M,
-                                            const double* P, const double* Q, const double* STM, const double* Hvec,
-                                            const double* pos, int32_t per_window, const cngp_stop_config* cfg,
-                                            int32_t* triggered, int32_t* i_stop, int32_t* step_stop, double* xy_err,
-                                            double* P_final, double* K_final, double* R_final, int32_t mem) {
+namespace {
+// any m[b] outside [0, ldm] sets *bad
+__global__ void ragged_m_check_kernel(const int* m, long long B, int ldm, int* bad) {
+  const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B && (m[b] < 0 || m[b] > ldm)) atomicOr(bad, 1);
+}
+}  // namespace
+
+// M: points per window, or (m != null) the row stride of mean / sigma with m[b] <= M points in row b
+static int lookahead_impl(cngp_ctx* ctx, const double* mean, const double* sigma, int64_t B, int32_t M, const int32_t* m,
+                          const double* P, const double* Q, const double* STM, const double* Hvec, const double* pos,
+                          int32_t per_window, const cngp_stop_config* cfg, int32_t* triggered, int32_t* i_stop,
+                          int32_t* step_stop, double* xy_err, double* P_final, double* K_final, double* R_final,
+                          int32_t mem) {
   if (!ctx) return CNGP_ERR_INVALID;
   if ((K_final || R_final) && !P_final) return fail(ctx, CNGP_ERR_INVALID, "lookahead: K_final / R_final need P_final");
   if (!mean || !sigma || !P || !Q || !STM || !Hvec || !pos || !triggered || !i_stop || B < 0 || M <= 0)
@@ -822,6 +836,22 @@ extern "C" int cngp_zupt_lookahead_batch_ex(cngp_ctx* ctx, const double* mean, c
   if (c.ratio <= 0) return fail(ctx, CNGP_ERR_INVALID, "lookahead: ratio must be positive");
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   Stage st{ctx, mem};
+  const int* d_m = (const int*)st.in(m, sizeof(int) * (size_t)B);
+  if (m) {   // every count within its row: one flag read back (device memory) or a host loop
+    if (mem == CNGP_MEM_HOST) {
+      for (int64_t b = 0; b < B; ++b)
+        if (m[b] < 0 || m[b] > M) return fail(ctx, CNGP_ERR_INVALID, "lookahead_ragged: m[%lld] = %d outside [0, ldm = %d]", (long long)b, m[b], M);
+    } else {
+      int* d_bad = (int*)ctx->buf(20, 64);
+      int bad = 0;
+      if (!d_bad) return fail(ctx, CNGP_ERR_NOMEM, "lookahead_ragged: flag buffer");
+      CU(ctx, cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
+      ragged_m_check_kernel<<<(unsigned)((B + 255) / 256), 256, 0, ctx->stream>>>(d_m, B, M, d_bad);
+      CU(ctx, cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+      CU(ctx, cudaStreamSynchronize(ctx->stream));
+      if (bad) return fail(ctx, CNGP_ERR_INVALID, "lookahead_ragged: some m[b] outside [0, ldm = %d]", M);
+    }
+  }
   auto cnt = [&](int bit, size_t sz) { return sizeof(double) * sz * ((per_window & bit) ? (size_t)B : 1); };
   const double* d_mean = (const double*)st.in(mean, sizeof(double) * (size_t)B * M);
   const double* d_sigma = (const double*)st.in(sigma, sizeof(double) * (size_t)B * M);
@@ -848,12 +878,32 @@ extern "C" int cngp_zupt_lookahead_batch_ex(cngp_ctx* ctx, const double* mean, c
   if (d_Kf) CU(ctx, cudaMemsetAsync(d_Kf, 0, sizeof(double) * 60 * (size_t)B, ctx->stream));   // windows without an update
   if (d_Rf) CU(ctx, cudaMemsetAsync(d_Rf, 0, sizeof(double) * 16 * (size_t)B, ctx->stream));
   const int e = cngp_launch_lookahead(d_mean, d_sigma, B, M, d_P, d_Q, d_F, d_H, d_pos, per_window, &c, d_trig, d_i,
-                                      d_step, d_xy, d_counter, d_Pf, d_Kf, d_Rf, nullptr, 0, ctx->stream);
+                                      d_step, d_xy, d_counter, d_Pf, d_Kf, d_Rf, nullptr, 0, ctx->stream, d_m);
   ctx->end();
   if (e) return fail(ctx, CNGP_ERR_CUDA, "lookahead launch: %s", cudaGetErrorString((cudaError_t)e));
   const int rc = st.finish();
   if (rc) return fail(ctx, rc, "lookahead: copy-out failed: %s", cudaGetErrorString(cudaGetLastError()));
   return CNGP_OK;
+}
+
+extern "C" int cngp_zupt_lookahead_batch_ex(cngp_ctx* ctx, const double* mean, const double* sigma, int64_t B, int32_t M,
+                                            const double* P, const double* Q, const double* STM, const double* Hvec,
+                                            const double* pos, int32_t per_window, const cngp_stop_config* cfg,
+                                            int32_t* triggered, int32_t* i_stop, int32_t* step_stop, double* xy_err,
+                                            double* P_final, double* K_final, double* R_final, int32_t mem) {
+  return lookahead_impl(ctx, mean, sigma, B, M, nullptr, P, Q, STM, Hvec, pos, per_window, cfg, triggered, i_stop,
+                        step_stop, xy_err, P_final, K_final, R_final, mem);
+}
+
+extern "C" int cngp_zupt_lookahead_ragged(cngp_ctx* ctx, const double* mean, const double* sigma, int64_t B,
+                                          const int32_t* m, int32_t ldm, const double* P, const double* Q,
+                                          const double* STM, const double* Hvec, const double* pos, int32_t per_window,
+                                          const cngp_stop_config* cfg, int32_t* triggered, int32_t* i_stop,
+                                          int32_t* step_stop, double* xy_err, double* P_final, double* K_final,
+                                          double* R_final, int32_t mem) {
+  if (!m) return ctx ? fail(ctx, CNGP_ERR_INVALID, "lookahead_ragged: m is null") : CNGP_ERR_INVALID;
+  return lookahead_impl(ctx, mean, sigma, B, ldm, m, P, Q, STM, Hvec, pos, per_window, cfg, triggered, i_stop, step_stop,
+                        xy_err, P_final, K_final, R_final, mem);
 }
 
 // The filter's own covariance recursion for B operating points (SURVEY.md 8f row N4, the P half): n_steps IMU steps of

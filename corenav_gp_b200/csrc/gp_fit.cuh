@@ -86,6 +86,9 @@ struct FitArgs {
   // evaluated - tile (i, j) of the block at Asrc + j * a_col_stride + i * 64 (lower tiles only are read).
   const double* Asrc;
   long long a_col_stride;
+  // ragged batches: valid training points of each window (n_win[window] <= N, ceil(n_win / 8) == nt); N is then the row
+  // stride of x / y only, and the window is identity-padded beyond its own count.  null: every window has N points.
+  const int* n_win;
 #ifdef CNGP_FIT_TIMING
   long long* dbg;        // tools/fit_bench.cu: per-warp phase cycle counters of block 0, [warp][8]
 #endif
@@ -185,13 +188,13 @@ __global__ void __launch_bounds__((NW + 1) * 32, NW * T > 18 ? 1 : 2) gp_fit_ker
   const int win = a.win_map ? a.win_map[p] : (int)(p % a.n_windows);
   const long long ti = a.theta_mode == 0 ? 0 : (a.theta_mode == 1 ? (long long)win : (a.theta_mode == 3 ? p : p / a.n_windows));
   const double* th = a.theta + ti * a.theta_stride;
-  const int N = a.N, nt = a.nt;
+  const int ld = a.N, N = a.n_win ? a.n_win[win] : a.N, nt = a.nt;
   const int h = (nt + 1) / 2;                       // columns >= h re-use the dead heads of columns < h
   const double noise = (KID == KID_TILES) ? 0.0 : th[a.kp.n_params];
   FastK<KID> fk;
   if (KID != KID_GENERIC && KID != KID_TILES) {
     fk.init(th);
-    fk.base = a.x[(long long)win * N];        // phase origin: the window's first stamp (gp_var_kernel uses the same)
+    fk.base = a.x[(long long)win * ld];        // phase origin: the window's first stamp (gp_var_kernel uses the same)
     if (tid < 64) {
       const double t = EXP2_TAB64[tid];
       etab[tid] = fk.scale1() * t;
@@ -200,8 +203,8 @@ __global__ void __launch_bounds__((NW + 1) * 32, NW * T > 18 ? 1 : 2) gp_fit_ker
   }
 
   for (int i = tid; i < nt * 8; i += FIT_THREADS) {
-    const double xv = (KID != KID_TILES && i < N) ? a.x[(long long)win * N + i] : 0.0;
-    ys[i] = (KID != KID_TILES && i < N) ? a.y[(long long)win * N + i] : 0.0;
+    const double xv = (KID != KID_TILES && i < N) ? a.x[(long long)win * ld + i] : 0.0;
+    ys[i] = (KID != KID_TILES && i < N) ? a.y[(long long)win * ld + i] : 0.0;
     PointFeat f{xv, __dmul_rn(xv, xv), 0.0, 0.0};
     if (KID != KID_GENERIC && KID != KID_TILES) f = fk.point(xv);
     fx[i] = f.x; fxx[i] = f.xx; fc[i] = f.c; fs[i] = f.s;

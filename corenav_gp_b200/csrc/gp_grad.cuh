@@ -38,6 +38,7 @@ struct GradArgs {
   const int* status;       // [n_problems]
   double* grad;            // [n_problems][P]
   const int* skip;         // [n_problems] or null: problems with skip[p] != 0 are left untouched
+  const int* n_win;        // ragged batches: valid points of each window (x rows keep the stride N), or null
   int lag_ok;              // host check of the expression: 1 stationary, 2 at most GRAD_UNI_TERMS product terms with Brownian
                            // / Linear factors - the uniform-stamp contraction may be used; 0 never
 };
@@ -80,13 +81,13 @@ __global__ void __launch_bounds__(GRAD_WARPS * 32) gp_grad_kernel(const GradArgs
   const int win = a.win_map ? a.win_map[p] : (int)(p % a.n_windows);
   const long long cand = a.win_map ? p : p / a.n_windows;
   const double* th = a.theta + cand * a.theta_stride;
-  const int N = a.N, nt = a.nt, P = a.kp.n_params + 1;
+  const int ld = a.N, N = a.n_win ? a.n_win[win] : a.N, nt = a.nt, P = a.kp.n_params + 1;
   const double* Lp = a.L + lp * (long long)tiles_in_lower(nt) * 64;
   double* Wp = SMEM ? gsm + (size_t)tiles_in_lower(nt) * 64 : a.W + lp * (long long)tiles_in_lower(nt) * 64;
   const double* zp = a.z + lp * (long long)(nt * 8);
 
   for (int i = tid; i < nt * 8; i += GRAD_THREADS) {
-    xs[i] = i < N ? a.x[(long long)win * N + i] : 0.0;
+    xs[i] = i < N ? a.x[(long long)win * ld + i] : 0.0;
     zs[i] = zp[i];
   }
   if (tid < P) thv[tid] = th[tid];
@@ -108,7 +109,7 @@ __global__ void __launch_bounds__(GRAD_WARPS * 32) gp_grad_kernel(const GradArgs
   // stamps x_i = x_0 + i exactly (integers below 2^26, so that the expanded-form r^2 is exact) and a stationary expression
   int uni = a.lag_ok != 0;
   for (int i = tid; i < N; i += GRAD_THREADS) {
-    const double v = a.x[(long long)win * N + i], v0 = a.x[(long long)win * N];
+    const double v = a.x[(long long)win * ld + i], v0 = a.x[(long long)win * ld];
     uni &= (v == v0 + (double)i) && (v0 == rint(v0)) && (fabs(v) < 67108864.0);
   }
   const bool uniform = __syncthreads_and(uni) != 0;

@@ -125,16 +125,6 @@ int cngp_optimize_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
   if (cudaSetDevice(cngp_ctx_device(ctx)) != cudaSuccess) return cngp_set_error(ctx, CNGP_ERR_CUDA, "optimize: cudaSetDevice failed");
   cudaStream_t s = cngp_ctx_stream(ctx);
   const size_t xy = sizeof(double) * (size_t)B * N;
-  Optimizer* d_st = (Optimizer*)cngp_ctx_buf(ctx, SLOT_OPT_STATE, sizeof(Optimizer) * (size_t)B);
-  double* d_th = (double*)cngp_ctx_buf(ctx, SLOT_OPT_TH, sizeof(double) * B * P);
-  int* d_map = (int*)cngp_ctx_buf(ctx, SLOT_OPT_MAP, sizeof(int) * B);
-  double* d_lml = (double*)cngp_ctx_buf(ctx, SLOT_OPT_LML, sizeof(double) * B);
-  double* d_grad = (double*)cngp_ctx_buf(ctx, SLOT_OPT_GRAD, sizeof(double) * B * P);
-  int* d_st_fit = (int*)cngp_ctx_buf(ctx, SLOT_OPT_ST, sizeof(int) * B);
-  int* d_done = (int*)cngp_ctx_buf(ctx, SLOT_OPT_DONE, sizeof(int) * B);
-  int* d_nact = (int*)cngp_ctx_buf(ctx, SLOT_OPT_NACT, 64);
-  if (!d_st || !d_th || !d_map || !d_lml || !d_grad || !d_st_fit || !d_done || !d_nact)
-    return cngp_set_error(ctx, CNGP_ERR_NOMEM, "optimize: device allocation failed");
   const double *d_x = x, *d_y = y, *d_th0 = theta0;
   double* d_out = theta_out; double* d_lout = lml_out; int* d_iout = iters_out;
   if (host) {
@@ -151,7 +141,42 @@ int cngp_optimize_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
     d_x = bx; d_y = by; d_th0 = b0;
     d_out = bo; d_lout = bo + (size_t)B * P; d_iout = (int*)(bo + (size_t)B * (P + 1));
   }
+  const OptBucket all{0, B, N, d_x, d_y, nullptr};
+  const int rc = cngp_optimize_run(ctx, &kk, d_th0, theta0_stride, B, max_iters, &all, 1, d_out, d_lout, d_iout);
+  if (rc) return rc;
+  if (host) {
+    if (cudaMemcpyAsync(theta_out, d_out, sizeof(double) * B * P, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+        (lml_out && cudaMemcpyAsync(lml_out, d_lout, sizeof(double) * B, cudaMemcpyDeviceToHost, s) != cudaSuccess) ||
+        (iters_out && cudaMemcpyAsync(iters_out, d_iout, sizeof(int) * B, cudaMemcpyDeviceToHost, s) != cudaSuccess) ||
+        cudaStreamSynchronize(s) != cudaSuccess)
+      return cngp_set_error(ctx, CNGP_ERR_CUDA, "optimize: download failed");
+  }
+  return CNGP_OK;
+}
+
+// The optimiser loop over B windows held in buckets (see OptBucket): one fit + gradient per bucket and one
+// opt_feed_kernel over all B windows per iteration.  Every pointer is a device pointer.
+int cngp_optimize_run(cngp_ctx* ctx, const cngp_kernel* kernel, const double* d_th0, int64_t theta0_stride, int64_t B,
+                      int32_t max_iters, const OptBucket* buckets, int n_buckets, double* d_out, double* d_lout,
+                      int32_t* d_iout) {
+  cngp_kernel kk = *kernel;
+  if (cngp_kernel_finalize(&kk) != CNGP_OK) return cngp_set_error(ctx, CNGP_ERR_INVALID, "optimize: invalid kernel expression");
+  const int P = kk.n_params + 1;
+  if (P > kMaxP) return cngp_set_error(ctx, CNGP_ERR_UNSUPPORTED, "optimize: too many hyper-parameters");
+  if (max_iters <= 0) max_iters = 1000;
+  cudaStream_t s = cngp_ctx_stream(ctx);
+  Optimizer* d_st = (Optimizer*)cngp_ctx_buf(ctx, SLOT_OPT_STATE, sizeof(Optimizer) * (size_t)B);
+  double* d_th = (double*)cngp_ctx_buf(ctx, SLOT_OPT_TH, sizeof(double) * B * P);
+  int* d_map = (int*)cngp_ctx_buf(ctx, SLOT_OPT_MAP, sizeof(int) * B);
+  double* d_lml = (double*)cngp_ctx_buf(ctx, SLOT_OPT_LML, sizeof(double) * B);
+  double* d_grad = (double*)cngp_ctx_buf(ctx, SLOT_OPT_GRAD, sizeof(double) * B * P);
+  int* d_st_fit = (int*)cngp_ctx_buf(ctx, SLOT_OPT_ST, sizeof(int) * B);
+  int* d_done = (int*)cngp_ctx_buf(ctx, SLOT_OPT_DONE, sizeof(int) * B);
+  int* d_nact = (int*)cngp_ctx_buf(ctx, SLOT_OPT_NACT, 64);
+  if (!d_st || !d_th || !d_map || !d_lml || !d_grad || !d_st_fit || !d_done || !d_nact)
+    return cngp_set_error(ctx, CNGP_ERR_NOMEM, "optimize: device allocation failed");
   const unsigned blocks = (unsigned)((B + 63) / 64);
+  // d_map[b] = b: problem p of a bucket is the bucket's window p (theta row p of the bucket's slice)
   opt_init_kernel<<<blocks, 64, 0, s>>>(d_st, d_th0, theta0_stride, P, max_iters, B, d_th, d_map, d_done);
   constexpr int OPT_BLIND = 6;
   const unsigned feed_blocks = (unsigned)((B + FEED_WPB - 1) / FEED_WPB);
@@ -162,8 +187,13 @@ int cngp_optimize_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
   for (int round = 0; n_active > 0 && round * OPT_BLIND <= max_iters + OPT_BLIND; ++round) {
     for (int k = 0; k < OPT_BLIND; ++k) {
       if (cudaMemsetAsync(d_nact, 0, sizeof(int), s) != cudaSuccess) return cngp_set_error(ctx, CNGP_ERR_CUDA, "optimize: memset failed");
-      const int rc = cngp_lml_grad_impl(ctx, &kk, d_th, B, d_x, d_y, B, N, d_lml, d_grad, d_st_fit, CNGP_MEM_DEVICE, d_map, d_done);
-      if (rc) return rc;
+      for (int k = 0; k < n_buckets; ++k) {
+        const OptBucket& bk = buckets[k];
+        const int rc = cngp_lml_grad_impl(ctx, &kk, d_th + bk.off * P, bk.nb, bk.x, bk.y, bk.nb, bk.ld, d_lml + bk.off,
+                                          d_grad + bk.off * P, d_st_fit + bk.off, CNGP_MEM_DEVICE, d_map, d_done + bk.off,
+                                          bk.n_win);
+        if (rc) return rc;
+      }
       cngp_ctx_begin(ctx, CNGP_PROF_MISC);
       opt_feed_kernel<<<feed_blocks, FEED_WPB * 32, feed_smem, s>>>(d_st, d_lml, d_grad, d_st_fit, P, B, d_th, d_done, d_nact);
       cngp_ctx_end(ctx);
@@ -174,13 +204,6 @@ int cngp_optimize_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
   }
   opt_result_kernel<<<blocks, 64, 0, s>>>(d_st, P, B, d_out, d_lout, d_iout);
   if (cudaGetLastError() != cudaSuccess) return cngp_set_error(ctx, CNGP_ERR_CUDA, "optimize: kernel launch failed");
-  if (host) {
-    if (cudaMemcpyAsync(theta_out, d_out, sizeof(double) * B * P, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-        (lml_out && cudaMemcpyAsync(lml_out, d_lout, sizeof(double) * B, cudaMemcpyDeviceToHost, s) != cudaSuccess) ||
-        (iters_out && cudaMemcpyAsync(iters_out, d_iout, sizeof(int) * B, cudaMemcpyDeviceToHost, s) != cudaSuccess) ||
-        cudaStreamSynchronize(s) != cudaSuccess)
-      return cngp_set_error(ctx, CNGP_ERR_CUDA, "optimize: download failed");
-  }
   return CNGP_OK;
 }
 

@@ -60,6 +60,10 @@ struct VarArgs {
   const int* kxi;          // [chunk][nt*8]
   const int* n_lazy;       // windows of this launch without a valid table: the TAB kernel runs iff it is 0, the lazy one
                            // iff it is not (both are launched; one of them returns at once).  null: lazy only.
+  // ragged batches (null: every window has N training / M test points).  n_win[win]: valid training points, ceil(/8) == nt;
+  // m_win[win] <= M: valid test points - mean / var entries at or beyond it are not written (M stays the row stride).
+  const int* n_win;
+  const int* m_win;
 };
 
 struct VarGroupShared {
@@ -102,7 +106,7 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int grp = w / WG, wg = w % WG;
   const int r = lane >> 2, q = lane & 3;
-  const int N = FULL ? NT_MAX * 8 : a.N, nt = FULL ? NT_MAX : a.nt, M = a.M, mt = a.mt;
+  const int nt = FULL ? NT_MAX : a.nt, M = a.M, mt = a.mt;
   const int n8 = nt * 8;
   const int n_tiles = tiles_in_lower(nt);
   const int ce_max = (n_tiles - 1) / VAR_CT;      // chunk ids count from the END of a window's factor
@@ -190,6 +194,7 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
     const double* km = TAB ? a.kmeta + lw * (long long)VAR_META : nullptr;
     const double noise = TAB ? km[2] : th[a.kp.n_params];
     const bool bad = a.status && a.status[win] < 0;
+    const int N = FULL ? NT_MAX * 8 : (a.n_win ? a.n_win[win] : a.N);
 
     const int m = min(8 * m8 + r, M - 1);
     const double xm = a.xstar[(a.xstar_stride ? win * a.xstar_stride : 0) + m];
@@ -301,7 +306,7 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
     vs += __shfl_xor_sync(0xffffffffu, vs, 2);
     ms += __shfl_xor_sync(0xffffffffu, ms, 1);
     ms += __shfl_xor_sync(0xffffffffu, ms, 2);
-    if (q == 0 && 8 * m8 + r < M) {
+    if (q == 0 && 8 * m8 + r < (a.m_win ? a.m_win[win] : M)) {
       const double kss = TAB ? km[0] : (KID == KID_GENERIC) ? kdiag_eval(kps, hc, xm) : fk.kdiag(xm);
       const double nanv = __longlong_as_double(0x7ff8000000000000LL);
       a.mean[win * M + m] = bad ? nanv : ms;

@@ -63,7 +63,7 @@ __global__ void __launch_bounds__(WG * 32, 1) gp_var32_kernel(const VarArgs a) {
   __shared__ VarGroupShared shg[1];
   const int lane = threadIdx.x & 31, wg = threadIdx.x >> 5;
   const int g8 = lane >> 2, t = lane & 3;
-  const int N = FULL ? NT_MAX * 8 : a.N, nt = FULL ? NT_MAX : a.nt, M = a.M, mt = a.mt;   // mt = ceil(M / 16) here
+  const int nt = FULL ? NT_MAX : a.nt, M = a.M, mt = a.mt;   // mt = ceil(M / 16) here
   const int n8 = nt * 8;
   const int n_tiles = tiles_in_lower(nt);
   const int ce_max = (n_tiles - 1) / VAR_CT;
@@ -129,6 +129,7 @@ __global__ void __launch_bounds__(WG * 32, 1) gp_var32_kernel(const VarArgs a) {
     const bool tab = km && km[3] != 0.0;
     const double noise = th[a.kp.n_params];
     const bool bad = a.status && a.status[win] < 0;
+    const int N = FULL ? NT_MAX * 8 : (a.n_win ? a.n_win[win] : a.N);
     const int m_lo = min(16 * m16 + g8, M - 1), m_hi = min(16 * m16 + 8 + g8, M - 1);
     const double* xsp = a.xstar + (a.xstar_stride ? win * a.xstar_stride : 0);
     const double x_lo = xsp[m_lo], x_hi = xsp[m_hi];
@@ -222,7 +223,7 @@ __global__ void __launch_bounds__(WG * 32, 1) gp_var32_kernel(const VarArgs a) {
     ms_hi += __shfl_xor_sync(0xffffffffu, ms_hi, 1); ms_hi += __shfl_xor_sync(0xffffffffu, ms_hi, 2);
     if (t < 2) {     // lane t = 0 writes the point of row g, t = 1 the point of row g + 8
       const int mrow = 16 * m16 + g8 + 8 * t;
-      if (mrow < M) {
+      if (mrow < (a.m_win ? a.m_win[win] : M)) {
         const double xm = t ? x_hi : x_lo;
         const double kss = tab ? km[0] : kdiag_eval(kps, hc, xm);
         const double vsum = t ? (double)vs_hi : (double)vs_lo, msum = t ? (double)ms_hi : (double)ms_lo;

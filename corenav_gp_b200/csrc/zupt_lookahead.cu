@@ -35,6 +35,7 @@ struct LookaheadArgs {
   // predicted slip (CoreNav.cpp:228 uses the filter's constant R_), tensor-core kernel only
   const double* R_fixed; int R_per_window;
   long long ms_stride;   // row stride of mean / sigma: M, or 0 when every window shares one row
+  const int* m_win;      // ragged batches: GP_Output points of each window (<= M; the loop runs ratio * m_win[b] steps), or null
 };
 
 struct LlhConst {
@@ -322,7 +323,7 @@ __global__ void __launch_bounds__(TC_WARPS * 32, 2) zupt_lookahead_tc_kernel(con
 
   const double* mean = a.mean + b * a.ms_stride;
   const double* sigma = a.sigma + b * a.ms_stride;
-  const int nsteps = cfg.ratio * a.M;
+  const int nsteps = cfg.ratio * (a.m_win ? a.m_win[b] : a.M);
   int i_upd = 0, trig = 0, step = nsteps;
   double xy = 0.0;
   // R1 of gp_predictor.cpp:84-87 seen from this lane: row g (as the left factor), rows 2t, 2t+1 (as the right factor)
@@ -591,7 +592,7 @@ __global__ void __launch_bounds__(LA_WARPS * 32) zupt_lookahead_kernel(const Loo
 
   const double* mean = a.mean + b * a.ms_stride;
   const double* sigma = a.sigma + b * a.ms_stride;
-  const int nsteps = cfg.ratio * a.M;
+  const int nsteps = cfg.ratio * (a.m_win ? a.m_win[b] : a.M);
   int i_upd = 0, trig = 0, step = nsteps;
   double xy = 0.0;
 
@@ -830,7 +831,7 @@ __global__ void __launch_bounds__(LA_CTA_THREADS) zupt_lookahead_cta_kernel(cons
 
   const double* mean = a.mean + b * a.ms_stride;
   const double* sigma = a.sigma + b * a.ms_stride;
-  const int nsteps = cfg.ratio * a.M;
+  const int nsteps = cfg.ratio * (a.m_win ? a.m_win[b] : a.M);
   const bool ent = tid < 225;
   const int rr = tid / 15, cc = tid % 15;      // entry (rr, cc) of a 15x15 matrix
   const int r4 = tid / 4, m4 = tid % 4;        // entry (r4, m4) of a 15x4 matrix (tid < 60), (m4', n4) of 4x4 (tid < 16)
@@ -980,11 +981,11 @@ extern "C" int cngp_launch_lookahead(const double* mean, const double* sigma, lo
                                      int per_window, const cngp_stop_config* cfg, int* triggered, int* i_stop,
                                      int* step_stop, double* xy_err, unsigned long long* work_counter,
                                      double* P_final, double* K_final, double* R_final, const double* R_fixed,
-                                     int R_per_window, cudaStream_t stream) {
+                                     int R_per_window, cudaStream_t stream, const int* m_win) {
   using namespace cngp;
   // M < 0: |M| entries of mean / sigma shared by every window (cngp_ekf_covariance_batch)
   LookaheadArgs a{mean, sigma, B, M < 0 ? -M : M, P, Q, STM, Hvec, pos, per_window, *cfg, triggered, i_stop, step_stop,
-                  xy_err, nullptr, P_final, K_final, R_final, R_fixed, R_per_window, M < 0 ? 0LL : (long long)M};
+                  xy_err, nullptr, P_final, K_final, R_final, R_fixed, R_per_window, M < 0 ? 0LL : (long long)M, m_win};
   const size_t smem = (size_t)LA_WARPS * LA_WS * sizeof(double);
   static bool attr_set = false;
   if (!attr_set) {

@@ -294,11 +294,15 @@ def monte_carlo_contexts(first: int, count: int, seed: int = SEED, decades: floa
                 quality=u)
 
 
-def drives(first: int, count: int, T: int = 400, seed: int = SEED, stop_events: bool = True):
+def drives(first: int, count: int, T: int = 400, seed: int = SEED, stop_events: bool = True, pauses: bool = False):
     """Synthetic odometry logs for the slip recorder (SURVEY.md 8f row N1): dict(joint [B,T,4], att [B,T,3],
     vel [B,T,3], cmd [B,T], stop_cmd [B,T]).  10 Hz updates: standstill for a per-drive lead-in, then a 0.8 m/s drive at
     the survey heading with wheel slip of the slipVal.csv scale on the right/left wheel pairs, an occasional stuck phase
-    (slip clamps to 1) and, on some drives, a stop command shortly after the first window closes."""
+    (slip clamps to 1) and, on some drives, a stop command shortly after the first window closes.
+
+    pauses: the drive command is released (cmd = 0) for 0-134 updates at a per-drive place inside the first window, so
+    the recorder's windows hold different numbers of samples (from a few up to the window length) with gaps in their
+    stamps - the ragged GP_Input a real drive produces (CoreNav.cpp:264-300)."""
     ids = np.arange(first, first + count, dtype=np.int64)
     k = np.arange(T)[None, :]
     lead = (5 + 40 * _uniforms(ids, seed, stream=11)).astype(np.int64)[:, None]
@@ -317,6 +321,10 @@ def drives(first: int, count: int, T: int = 400, seed: int = SEED, stop_events: 
     R = 0.11
     joint = np.stack([-wl / R, wr / R, -wl / R * 0.999, wr / R * 1.001], axis=-1)
     cmd = np.where(driving, 1.0, 0.0)
+    if pauses:
+        p0 = lead + 12 + np.floor(140.0 * _uniforms(ids, seed, stream=19)).astype(np.int64)[:, None]
+        plen = np.floor(135.0 * _uniforms(ids, seed, stream=20)).astype(np.int64)[:, None]
+        cmd = np.where((k >= p0) & (k < p0 + plen), 0.0, cmd)
     stop_cmd = np.full((count, T), np.nan)
     if stop_events:
         has = _uniforms(ids, seed, stream=18) < 0.5

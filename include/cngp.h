@@ -19,6 +19,7 @@
  *   cngp_slip_record_batch      replaces the slip extraction + GP_Input recorder of CoreNav::Update, CoreNav.cpp:244-329
  *   cngp_ekf_context_batch      replaces insErrorStateModel_LNF / calc_Q (CoreNav.cpp:411-527) behind SetStopping
  *   cngp_chol_large*            the N = 32768 single-window factorisation of BASELINE.json configs[4] (same math as a3)
+ *   cngp_*_ragged               the same entry points for windows of different sizes in one call (recorder output)
  *
  * Conventions: plain C, int status returns (0 = ok, negative = error; text via cngp_last_error), no exceptions
  * cross the ABI, caller-owned buffers, row-major, FP64.  Every array argument is either a HOST pointer or a DEVICE
@@ -173,6 +174,45 @@ int cngp_gp_slip_batch(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
                        const double* time_array, const double* slip_array, int64_t B, int32_t n,
                        int32_t horizon, int32_t m_cap, double* mean, double* sigma, int32_t* m_out, int32_t* status);
 
+/* ---- ragged window batches ----
+ * The windows GP_Input carries differ in size (CoreNav.cpp:264-300: n_samples from min_samples up to the window length,
+ * stamps with gaps), so these entry points take per-window counts.  Window b has n[b] valid samples in a row of ld
+ * doubles of x / y (time_array / slip_array) and m[b] valid test points in a row of ldm doubles of xstar / mean / var /
+ * sigma.  Entries beyond n[b] and m[b] are never read and never written (NaN there does not matter).  A window with
+ * n[b] = 0 is skipped: nothing is written for it and its status is 0.  The windows are grouped on the device by
+ * ceil(n[b] / 8) and every group runs the launch shape of the fixed-size entry points, so results equal theirs; each
+ * call makes one small device-to-host read (the group sizes).  All arrays follow `mem`. */
+
+/* cngp_predict_batch (gp_slip_node.py:35,47-50, rows a3 + a6) for ragged windows: theta [B][P] or shared (stride 0);
+ * x, y [B][ld]; xstar, mean, var [B][ldm]; lml [B] (lml uses each window's own n: -n/2 log 2 pi); status [B]. */
+int cngp_predict_ragged(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, int64_t theta_stride,
+                        const double* x, const double* y, const int32_t* n, int32_t ld, const double* xstar,
+                        const int32_t* m, int32_t ldm, int64_t B, double* mean, double* var, double* lml,
+                        int32_t* status, int32_t mem);
+
+/* cngp_lml_grad_batch (gp_slip_node.py:36, rows a3 + a4) for C candidates x B ragged windows: theta [C][P];
+ * x, y [B][ld]; lml [C][B]; grad [C][B][P] (may be NULL); status [C][B]. */
+int cngp_lml_grad_ragged(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, int64_t C, const double* x,
+                         const double* y, const int32_t* n, int32_t ld, int64_t B, double* lml, double* grad,
+                         int32_t* status, int32_t mem);
+
+/* cngp_optimize_batch_mem (m.optimize(), gp_slip_node.py:36, row a4) for ragged windows: theta0 [B][P] or shared
+ * (stride 0) or NULL (all ones, as GPy); theta_out [B][P]; lml_out, iters_out [B] (may be NULL). */
+int cngp_optimize_ragged(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta0, int64_t theta0_stride,
+                         const double* x, const double* y, const int32_t* n, int32_t ld, int64_t B, int32_t max_iters,
+                         double* theta_out, double* lml_out, int32_t* iters_out, int32_t mem);
+
+/* The node callback gp_slip_node.py:16-63 (rows a1-a7) for ragged windows, e.g. cngp_slip_record_batch output in place
+ * (rows [B * max_windows] of cap doubles, n = n_samples of the published windows, 0 elsewhere).  Per window:
+ * ntr = int(0.9 n) training samples, grid arange(min, max + horizon, 1), m_out[b] = len(grid) - n published points
+ * in mean / sigma [B][ldm] (sigma = 2 sqrt(var)).  n[b] < 2: m_out[b] = 0, status 0, nothing written.  n[b] > ld or
+ * m_out[b] > ldm: CNGP_ERR_INVALID before any work; ntr > CNGP_MAX_N: CNGP_ERR_UNSUPPORTED.  theta [B][P] or shared;
+ * NULL fits the hypers first (cngp_optimize_ragged from all ones). */
+int cngp_gp_slip_ragged(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, int64_t theta_stride,
+                        const double* time_array, const double* slip_array, const int32_t* n, int32_t ld, int64_t B,
+                        int32_t horizon, int32_t ldm, double* mean, double* sigma, int32_t* m_out, int32_t* status,
+                        int32_t mem);
+
 /* ---- stop predictor ---- */
 typedef struct cngp_stop_config {
   double v_nom;      /* 0.8    gp_predictor.cpp:73-75 */
@@ -217,6 +257,16 @@ int cngp_zupt_lookahead_batch_ex(cngp_ctx* ctx, const double* mean, const double
                                  const double* pos, int32_t per_window, const cngp_stop_config* cfg,
                                  int32_t* triggered, int32_t* i_stop, int32_t* step_stop, double* xy_err,
                                  double* P_final, double* K_final, double* R_final, int32_t mem);
+
+/* cngp_zupt_lookahead_batch_ex (gp_predictor.cpp:58-130, rows a9-a12) for GP_Output of ragged length: mean, sigma
+ * [B][ldm] with m[b] <= ldm points in row b.  The loop of window b runs ratio * m[b] steps (the reference's
+ * slip_i < ratio * mean.size()), so a window that does not trigger reports step_stop = ratio * m[b]; m[b] = 0 gives
+ * triggered = 0.  P_final / K_final / R_final may be NULL as in _batch_ex. */
+int cngp_zupt_lookahead_ragged(cngp_ctx* ctx, const double* mean, const double* sigma, int64_t B, const int32_t* m,
+                               int32_t ldm, const double* P, const double* Q, const double* STM, const double* Hvec,
+                               const double* pos, int32_t per_window, const cngp_stop_config* cfg, int32_t* triggered,
+                               int32_t* i_stop, int32_t* step_stop, double* xy_err, double* P_final, double* K_final,
+                               double* R_final, int32_t mem);
 
 /* The filter's own covariance recursion for B operating points (SURVEY.md 8f row N4): n_steps IMU steps of
  * P <- STM P STM' + Q (CoreNav.cpp:101) with the odometry update's Joseph form every ratio-th step (CoreNav.cpp:226-230)
