@@ -14,6 +14,7 @@
 
 #include "cngp_internal.h"
 #include "gp_fit.cuh"
+#include "gp_fit_toeplitz.cuh"
 #include "gp_grad.cuh"
 #include "gp_var.cuh"
 #include "gp_var32.cuh"
@@ -483,13 +484,37 @@ static void launch_fit_w(const FitArgs& fa, long long nprob, cudaStream_t s) {
   else if (fa.nt <= 18) launch_fit_k<KID, 9, 2>(fa, nprob, s);   // the reference's own window (134 of 149 samples): two CTAs per SM
   else launch_fit_k<KID, FIT_NW_FULL, FIT_T_FULL>(fa, nprob, s);
 }
-static void launch_fit(int kid, const FitArgs& fa, long long nprob, cudaStream_t s) {
+template <int KID>
+static void launch_fit_toeplitz(const FitArgs& fa, long long nprob, cudaStream_t s) {
+  const size_t smem = toep_smem_bytes(fa.nt);
+  cudaFuncSetAttribute(gp_fit_toeplitz_kernel<KID>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  gp_fit_toeplitz_kernel<KID><<<(unsigned)((nprob + TOEP_WARPS - 1) / TOEP_WARPS), TOEP_WARPS * 32, smem, s>>>(fa, nprob);
+}
+// Phase A of a chunk.  With lag tables on and more problems than SMs, gp_fit_toeplitz_kernel first takes the windows
+// whose Ky is Toeplitz (uniform integer stamps) and well conditioned, and marks them in done (slot SLOT_FIT_DONE,
+// [n_problems], merged with fa.skip); gp_fit_kernel then factors the others.  Up to one problem per SM gp_fit_kernel
+// finishes the whole chunk in its single-window time, which is shorter than one warp's Schur recursion (one N = 100
+// window on a B200: 36 us against 89 us); beyond that its waves run one after the other and the Schur path wins
+// (4096 windows of N = 256: 0.57 ms against 2.37 ms).
+enum { SLOT_FIT_DONE = 26 };
+static int launch_fit(cngp_ctx* ctx, int kid, const FitArgs& fa_in, long long n_problems, long long nprob, cudaStream_t s) {
+  FitArgs fa = fa_in;
+  if (fa.lag_ok && kid != KID_RBF_BROWN && nprob > g_sm_count) {
+    fa.done = (int*)ctx->buf(SLOT_FIT_DONE, sizeof(int) * (size_t)n_problems);
+    if (!fa.done) return CNGP_ERR_NOMEM;
+    // the features of KID_RBF are those of the interpreter: only the periodic phases need their own instance
+    if (kid == KID_RBF_PER) launch_fit_toeplitz<KID_RBF_PER>(fa, nprob, s);
+    else launch_fit_toeplitz<KID_GENERIC>(fa, nprob, s);
+    ctx->launches++;
+    fa.skip = fa.done;
+  }
   switch (kid) {
     case KID_RBF: launch_fit_w<KID_RBF>(fa, nprob, s); break;
     case KID_RBF_PER: launch_fit_w<KID_RBF_PER>(fa, nprob, s); break;
     case KID_RBF_BROWN: launch_fit_w<KID_RBF_BROWN>(fa, nprob, s); break;
     default: launch_fit_w<KID_GENERIC>(fa, nprob, s); break;
   }
+  return CNGP_OK;
 }
 
 // every leaf a function of |x - x'| only (White: zero off the diagonal) - what the lag tables of gp_fit.cuh need
@@ -616,8 +641,9 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
     fa.Asrc = nullptr; fa.a_col_stride = 0;
     fa.n_win = n_win;
     ctx->begin(CNGP_PROF_FIT);
-    launch_fit(kid, fa, nw, ctx->stream);
+    rc = launch_fit(ctx, kid, fa, B, nw, ctx->stream);
     ctx->end();
+    if (rc) return fail(ctx, rc, "predict: flag buffer");
     if (M > 0) {
       VarArgs va;
       memset(&va, 0, sizeof va);
@@ -751,8 +777,9 @@ int cngp_lml_grad_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* t
     fa.Asrc = nullptr; fa.a_col_stride = 0;
     fa.n_win = n_win;
     ctx->begin(CNGP_PROF_FIT);
-    launch_fit(match_fast_kernel(kp), fa, np, ctx->stream);
+    rc = launch_fit(ctx, match_fast_kernel(kp), fa, n_prob, np, ctx->stream);
     ctx->end();
+    if (rc) return fail(ctx, rc, "lml_grad: flag buffer");
     if (grad) {
       GradArgs ga;
       ga.kp = kp;

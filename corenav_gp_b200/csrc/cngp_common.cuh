@@ -52,11 +52,15 @@ __device__ __forceinline__ uint32_t to_tf32(float x) {
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
   return r;
 }
-__device__ __forceinline__ void tile_store_split(double* tile, int lane, const tile2& t) {
-  const float a = (float)t.a, b = (float)t.b;
+// the 16 bytes of one entry pair (T[r][2q], T[r][2q+1]), at the place the two doubles would take
+__device__ __forceinline__ void pair_store_split(double* dst, double x0, double x1) {
+  const float a = (float)x0, b = (float)x1;
   const uint32_t ha = to_tf32(a), hb = to_tf32(b);
   const uint32_t la = to_tf32(a - __uint_as_float(ha)), lb = to_tf32(b - __uint_as_float(hb));
-  *reinterpret_cast<uint4*>(reinterpret_cast<char*>(tile) + 16 * lane) = make_uint4(ha, hb, la, lb);
+  *reinterpret_cast<uint4*>(dst) = make_uint4(ha, hb, la, lb);
+}
+__device__ __forceinline__ void tile_store_split(double* tile, int lane, const tile2& t) {
+  pair_store_split(tile + 2 * lane, t.a, t.b);
 }
 
 // Packed lower-triangular tile storage, column-major: column j holds tiles i = j..nt-1 and starts after the

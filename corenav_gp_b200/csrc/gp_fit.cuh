@@ -89,10 +89,87 @@ struct FitArgs {
   // ragged batches: valid training points of each window (n_win[window] <= N, ceil(n_win / 8) == nt); N is then the row
   // stride of x / y only, and the window is identity-padded beyond its own count.  null: every window has N points.
   const int* n_win;
+  int* done;             // [n_problems] gp_fit_toeplitz_kernel only: 1 for the problems it factored (or skipped), else 0
 #ifdef CNGP_FIT_TIMING
   long long* dbg;        // tools/fit_bench.cu: per-warp phase cycle counters of block 0, [warp][8]
 #endif
 };
+
+// Which lag tables a window gets (both false: the lazy evaluators).
+struct LagTab {
+  bool fit_tab;          // K(X,X) by integer lag: every stamp an integer, the span of the training stamps < FIT_TAB_MAX
+  bool var_tab;          // the whole table (training and test lags) for gp_var_kernel
+};
+
+// Lag-table prologue of one window, shared by gp_fit_kernel (NTH = the whole CTA) and gp_fit_toeplitz_kernel (NTH = one
+// warp), so that both write the same table bits and take the same table / lazy decision.  fx: the window's stamps.
+// s_tab: k by lag for the caller's own assembly, or null.  s_xi: training stamps minus the base stamp.  tid 0 writes
+// *s_kdiag (K(x,x), White included) and the window's meta row; the caller syncs before reading them.  For NTH > 32,
+// s_mm [4][NTH / 32] and s_okv [NTH / 32] carry the cross-warp reduction.  The caller counts the window in n_lazy.
+template <int NTH>
+__device__ __forceinline__ LagTab fit_lag_tables(const FitArgs& a, long long lp, int win, int N, int nt, int tid,
+                                                 const double* fx, const KProg* kps, const LeafConst* hc, double noise,
+                                                 double* s_tab, int* s_xi, double* s_kdiag, double* s_mm, int* s_okv) {
+  constexpr int NWARPS = NTH / 32;
+  const int lane = tid & 31, w = tid >> 5;
+  const double big = 67108864.0;   // 2^26: x^2 and x x' stay exact integers, r^2 of the expanded form is exact
+  double xlo = 1e300, xhi = -1e300, slo = 1e300, shi = -1e300;
+  int ok = 1;
+  for (int i = tid; i < N; i += NTH) {
+    const double v = fx[i];
+    ok &= (v == rint(v)) && (fabs(v) < big);
+    xlo = fmin(xlo, v); xhi = fmax(xhi, v);
+  }
+  if (a.xstar) {
+    const double* xs = a.xstar + (a.xstar_stride ? (long long)win * a.xstar_stride : 0);
+    for (int i = tid; i < a.M; i += NTH) {
+      const double v = xs[i];
+      ok &= (v == rint(v)) && (fabs(v) < big);
+      slo = fmin(slo, v); shi = fmax(shi, v);
+    }
+  }
+  for (int o = 16; o; o >>= 1) {
+    xlo = fmin(xlo, __shfl_xor_sync(0xffffffffu, xlo, o)); xhi = fmax(xhi, __shfl_xor_sync(0xffffffffu, xhi, o));
+    slo = fmin(slo, __shfl_xor_sync(0xffffffffu, slo, o)); shi = fmax(shi, __shfl_xor_sync(0xffffffffu, shi, o));
+    ok &= __shfl_xor_sync(0xffffffffu, ok, o);
+  }
+  if (NWARPS > 1) {
+    if (lane == 0) { s_mm[w] = xlo; s_mm[NWARPS + w] = xhi; s_mm[2 * NWARPS + w] = slo; s_mm[3 * NWARPS + w] = shi; s_okv[w] = ok; }
+    __syncthreads();
+    for (int i = 0; i < NWARPS; ++i) {
+      xlo = fmin(xlo, s_mm[i]); xhi = fmax(xhi, s_mm[NWARPS + i]); slo = fmin(slo, s_mm[2 * NWARPS + i]); shi = fmax(shi, s_mm[3 * NWARPS + i]);
+      ok &= s_okv[i];
+    }
+  }
+  const double base = fmin(xlo, slo);
+  const double span = xhi - xlo;                                   // largest lag inside K(X,X)
+  const double dmax = fmax(xhi, shi) - base;                       // largest lag of K(X,X) and K(X,X*)
+  const bool fit_tab = ok && span < (double)FIT_TAB_MAX;
+  const bool var_tab = ok && a.ktab && dmax < (double)VAR_TAB_MAX;
+  if (fit_tab || var_tab) {
+    const int nl = (int)(var_tab ? dmax : span) + 1;
+    double* gt = var_tab ? a.ktab + lp * (long long)VAR_TAB_MAX : nullptr;
+    for (int d = tid; d < nl; d += NTH) {
+      const double v = keval_generic_cross(kps, hc, (double)d, 0.0);
+      if (s_tab && fit_tab && d < FIT_TAB_MAX && (double)d <= span) s_tab[d] = v;
+      if (gt) gt[d] = v;
+    }
+    for (int i = tid; i < nt * 8; i += NTH) {
+      const int xi = i < N ? (int)(fx[i] - base) : 0;
+      s_xi[i] = xi;
+      if (var_tab) a.kxi[lp * (long long)(nt * 8) + i] = xi;
+    }
+    if (tid == 0) *s_kdiag = keval_generic_sym(kps, hc, 0.0, 0.0, true);
+  }
+  if (tid == 0 && a.kmeta) {
+    double* km = a.kmeta + lp * (long long)VAR_META;
+    km[0] = kdiag_eval(*kps, hc, 0.0);
+    km[1] = base;
+    km[2] = noise;
+    km[3] = var_tab ? 1.0 : 0.0;
+  }
+  return LagTab{fit_tab, var_tab};
+}
 
 #ifdef CNGP_FIT_TIMING
 #define FIT_STAMP(ph) do { const long long now_ = clock64(); t_acc[ph] += now_ - t_last; t_last = now_; } while (0)
@@ -174,9 +251,8 @@ __global__ void __launch_bounds__((NW + 1) * 32, NW * T > 18 ? 1 : 2) gp_fit_ker
   __shared__ int s_fail;
   __shared__ double s_tab[KID == KID_TILES ? 1 : FIT_TAB_MAX];   // k by integer lag, lags 0 .. span
   __shared__ int s_xi[KID == KID_TILES ? 2 : NPAD];              // training stamps minus the base stamp
-  __shared__ double s_mm[4][NW + 1];
+  __shared__ double s_mm[4 * (NW + 1)];
   __shared__ int s_okv[NW + 1];
-  __shared__ int s_tabmode;
   __shared__ double s_kdiag;
 
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -217,74 +293,19 @@ __global__ void __launch_bounds__((NW + 1) * 32, NW * T > 18 ? 1 : 2) gp_fit_ker
     if (tid < a.kp.n_leaves) hc[tid] = leaf_prepare(a.kp.leaf_type[tid], th + a.kp.leaf_param[tid]);
     if (tid == 0) kps = a.kp;
   }
-  if (tid == 0) s_tabmode = 0;
   __syncthreads();
 
   // ---- lag table (stationary expression, integer stamps) ----
+  bool tabmode = false;
   if (KID != KID_TILES && a.lag_ok) {
-    const double big = 67108864.0;   // 2^26: x^2 and x x' stay exact integers, r^2 of the expanded form is exact
-    double xlo = 1e300, xhi = -1e300, slo = 1e300, shi = -1e300;
-    int ok = 1;
-    for (int i = tid; i < N; i += FIT_THREADS) {
-      const double v = fx[i];
-      ok &= (v == rint(v)) && (fabs(v) < big);
-      xlo = fmin(xlo, v); xhi = fmax(xhi, v);
-    }
-    if (a.xstar) {
-      const double* xs = a.xstar + (a.xstar_stride ? (long long)win * a.xstar_stride : 0);
-      for (int i = tid; i < a.M; i += FIT_THREADS) {
-        const double v = xs[i];
-        ok &= (v == rint(v)) && (fabs(v) < big);
-        slo = fmin(slo, v); shi = fmax(shi, v);
-      }
-    }
-    for (int o = 16; o; o >>= 1) {
-      xlo = fmin(xlo, __shfl_xor_sync(0xffffffffu, xlo, o)); xhi = fmax(xhi, __shfl_xor_sync(0xffffffffu, xhi, o));
-      slo = fmin(slo, __shfl_xor_sync(0xffffffffu, slo, o)); shi = fmax(shi, __shfl_xor_sync(0xffffffffu, shi, o));
-      ok &= __shfl_xor_sync(0xffffffffu, ok, o);
-    }
-    if (lane == 0) { s_mm[0][w] = xlo; s_mm[1][w] = xhi; s_mm[2][w] = slo; s_mm[3][w] = shi; s_okv[w] = ok; }
-    __syncthreads();
-    for (int i = 0; i <= NW; ++i) {
-      xlo = fmin(xlo, s_mm[0][i]); xhi = fmax(xhi, s_mm[1][i]); slo = fmin(slo, s_mm[2][i]); shi = fmax(shi, s_mm[3][i]);
-      ok &= s_okv[i];
-    }
-    const double base = fmin(xlo, slo);
-    const double span = xhi - xlo;                                   // largest lag inside K(X,X)
-    const double dmax = fmax(xhi, shi) - base;                       // largest lag of K(X,X) and K(X,X*)
-    const bool fit_tab = ok && span < (double)FIT_TAB_MAX;
-    const bool var_tab = ok && a.ktab && dmax < (double)VAR_TAB_MAX;
-    if (fit_tab || var_tab) {
-      const int nl = (int)(var_tab ? dmax : span) + 1;
-      double* gt = var_tab ? a.ktab + lp * (long long)VAR_TAB_MAX : nullptr;
-      for (int d = tid; d < nl; d += FIT_THREADS) {
-        const double v = keval_generic_cross(&kps, hc, (double)d, 0.0);
-        if (fit_tab && d < FIT_TAB_MAX && (double)d <= span) s_tab[d] = v;
-        if (gt) gt[d] = v;
-      }
-      for (int i = tid; i < nt * 8; i += FIT_THREADS) {
-        const int xi = i < N ? (int)(fx[i] - base) : 0;
-        s_xi[i] = xi;
-        if (var_tab) a.kxi[lp * (long long)(nt * 8) + i] = xi;
-      }
-      if (tid == 0) {
-        s_tabmode = fit_tab ? 1 : 0;
-        s_kdiag = keval_generic_sym(&kps, hc, 0.0, 0.0, true);     // K(X,X) diagonal (White included)
-      }
-    }
-    if (tid == 0 && a.kmeta) {
-      double* km = a.kmeta + lp * (long long)VAR_META;
-      km[0] = kdiag_eval(kps, hc, 0.0);
-      km[1] = base;
-      km[2] = noise;
-      km[3] = var_tab ? 1.0 : 0.0;
-      if (!var_tab && a.n_lazy) atomicAdd(a.n_lazy, 1);
-    }
+    const LagTab lt = fit_lag_tables<FIT_THREADS>(a, lp, win, N, nt, tid, fx, &kps, hc, noise, s_tab, s_xi, &s_kdiag,
+                                                  s_mm, s_okv);
+    tabmode = lt.fit_tab;
+    if (tid == 0 && a.kmeta && !lt.var_tab && a.n_lazy) atomicAdd(a.n_lazy, 1);
     __syncthreads();
   } else if (KID != KID_TILES && tid == 0 && a.n_lazy) {
     atomicAdd(a.n_lazy, 1);
   }
-  const bool tabmode = KID != KID_TILES && s_tabmode != 0;
 
   const bool full_window = N == 8 * nt;
   auto feat_at = [&](int i) -> PointFeat {
