@@ -18,6 +18,7 @@
 #include "gp_grad.cuh"
 #include "gp_var.cuh"
 #include "gp_var32.cuh"
+#include "gp_var_toeplitz.cuh"
 
 extern "C" int cngp_launch_lookahead(const double*, const double*, long long, int, const double*, const double*,
                                      const double*, const double*, const double*, int, const cngp_stop_config*, int*,
@@ -517,6 +518,26 @@ static int launch_fit(cngp_ctx* ctx, int kid, const FitArgs& fa_in, long long n_
   return CNGP_OK;
 }
 
+// Phase B of a chunk, first step.  With lag tables on, FP64 and more windows than SMs (the gate of the Schur fit),
+// gp_var_toeplitz_kernel takes the windows whose Ky is Toeplitz and whose test points lie on the training lattice, and
+// marks them in taken (slot SLOT_VAR_TAKEN, [nw]); var_compact_kernel lists the others (slot SLOT_VAR_LIST: count, then
+// the list) for gp_var_kernel.  On one window the warp's recurrence is latency-bound, and gp_var_kernel's single window
+// is spread over a whole SM, so below the gate every window stays on gp_var_kernel.
+enum { SLOT_VAR_TAKEN = 27, SLOT_VAR_LIST = 28 };
+static int launch_var_toeplitz(cngp_ctx* ctx, VarArgs& va, long long nw, cudaStream_t s) {
+  int* taken = (int*)ctx->buf(SLOT_VAR_TAKEN, sizeof(int) * (size_t)nw);
+  int* lst = (int*)ctx->buf(SLOT_VAR_LIST, sizeof(int) * ((size_t)nw + 32));
+  if (!taken || !lst) return CNGP_ERR_NOMEM;
+  const size_t smem = tvt_smem_bytes(va.nt, va.M);
+  cudaFuncSetAttribute(gp_var_toeplitz_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  gp_var_toeplitz_kernel<<<(unsigned)((nw + TVT_WARPS - 1) / TVT_WARPS), TVT_WARPS * 32, smem, s>>>(va, taken);
+  var_compact_kernel<<<1, 1024, 0, s>>>(taken, nw, lst + 32, lst);
+  ctx->launches += 2;
+  va.list = lst + 32;
+  va.list_count = lst;
+  return CNGP_OK;
+}
+
 // every leaf a function of |x - x'| only (White: zero off the diagonal) - what the lag tables of gp_fit.cuh need
 static bool kprog_stationary(const KProg& kp) {
   for (int u = 0; u < kp.n_leaves; ++u)
@@ -657,7 +678,12 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
       va.kstage = nullptr;
       va.n_win = n_win; va.m_win = m_win;
       ctx->begin(CNGP_PROF_VAR);
-      int vrc;
+      int vrc = CNGP_OK;
+      if (!f32 && lag_ok && nw > g_sm_count) vrc = launch_var_toeplitz(ctx, va, nw, ctx->stream);
+      if (vrc) {
+        ctx->end();
+        return fail(ctx, vrc, "predict: flag buffer");
+      }
       if (f32) {
         va.n_lazy = nullptr;
         va.kmeta = lag_ok ? mbuf : nullptr;      // the FP32 kernel picks table or interpreter per window

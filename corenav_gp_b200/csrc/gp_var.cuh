@@ -64,6 +64,10 @@ struct VarArgs {
   // m_win[win] <= M: valid test points - mean / var entries at or beyond it are not written (M stays the row stride).
   const int* n_win;
   const int* m_win;
+  // windows left by gp_var_toeplitz_kernel (null: every window of the launch): local windows list[0 .. *list_count) in
+  // increasing order, in place of 0 .. n_windows_launch-1
+  const int* list;
+  const int* list_count;
 };
 
 struct VarGroupShared {
@@ -72,6 +76,7 @@ struct VarGroupShared {
   int ce_max, nchunks, nrounds, n_tiles, ct;
   long long unit0, n_units, unit_stride;
   const double* Lbase;
+  const int* list;
   uint32_t ring_u32, full_u32;
 };
 
@@ -83,7 +88,7 @@ static __device__ __noinline__ void var_issue_chunk(const VarGroupShared* sh, in
   const int ce = sh->ce_max - (gc - k * sh->nchunks);
   const long long u = sh->unit0 + (long long)k * sh->unit_stride;
   if (u >= sh->n_units) return;
-  const long long lw = u / sh->nrounds;
+  const long long lw = sh->list ? sh->list[u / sh->nrounds] : u / sh->nrounds;
   const int ct = sh->ct;
   const double* src = sh->Lbase + (lw + 1) * (long long)sh->n_tiles * 64 - (long long)(ct * ce + ct) * 64;
   mbar_expect_tx(sh->full_u32 + 8 * slot, ct * 512);
@@ -96,6 +101,8 @@ static __device__ __noinline__ void var_issue_chunk(const VarGroupShared* sh, in
 template <int NT_MAX, int G, int WG, int NSLOT, int VAR_CT, int KID, bool FULL, bool TAB = false>
 __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a) {
   if (a.n_lazy && ((*a.n_lazy == 0) != TAB)) return;
+  const long long n_windows = a.list ? (long long)*a.list_count : a.n_windows_launch;
+  if (n_windows == 0) return;
   static_assert(NSLOT <= VAR_MAX_SLOTS && VAR_CT <= VAR_MAX_CT, "ring too deep / chunk too large");
   constexpr int WARPS = G * WG;
   constexpr int VAR_CHUNK_DOUBLES = VAR_CT * 64;
@@ -112,7 +119,7 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
   const int ce_max = (n_tiles - 1) / VAR_CT;      // chunk ids count from the END of a window's factor
   const int nchunks = ce_max + 1;
   const int nrounds = (mt - a.mt0 + WG - 1) / WG;
-  const long long n_units = a.n_windows_launch * nrounds;
+  const long long n_units = n_windows * nrounds;
   const long long unit_stride = (long long)gridDim.x * G;
   const long long unit0 = (long long)blockIdx.x * G + grp;
 
@@ -128,7 +135,7 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
     for (int s = 0; s < NSLOT; ++s) { mbar_init(full_u32 + 8 * s, 1); mbar_init(empty_u32 + 8 * s, WG); }
     sh.ce_max = ce_max; sh.nchunks = nchunks; sh.nrounds = nrounds; sh.n_tiles = n_tiles; sh.ct = VAR_CT;
     sh.unit0 = unit0; sh.n_units = n_units; sh.unit_stride = unit_stride;
-    sh.Lbase = a.L; sh.ring_u32 = ring_u32; sh.full_u32 = full_u32;
+    sh.Lbase = a.L; sh.list = a.list; sh.ring_u32 = ring_u32; sh.full_u32 = full_u32;
     mbar_fence_init();
     for (int s = 0; s < NSLOT; ++s) var_issue_chunk(&sh, s, s);   // chunk g of the group goes to slot g % NSLOT
   }
@@ -139,8 +146,9 @@ __global__ void __launch_bounds__(G * WG * 32, 1) gp_var_kernel(const VarArgs a)
   int g = 0;   // chunk counter of this warp within its group's stream (over units x chunks)
 
   for (long long u = unit0; u < n_units; u += unit_stride) {
-    const long long lw = u / nrounds;                 // window within this launch
-    const int round = (int)(u - lw * nrounds);
+    const long long ui = u / nrounds;
+    const long long lw = a.list ? a.list[ui] : ui;    // window within this launch
+    const int round = (int)(u - ui * nrounds);
     const long long win = a.window0 + lw;
     const double* th = a.theta + (a.theta_mode == 0 ? 0 : win) * a.theta_stride;
     const int m8 = a.mt0 + round * WG + wg;

@@ -83,7 +83,7 @@ __global__ void __launch_bounds__(WG * 32, 1) gp_var32_kernel(const VarArgs a) {
     for (int s = 0; s < NSLOT; ++s) { mbar_init(full_u32 + 8 * s, 1); mbar_init(empty_u32 + 8 * s, WG); }
     sh.ce_max = ce_max; sh.nchunks = nchunks; sh.nrounds = nrounds; sh.n_tiles = n_tiles; sh.ct = VAR_CT;
     sh.unit0 = unit0; sh.n_units = n_units; sh.unit_stride = unit_stride;
-    sh.Lbase = a.L; sh.ring_u32 = ring_u32; sh.full_u32 = full_u32;
+    sh.Lbase = a.L; sh.list = nullptr; sh.ring_u32 = ring_u32; sh.full_u32 = full_u32;   // every window of the launch
     mbar_fence_init();
     for (int s = 0; s < NSLOT; ++s) var_issue_chunk(&sh, s, s);
   }

@@ -1,0 +1,44 @@
+"""Roofline figures of gp_var_toeplitz_kernel (DESIGN.md section 4.2c), from the shapes and a measured phase time.
+
+bench.py's roofline block still counts the N^2 M flop of gp_var_kernel's forward substitution, which the recurrence does
+not do; its `achieved` and `frac` are no longer a share of anything.  The two honest bounds of the recurrence are:
+  - HBM: the packed factor (tiles_in_lower(nt) * 512 bytes per window) is read once by the back substitution;
+  - FP64 pipe: 4 FMA per factor entry pair and right-hand side of the back substitution, 3 n FMA per chain point.
+Usage: python tools/var_toeplitz_roofline.py --ms <variance phase ms> [--B 4096 --N 256 --M 600]
+       [--hbm-tbs 7.7] [--fp64-tflops 33.9]   (data-sheet HBM bandwidth; DFMA issue peak of profiles/fp64_peak_r01.json)"""
+import argparse
+import json
+
+
+def figures(B, N, M, ms, hbm_tbs, fp64_tflops):
+    nt = (N + 7) // 8
+    tiles = nt * (nt + 1) // 2
+    factor_bytes = tiles * 512 * B
+    chain = M + 1 if M > 0 else 0                 # the benchmark grid x_{N-1} + 1 + j: chain from m0 = N - 1
+    fma_back = tiles * 64 * 2 * B                 # two right-hand sides, one FMA per factor entry each
+    fma_chain = 3 * N * chain * B
+    fma = fma_back + fma_chain
+    t = ms * 1e-3
+    return {
+        "B": B, "N": N, "M": M, "phase_ms": ms,
+        "factor_bytes": factor_bytes, "hbm_tb_per_s": factor_bytes / t * 1e-12,
+        "hbm_frac": factor_bytes / t * 1e-12 / hbm_tbs,
+        "fma": fma, "fp64_tflops": 2 * fma / t * 1e-12, "fp64_frac": 2 * fma / t * 1e-12 / fp64_tflops,
+        "lower_bound_ms": 1e3 * max(factor_bytes / (hbm_tbs * 1e12), 2 * fma / (fp64_tflops * 1e12)),
+    }
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--ms", type=float, required=True)
+    ap.add_argument("--B", type=int, default=4096)
+    ap.add_argument("--N", type=int, default=256)
+    ap.add_argument("--M", type=int, default=600)
+    ap.add_argument("--hbm-tbs", type=float, default=7.7)
+    ap.add_argument("--fp64-tflops", type=float, default=33.9)
+    a = ap.parse_args()
+    print(json.dumps(figures(a.B, a.N, a.M, a.ms, a.hbm_tbs, a.fp64_tflops), indent=1))
+
+
+if __name__ == "__main__":
+    main()
