@@ -16,6 +16,7 @@
 #include "gp_fit.cuh"
 #include "gp_fit_toeplitz.cuh"
 #include "gp_grad.cuh"
+#include "gp_toep_group.cuh"
 #include "gp_var.cuh"
 #include "gp_var32.cuh"
 #include "gp_var_toeplitz.cuh"
@@ -538,6 +539,65 @@ static int launch_var_toeplitz(cngp_ctx* ctx, VarArgs& va, long long nw, cudaStr
   return CNGP_OK;
 }
 
+// Shared covariance (gp_toep_group.cuh, DESIGN.md section 4.2d).  Under the gate of the Toeplitz kernels and with one
+// theta for the whole call, the chunk's largest group of windows with the same key is factored once: the key and group
+// kernels, the one-window Schur fit into a slot of its own (slot SLOT_TG_DATA: factor | z | L_jj | table | meta |
+// integer stamps | variance row | mean row | log det) and the member kernel, which clears flag (slot SLOT_TG_FLAG,
+// [n_windows]) for whatever goes back to the per-window kernels.  Those then run with flag as their skip list.
+enum { SLOT_TG_KEY = 29, SLOT_TG_FLAG = 30, SLOT_TG_LIST = 31, SLOT_TG_REC = 32, SLOT_TG_DATA = 33 };
+struct TGroup {
+  int* flag = nullptr;
+  int* list = nullptr;
+  int* rec = nullptr;
+  double* gvar = nullptr;
+};
+static int launch_toep_group(cngp_ctx* ctx, const FitArgs& fa, const VarArgs& va, const int* m_win, long long B,
+                             long long nw, TGroup& tg, cudaStream_t s) {
+  const int nt = fa.nt, R = 8 * nt, M = fa.M;
+  int4* key = (int4*)ctx->buf(SLOT_TG_KEY, sizeof(int4) * (size_t)nw);
+  tg.flag = (int*)ctx->buf(SLOT_TG_FLAG, sizeof(int) * (size_t)B);
+  tg.list = (int*)ctx->buf(SLOT_TG_LIST, sizeof(int) * (size_t)nw);
+  tg.rec = (int*)ctx->buf(SLOT_TG_REC, sizeof(int) * TG_INTS);
+  const size_t nd = (size_t)tiles_in_lower(nt) * 64 + R + (size_t)nt * 64 + VAR_TAB_MAX + VAR_META + R / 2 + 2 * (size_t)M + 1;
+  double* gd = (double*)ctx->buf(SLOT_TG_DATA, sizeof(double) * nd);
+  if (!key || !tg.flag || !tg.list || !tg.rec || !gd) return CNGP_ERR_NOMEM;
+  double* gL = gd;
+  double* gz = gL + (size_t)tiles_in_lower(nt) * 64;
+  double* gdiag = gz + R;
+  double* gtab = gdiag + (size_t)nt * 64;
+  double* gmeta = gtab + VAR_TAB_MAX;
+  int* gxi = (int*)(gmeta + VAR_META);
+  tg.gvar = gmeta + VAR_META + R / 2;
+  double* gmean = tg.gvar + M;
+  double* glogdet = gmean + M;
+
+  toep_key_kernel<<<(unsigned)((nw + TG_KEY_WARPS - 1) / TG_KEY_WARPS), TG_KEY_WARPS * 32, 0, s>>>(fa, m_win, nw, key);
+  toep_group_kernel<<<1, 1024, 0, s>>>(key, nw, fa.problem0, tg.flag, tg.list, tg.rec);
+  // the one-window fit: the first member's stamps, y = 0
+  FitArgs g = fa;
+  g.problem0 = 0; g.win_map = tg.rec + TG_REP; g.skip = tg.rec + TG_NONE; g.theta_mode = 0;
+  g.y = nullptr; g.L = gL; g.z = gz; g.feat = nullptr; g.lml = nullptr; g.logdet = glogdet; g.quad = nullptr;
+  g.status = nullptr; g.ktab = gtab; g.kmeta = gmeta; g.kxi = gxi; g.n_lazy = nullptr; g.done = tg.rec + TG_FIT;
+  g.ldiag = gdiag; g.f32_factor = 0;
+  launch_fit_toeplitz<KID_GENERIC>(g, 1, s);
+  ctx->launches += 2;   // + the begin() below that re-opens the fit span
+  ctx->end();
+  ctx->begin(CNGP_PROF_VAR);
+  TGArgs t;
+  memset(&t, 0, sizeof t);
+  t.g = va;
+  t.g.L = gL; t.g.z = gz; t.g.ktab = gtab; t.g.kmeta = gmeta; t.g.kxi = gxi; t.g.status = nullptr;
+  t.ldiag = gdiag; t.logdet = glogdet; t.gvar = tg.gvar; t.gmean = gmean;
+  t.y = fa.y; t.lml = fa.lml; t.status = fa.status; t.mean = va.mean; t.flag = tg.flag; t.list = tg.list; t.rec = tg.rec;
+  t.w0 = fa.problem0;
+  const size_t smem = tg_smem_bytes(nt, M);
+  cudaFuncSetAttribute(gp_toep_member_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  gp_toep_member_kernel<<<(unsigned)(1 + (nw + TG_WARPS - 1) / TG_WARPS), TG_WARPS * 32, smem, s>>>(t);
+  ctx->end();
+  ctx->begin(CNGP_PROF_FIT);
+  return CNGP_OK;
+}
+
 // every leaf a function of |x - x'| only (White: zero off the diagonal) - what the lag tables of gp_fit.cuh need
 static bool kprog_stationary(const KProg& kp) {
   for (int u = 0; u < kp.n_leaves; ++u)
@@ -661,13 +721,14 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
     fa.jitter_retry = ctx->cfg.jitter_retry;
     fa.Asrc = nullptr; fa.a_col_stride = 0;
     fa.n_win = n_win;
+    VarArgs va;
+    memset(&va, 0, sizeof va);
+    // the gate of the Toeplitz kernels (launch_fit, launch_var_toeplitz), one theta for the call
+    const bool toep = !f32 && lag_ok && nw > g_sm_count && M > 0;
+    const bool grouped = toep && theta_stride == 0;
+    TGroup tg;
     ctx->begin(CNGP_PROF_FIT);
-    rc = launch_fit(ctx, kid, fa, B, nw, ctx->stream);
-    ctx->end();
-    if (rc) return fail(ctx, rc, "predict: flag buffer");
     if (M > 0) {
-      VarArgs va;
-      memset(&va, 0, sizeof va);
       va.kp = kp;
       va.ktab = tbuf; va.kmeta = mbuf; va.kxi = xibuf; va.n_lazy = lag_ok ? d_nlazy : nullptr;
       va.theta = d_theta; va.theta_stride = theta_stride; va.theta_mode = theta_stride ? 1 : 0;
@@ -677,9 +738,23 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
       va.sigma_mode = sigma_mode;
       va.kstage = nullptr;
       va.n_win = n_win; va.m_win = m_win;
+    }
+    if (grouped) {
+      rc = launch_toep_group(ctx, fa, va, m_win, B, nw, tg, ctx->stream);
+      if (rc) {
+        ctx->end();
+        return fail(ctx, rc, "predict: shared-covariance buffers");
+      }
+      fa.skip = tg.flag;
+      va.skip = tg.flag;
+    }
+    rc = launch_fit(ctx, kid, fa, B, nw, ctx->stream);
+    ctx->end();
+    if (rc) return fail(ctx, rc, "predict: flag buffer");
+    if (M > 0) {
       ctx->begin(CNGP_PROF_VAR);
       int vrc = CNGP_OK;
-      if (!f32 && lag_ok && nw > g_sm_count) vrc = launch_var_toeplitz(ctx, va, nw, ctx->stream);
+      if (toep) vrc = launch_var_toeplitz(ctx, va, nw, ctx->stream);
       if (vrc) {
         ctx->end();
         return fail(ctx, vrc, "predict: flag buffer");
@@ -710,6 +785,11 @@ int cngp_predict_impl(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
         if (!vrc) vrc = launch_var<32, 4, 3, 3, 16>(ctx, kid, va, nw, ctx->stream);
       }
       else vrc = launch_var<32, 1, 12, 3, 64>(ctx, kid, va, nw, ctx->stream);
+      if (grouped && !vrc) {
+        toep_var_broadcast_kernel<<<(unsigned)((nw + 3) / 4), 128, 0, ctx->stream>>>(tg.list, tg.rec, tg.flag, tg.gvar, d_var,
+                                                                                     w0, M);
+        ctx->launches++;
+      }
       ctx->end();
       if (vrc) return fail(ctx, vrc, "predict: staging buffer for the generic kernel path");
     }

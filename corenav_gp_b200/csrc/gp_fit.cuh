@@ -90,6 +90,8 @@ struct FitArgs {
   // stride of x / y only, and the window is identity-padded beyond its own count.  null: every window has N points.
   const int* n_win;
   int* done;             // [n_problems] gp_fit_toeplitz_kernel only: 1 for the problems it factored (or skipped), else 0
+  double* ldiag;         // gp_fit_toeplitz_kernel only, or null: [nt][64] the diagonal tiles L_jj themselves (row-major) of
+                         // problem 0 of the launch - the one-window fit of a shared covariance (gp_toep_group.cuh)
 #ifdef CNGP_FIT_TIMING
   long long* dbg;        // tools/fit_bench.cu: per-warp phase cycle counters of block 0, [warp][8]
 #endif
@@ -101,18 +103,22 @@ struct LagTab {
   bool var_tab;          // the whole table (training and test lags) for gp_var_kernel
 };
 
-// Lag-table prologue of one window, shared by gp_fit_kernel (NTH = the whole CTA) and gp_fit_toeplitz_kernel (NTH = one
-// warp), so that both write the same table bits and take the same table / lazy decision.  fx: the window's stamps.
-// s_tab: k by lag for the caller's own assembly, or null.  s_xi: training stamps minus the base stamp.  tid 0 writes
-// *s_kdiag (K(x,x), White included) and the window's meta row; the caller syncs before reading them.  For NTH > 32,
-// s_mm [4][NTH / 32] and s_okv [NTH / 32] carry the cross-warp reduction.  The caller counts the window in n_lazy.
+// Stamp extent of one window, the part of the lag-table decision that writes nothing: every training stamp and every
+// one of the M test stamps an integer with |x| < 2^26 (x^2 and x x' stay exact integers, r^2 of the expanded form is
+// exact), the base stamp, the span of the training stamps and the largest lag of K(X,X) and K(X,X*).  fit_lag_tables
+// and the shared-covariance qualification (gp_toep_group.cuh) both decide from it.
+struct LagExtent {
+  bool ok;
+  double base, span, dmax;
+  __device__ __forceinline__ bool fit_tab() const { return ok && span < (double)FIT_TAB_MAX; }
+  __device__ __forceinline__ bool var_tab() const { return ok && dmax < (double)VAR_TAB_MAX; }
+};
 template <int NTH>
-__device__ __forceinline__ LagTab fit_lag_tables(const FitArgs& a, long long lp, int win, int N, int nt, int tid,
-                                                 const double* fx, const KProg* kps, const LeafConst* hc, double noise,
-                                                 double* s_tab, int* s_xi, double* s_kdiag, double* s_mm, int* s_okv) {
+__device__ __forceinline__ LagExtent lag_extent(const FitArgs& a, int win, int N, int tid, const double* fx, double* s_mm,
+                                                int* s_okv) {
   constexpr int NWARPS = NTH / 32;
   const int lane = tid & 31, w = tid >> 5;
-  const double big = 67108864.0;   // 2^26: x^2 and x x' stay exact integers, r^2 of the expanded form is exact
+  const double big = 67108864.0;   // 2^26
   double xlo = 1e300, xhi = -1e300, slo = 1e300, shi = -1e300;
   int ok = 1;
   for (int i = tid; i < N; i += NTH) {
@@ -142,10 +148,22 @@ __device__ __forceinline__ LagTab fit_lag_tables(const FitArgs& a, long long lp,
     }
   }
   const double base = fmin(xlo, slo);
-  const double span = xhi - xlo;                                   // largest lag inside K(X,X)
-  const double dmax = fmax(xhi, shi) - base;                       // largest lag of K(X,X) and K(X,X*)
-  const bool fit_tab = ok && span < (double)FIT_TAB_MAX;
-  const bool var_tab = ok && a.ktab && dmax < (double)VAR_TAB_MAX;
+  return LagExtent{ok != 0, base, xhi - xlo, fmax(xhi, shi) - base};   // span: largest lag inside K(X,X)
+}
+
+// Lag-table prologue of one window, shared by gp_fit_kernel (NTH = the whole CTA) and gp_fit_toeplitz_kernel (NTH = one
+// warp), so that both write the same table bits and take the same table / lazy decision.  fx: the window's stamps.
+// s_tab: k by lag for the caller's own assembly, or null.  s_xi: training stamps minus the base stamp.  tid 0 writes
+// *s_kdiag (K(x,x), White included) and the window's meta row; the caller syncs before reading them.  For NTH > 32,
+// s_mm [4][NTH / 32] and s_okv [NTH / 32] carry the cross-warp reduction.  The caller counts the window in n_lazy.
+template <int NTH>
+__device__ __forceinline__ LagTab fit_lag_tables(const FitArgs& a, long long lp, int win, int N, int nt, int tid,
+                                                 const double* fx, const KProg* kps, const LeafConst* hc, double noise,
+                                                 double* s_tab, int* s_xi, double* s_kdiag, double* s_mm, int* s_okv) {
+  const LagExtent ex = lag_extent<NTH>(a, win, N, tid, fx, s_mm, s_okv);
+  const double base = ex.base, span = ex.span, dmax = ex.dmax;
+  const bool fit_tab = ex.fit_tab();
+  const bool var_tab = a.ktab && ex.var_tab();
   if (fit_tab || var_tab) {
     const int nl = (int)(var_tab ? dmax : span) + 1;
     double* gt = var_tab ? a.ktab + lp * (long long)VAR_TAB_MAX : nullptr;

@@ -37,6 +37,29 @@ constexpr double TOEP_MIN_PIVOT2 = 1e-2;
 __host__ __device__ __forceinline__ int toep_col_stride(int nt) { return (8 * nt + 31) & ~31; }
 __host__ __device__ __forceinline__ size_t toep_smem_bytes(int nt) { return (size_t)TOEP_WARPS * 4 * toep_col_stride(nt) * sizeof(double); }
 
+// Uniform stamps x_i = x_0 + i d with d >= 1, from the integer stamps xi[0 .. n) (this lane's share of the check; the
+// caller takes the warp vote).  n < 2 passes with d = 1.
+__device__ __forceinline__ bool toep_uniform(const int* xi, int n, int lane, int& d) {
+  d = 1;
+  if (n < 2) return true;
+  d = xi[1] - xi[0];
+  bool ok = d >= 1;
+  for (int i = lane; i < n; i += 32) ok &= (xi[i] - xi[0] == i * d);
+  return ok;
+}
+// z'z of the warp's rows (sequential over the slots, then the xor tree) and the LML: the Schur fit and the members of a
+// shared covariance (gp_toep_group.cuh) compute them here, so both give the same bits
+__device__ __forceinline__ double toep_quad(const double (&rr)[TOEP_SLOTS]) {
+  double qs = 0.0;
+#pragma unroll
+  for (int s = 0; s < TOEP_SLOTS; ++s) qs += rr[s] * rr[s];
+  for (int o = 16; o; o >>= 1) qs += __shfl_xor_sync(0xffffffffu, qs, o);
+  return qs;
+}
+__device__ __forceinline__ double toep_lml(int N, double logdet, double qs) {
+  return 0.5 * (-(double)N * CNGP_LOG_2PI - logdet - qs);
+}
+
 // KID only selects the per-point features written for phase B (the periodic phases for KID_RBF_PER); the factorisation
 // itself reads the lag table, built by the interpreter for every expression.
 template <int KID>
@@ -97,13 +120,8 @@ __global__ void __launch_bounds__(TOEP_WARPS * 32, 4) gp_fit_toeplitz_kernel(con
   __syncwarp();
 
   // ---- uniform stamps: x_i = x_0 + i d ----
-  bool ok = lt.fit_tab;
   int d = 1;
-  if (ok && N > 1) {
-    d = s_xi[1] - s_xi[0];
-    for (int i = lane; i < N; i += 32) ok &= (s_xi[i] - s_xi[0] == i * d);
-    ok &= d >= 1;
-  }
+  const bool ok = lt.fit_tab && toep_uniform(s_xi, N, lane, d);
   if (!__all_sync(0xffffffffu, ok)) {
     if (lane == 0) a.done[p] = 0;
     return;
@@ -122,7 +140,7 @@ __global__ void __launch_bounds__(TOEP_WARPS * 32, 4) gp_fit_toeplitz_kernel(con
     else if (i < N) ui = keval_generic_cross(&kps, hc, (double)(i * d), 0.0) * ipiv;
     u[s] = ui;
     v[s] = i == 0 ? 0.0 : ui;
-    rr[s] = i < N ? a.y[(long long)win * ld + i] : 0.0;   // residual y - L z, row k becomes z_k at step k
+    rr[s] = (i < N && a.y) ? a.y[(long long)win * ld + i] : 0.0;   // residual y - L z (y = 0 without y), row k becomes z_k at step k
     pv[s] = 1.0;                                          // pivots (1 on the padding rows)
   }
   bool good = true;
@@ -212,6 +230,10 @@ __global__ void __launch_bounds__(TOEP_WARPS * 32, 4) gp_fit_toeplitz_kernel(con
         double* dst = Lp + (long long)tile_index(J, J, nt) * 64;
         if (f32) tile_store_split(dst, lane, x);
         else tile_store(dst, lane, x);
+        if (a.ldiag) {
+          a.ldiag[J * 64 + lane] = dtile[lane];
+          a.ldiag[J * 64 + 32 + lane] = dtile[32 + lane];
+        }
         __syncwarp();
       }
     }
@@ -233,12 +255,11 @@ __global__ void __launch_bounds__(TOEP_WARPS * 32, 4) gp_fit_toeplitz_kernel(con
   if (R > 224) block(FitIC<7>{});
 
   // ---- accept or hand the window to gp_fit_kernel ----
-  double qs = 0.0, hl = 0.0;
+  double hl = 0.0;
   bool fin = isfinite(piv) && isfinite(ipiv);
 #pragma unroll
   for (int s = 0; s < TOEP_SLOTS; ++s) {
     fin &= isfinite(rr[s]) && isfinite(pv[s]);
-    qs += rr[s] * rr[s];
     hl += log(pv[s]);   // padded rows have pivot 1
   }
   good = good && fin && minp2 >= TOEP_MIN_PIVOT2 * t0;
@@ -250,15 +271,13 @@ __global__ void __launch_bounds__(TOEP_WARPS * 32, 4) gp_fit_toeplitz_kernel(con
 #pragma unroll
   for (int s = 0; s < TOEP_SLOTS; ++s)
     if (lane + 32 * s < R) zp[lane + 32 * s] = rr[s];
-  for (int o = 16; o; o >>= 1) {
-    qs += __shfl_xor_sync(0xffffffffu, qs, o);
-    hl += __shfl_xor_sync(0xffffffffu, hl, o);
-  }
+  const double qs = toep_quad(rr);
+  for (int o = 16; o; o >>= 1) hl += __shfl_xor_sync(0xffffffffu, hl, o);
   if (lane == 0) {
     const double logdet = 2.0 * hl;
     if (a.quad) a.quad[p] = qs;
     if (a.logdet) a.logdet[p] = logdet;
-    if (a.lml) a.lml[p] = 0.5 * (-(double)N * CNGP_LOG_2PI - logdet - qs);
+    if (a.lml) a.lml[p] = toep_lml(N, logdet, qs);
     if (a.status) a.status[p] = 0;
     if (a.kmeta && !lt.var_tab && a.n_lazy) atomicAdd(a.n_lazy, 1);
     a.done[p] = 1;

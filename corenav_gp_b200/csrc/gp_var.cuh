@@ -68,6 +68,9 @@ struct VarArgs {
   // increasing order, in place of 0 .. n_windows_launch-1
   const int* list;
   const int* list_count;
+  // gp_var_toeplitz_kernel only, or null: [n_windows] windows whose results come from gp_toep_member_kernel (members of a
+  // shared covariance, gp_toep_group.cuh) - marked taken and left untouched
+  const int* skip;
 };
 
 struct VarGroupShared {

@@ -43,50 +43,35 @@ __host__ __device__ __forceinline__ int tvt_tab_cap(int nt, int M) {
 __host__ __device__ __forceinline__ int tvt_warp_doubles(int nt, int M) { return 3 * (8 * nt + TVT_P) + tvt_tab_cap(nt, M); }
 __host__ __device__ __forceinline__ size_t tvt_smem_bytes(int nt, int M) { return (size_t)TVT_WARPS * tvt_warp_doubles(nt, M) * sizeof(double); }
 
-__global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(const VarArgs a, int* taken) {
-  extern __shared__ __align__(16) double tvt_smem[];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const long long lw = (long long)blockIdx.x * TVT_WARPS + w;   // window within this launch
-  if (lw >= a.n_windows_launch) return;
-  const long long win = a.window0 + lw;
-  const int nt = a.nt, R = 8 * nt, M = a.M;
-  const int cap = tvt_tab_cap(nt, M);
-  double* s_al = tvt_smem + (size_t)w * tvt_warp_doubles(nt, M);
-  double* s_a = s_al + R + TVT_P;
-  double* s_t = s_a + R + TVT_P;
-  double* s_tab = s_t + R + TVT_P;
+// Test points x_0 + (m_s + j) d, j < mc, consecutive on the lattice of the stamps (m_s >= 0): this lane's share of the
+// check (the caller takes the warp vote).  base: the window's base stamp, xi0 = x_0 - base.
+__device__ __forceinline__ bool tvt_lattice(const double* xs, double base, int xi0, int d, int mc, int lane, int& ms) {
+  const int mi0 = (int)(xs[0] - base) - xi0;   // offset of the first test point from x_0, in stamp units
+  bool ok = mi0 >= 0 && mi0 % d == 0;
+  ms = ok ? mi0 / d : 0;
+  for (int j = lane; ok && j < mc; j += 32) ok = (int)(xs[j] - base) - xi0 == mi0 + j * d;
+  return ok;
+}
+// The chain of a window with n training points and the test grid m_s .. m_s + mc - 1: chain points m0 .. mend, the
+// passes over them and the table entries the passes read
+struct TvtShape {
+  int m0, mend, passes, need;
+  __device__ __forceinline__ TvtShape(int n, int ms, int mc) {
+    m0 = ms >= n - 1 ? n - 1 : 0;
+    mend = ms + mc - 1;
+    passes = (mend - m0 + 1 + 32 * TVT_P - 1) / (32 * TVT_P);
+    need = TVT_P + n - 1 + passes * 32 * TVT_P;
+  }
+};
+
+// [alpha, w] = L^-T [z, e_{n-1} / L_{n-1,n-1}] by one back substitution over the stored factor Lp, tile column
+// J = nt-1 .. 0, into s_al (and, with W, s_t).  W also returns max_k inv(L)_kk^2 over k < n (the conditioning guard).
+// Without W the alpha half is the same arithmetic, so alpha has the same bits either way.
+template <bool W>
+__device__ __forceinline__ double tvt_backsub(const double* Lp, const double* zp, int n, int nt, int lane, double* s_al,
+                                              double* s_t) {
   const unsigned FULL = 0xffffffffu;
-
-  // ---- the window's own qualification (no factor read yet) ----
-  const double* km = a.kmeta + lw * (long long)VAR_META;
-  const int* xi = a.kxi + lw * (long long)R;
-  const int n = a.n_win ? a.n_win[win] : a.N;
-  const int mc = a.m_win ? a.m_win[win] : M;
-  bool ok = km[3] != 0.0 && n >= 2 && mc >= 1 && !(a.status && a.status[win] != 0);
-  int d = 1, ms = 0;
-  if (ok) {
-    d = xi[1] - xi[0];
-    ok = d >= 1;
-    for (int i = lane; ok && i < n; i += 32) ok = xi[i] - xi[0] == i * d;
-    const double* xs = a.xstar + (a.xstar_stride ? win * a.xstar_stride : 0);
-    const int mi0 = (int)(xs[0] - km[1]) - xi[0];   // offset of the first test point from x_0, in stamp units
-    ok = ok && mi0 >= 0 && mi0 % d == 0;
-    ms = ok ? mi0 / d : 0;
-    for (int j = lane; ok && j < mc; j += 32) ok = (int)(xs[j] - km[1]) - xi[0] == mi0 + j * d;
-  }
-  const int m0 = ms >= n - 1 ? n - 1 : 0, mend = ms + mc - 1;
-  const int C = mend - m0 + 1, passes = (C + 32 * TVT_P - 1) / (32 * TVT_P);
-  const int need = TVT_P + n - 1 + passes * 32 * TVT_P;   // table entries the passes read
-  ok = ok && need <= cap;
-  if (!__all_sync(FULL, ok)) {
-    if (lane == 0) taken[lw] = 0;
-    return;
-  }
-
-  // ---- [alpha, w] = L^-T [z, e_{n-1} / L_{n-1,n-1}], tile column J = nt-1 .. 0 ----
   const int r = lane >> 2, q = lane & 3;
-  const double* Lp = a.L + lw * (long long)tiles_in_lower(nt) * 64;
-  const double* zp = a.z + lw * (long long)R;
   double inv_last = 0.0, maxinv2 = 0.0;
   for (int J = nt - 1; J >= 0; --J) {
     const double* col = Lp + (long long)tile_index(J, J, nt) * 64 + 2 * lane;
@@ -95,84 +80,81 @@ __global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(cons
 #pragma unroll 8
     for (int I = J + 1; I < nt; ++I) {
       const double2 l = *reinterpret_cast<const double2*>(col + (I - J) * 64);
-      const double xa = s_al[8 * I + r], xw = s_t[8 * I + r];
+      const double xa = s_al[8 * I + r];
       c0a = fma(l.x, xa, c0a); c0b = fma(l.y, xa, c0b);
-      c1a = fma(l.x, xw, c1a); c1b = fma(l.y, xw, c1b);
+      if (W) {
+        const double xw = s_t[8 * I + r];
+        c1a = fma(l.x, xw, c1a); c1b = fma(l.y, xw, c1b);
+      }
     }
     // rows of the diagonal tile: pivots of the guard, 1 / L_{n-1,n-1}
     const int row = 8 * J + r;
     const double dv = (r == 2 * q) ? dg.x : (r == 2 * q + 1 ? dg.y : 0.0);
-    if ((r >> 1) == q && row < n) maxinv2 = fmax(maxinv2, dv * dv);
-    if (J == nt - 1) {
-      const int kl = (n - 1) & 7;   // n-1 lies in the last tile column
-      inv_last = __shfl_sync(FULL, dv, 4 * kl + (kl >> 1));
+    if (W) {
+      if ((r >> 1) == q && row < n) maxinv2 = fmax(maxinv2, dv * dv);
+      if (J == nt - 1) {
+        const int kl = (n - 1) & 7;   // n-1 lies in the last tile column
+        inv_last = __shfl_sync(FULL, dv, 4 * kl + (kl >> 1));
+      }
     }
     for (int o = 4; o < 32; o <<= 1) {
       c0a += __shfl_xor_sync(FULL, c0a, o); c0b += __shfl_xor_sync(FULL, c0b, o);
-      c1a += __shfl_xor_sync(FULL, c1a, o); c1b += __shfl_xor_sync(FULL, c1b, o);
+      if (W) { c1a += __shfl_xor_sync(FULL, c1a, o); c1b += __shfl_xor_sync(FULL, c1b, o); }
     }
     // right-hand sides of rows 8J + 2q (+1), then gathered to row r = lane >> 2
     const int ca = 8 * J + 2 * q;
     const double2 zz = *reinterpret_cast<const double2*>(zp + ca);
     const double b0a = zz.x - c0a, b0b = zz.y - c0b;
-    const double b1a = (ca == n - 1 ? inv_last : 0.0) - c1a, b1b = (ca + 1 == n - 1 ? inv_last : 0.0) - c1b;
     const double g0a = __shfl_sync(FULL, b0a, r >> 1), g0b = __shfl_sync(FULL, b0b, r >> 1);
-    const double g1a = __shfl_sync(FULL, b1a, r >> 1), g1b = __shfl_sync(FULL, b1b, r >> 1);
-    const double h0 = (r & 1) ? g0b : g0a, h1 = (r & 1) ? g1b : g1a;
+    const double h0 = (r & 1) ? g0b : g0a;
+    double h1 = 0.0;
+    if (W) {
+      const double b1a = (ca == n - 1 ? inv_last : 0.0) - c1a, b1b = (ca + 1 == n - 1 ? inv_last : 0.0) - c1b;
+      const double g1a = __shfl_sync(FULL, b1a, r >> 1), g1b = __shfl_sync(FULL, b1b, r >> 1);
+      h1 = (r & 1) ? g1b : g1a;
+    }
     // x_J[c] = sum_r inv(L_JJ)[r][c] rhs[r]  (lower triangle only)
     const double la = r >= 2 * q ? dg.x : 0.0, lb = r >= 2 * q + 1 ? dg.y : 0.0;
-    double x0a = la * h0, x0b = lb * h0, x1a = la * h1, x1b = lb * h1;
+    double x0a = la * h0, x0b = lb * h0, x1a = 0.0, x1b = 0.0;
+    if (W) { x1a = la * h1; x1b = lb * h1; }
     for (int o = 4; o < 32; o <<= 1) {
       x0a += __shfl_xor_sync(FULL, x0a, o); x0b += __shfl_xor_sync(FULL, x0b, o);
-      x1a += __shfl_xor_sync(FULL, x1a, o); x1b += __shfl_xor_sync(FULL, x1b, o);
+      if (W) { x1a += __shfl_xor_sync(FULL, x1a, o); x1b += __shfl_xor_sync(FULL, x1b, o); }
     }
     if (r == 0) {
       s_al[ca] = x0a; s_al[ca + 1] = x0b;
-      s_t[ca] = x1a; s_t[ca + 1] = x1b;
+      if (W) { s_t[ca] = x1a; s_t[ca + 1] = x1b; }
     }
     __syncwarp();
   }
-  for (int o = 16; o; o >>= 1) maxinv2 = fmax(maxinv2, __shfl_xor_sync(FULL, maxinv2, o));
+  if (W)
+    for (int o = 16; o; o >>= 1) maxinv2 = fmax(maxinv2, __shfl_xor_sync(FULL, maxinv2, o));
+  return maxinv2;
+}
 
-  // ---- anchor, guard, a = J t, zero padding, the chain's lag table ----
-  const double kss = km[0], noise = km[2];
-  const double* ktab = a.ktab + lw * (long long)VAR_TAB_MAX;
-  const double t0 = kss + (noise + CNGP_JITTER);
-  const double s = t0 - ktab[0];
-  const double gam = s_t[n - 1];
-  const double q0 = t0 - 2.0 * s + s * s * gam;
-  // min_k L_kk^2 >= g t0  <=>  max_k inv(L)_kk^2 <= 1 / (g t0)
-  bool good = maxinv2 * (TOEP_MIN_PIVOT2 * t0) <= 1.0 && isfinite(q0) && gam > 0.0;
+// s_tab[j] = k*(|L| d), L = j - TVT_P - (n-1) + m0 the lag (in lattice steps) of chain offset c and row i at
+// j = TVT_P + n-1 + c - i; entries outside the real (c, i) range are 0.  Threads tid, tid + nth, ...
+__device__ __forceinline__ void tvt_table(double* s_tab, const double* ktab, const TvtShape& sh, int n, int d, int tid,
+                                          int nth) {
+  const int lmin = sh.m0 - (n - 1);
+  for (int j = tid; j < sh.need; j += nth) {
+    const int L = j - TVT_P - (n - 1) + sh.m0;
+    s_tab[j] = (L >= lmin && L <= sh.mend) ? ktab[(L < 0 ? -L : L) * d] : 0.0;
+  }
+}
+
+// The chain.  Every lane runs TVT_P consecutive chain points per pass; the mean alpha^T k always, and with UV the
+// recurrence terms a^T k, t^T k and the variance.  Returns this lane's "every result finite".
+template <bool UV>
+__device__ __forceinline__ bool tvt_chain(const double* s_tab, const double* s_al, const double* s_a, const double* s_t,
+                                          int n, const TvtShape& sh, int ms, int mc, double q0, double igam, double kss,
+                                          double noise, int sigma_mode, double* mean, double* var, int lane) {
+  const unsigned FULL = 0xffffffffu;
   const int npad = (n + TVT_P - 1) / TVT_P * TVT_P;
-  for (int i = lane; i < npad; i += 32) {
-    if (i < n) {
-      good &= isfinite(s_al[i]) && isfinite(s_t[i]);
-      s_a[i] = s_t[n - 1 - i];
-    } else {
-      s_al[i] = 0.0; s_a[i] = 0.0; s_t[i] = 0.0;
-    }
-  }
-  // s_tab[j] = k*(|L| d), L = j - TVT_P - (n-1) + m0 the lag (in lattice steps) of chain offset c and row i at
-  // j = TVT_P + n-1 + c - i; entries outside the real (c, i) range are 0
-  const int lmin = m0 - (n - 1);
-  for (int j = lane; j < need; j += 32) {
-    const int L = j - TVT_P - (n - 1) + m0;
-    s_tab[j] = (L >= lmin && L <= mend) ? ktab[(L < 0 ? -L : L) * d] : 0.0;
-  }
-  if (!__all_sync(FULL, good)) {
-    if (lane == 0) taken[lw] = 0;
-    return;
-  }
-  __syncwarp();
-
-  // ---- the chain ----
-  const double igam = 1.0 / gam;
-  double* mean = a.mean + win * (long long)M;
-  double* var = a.var + win * (long long)M;
-  const int cout0 = ms - m0;   // chain offset of test point 0
+  const int cout0 = ms - sh.m0;   // chain offset of test point 0
   double carry = 0.0, vcarry = 0.0;   // sum of the increments of the earlier passes; t^T k of the last point before
   bool fin = true;
-  for (int pass = 0; pass < passes; ++pass) {
+  for (int pass = 0; pass < sh.passes; ++pass) {
     const int c0 = pass * 32 * TVT_P + lane * TVT_P;   // this lane's first chain offset
     const double* tb = s_tab + TVT_P + (n - 1) + c0;    // K(i, p) = tb[p - i]
     double kw[TVT_P], mu[TVT_P], u[TVT_P], v[TVT_P];
@@ -186,15 +168,33 @@ __global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(cons
       for (int st = 0; st < TVT_P; ++st) {
         const int i = i0 + st;
         kw[(TVT_P - st) % TVT_P] = tb[-i];
-        const double al = s_al[i], aa = s_a[i], tt = s_t[i];
+        const double al = s_al[i];
 #pragma unroll
         for (int p = 0; p < TVT_P; ++p) {
           const double k = kw[(p - st + TVT_P) % TVT_P];
           mu[p] = fma(al, k, mu[p]);
-          u[p] = fma(aa, k, u[p]);
-          v[p] = fma(tt, k, v[p]);
+        }
+        if (UV) {
+          const double aa = s_a[i], tt = s_t[i];
+#pragma unroll
+          for (int p = 0; p < TVT_P; ++p) {
+            const double k = kw[(p - st + TVT_P) % TVT_P];
+            u[p] = fma(aa, k, u[p]);
+            v[p] = fma(tt, k, v[p]);
+          }
         }
       }
+    }
+    if (!UV) {
+#pragma unroll
+      for (int p = 0; p < TVT_P; ++p) {
+        const int j = c0 + p - cout0;
+        if (j >= 0 && j < mc) {
+          fin &= isfinite(mu[p]);
+          mean[j] = mu[p];
+        }
+      }
+      continue;
     }
     // increments delta_c = u_c^2 - v_{c-1}^2 (delta_0 = 0: the anchor), summed in chain order
     double vprev = __shfl_up_sync(FULL, v[TVT_P - 1], 1);
@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(cons
       if (j >= 0 && j < mc) {
         const double qm = fma(base + ps[p], igam, q0);
         const double vv = fmax(kss - qm, CNGP_VAR_FLOOR) + noise;
-        const double out = a.sigma_mode ? 2.0 * sqrt(vv) : vv;
+        const double out = sigma_mode ? 2.0 * sqrt(vv) : vv;
         fin &= isfinite(mu[p]) && isfinite(out);
         mean[j] = mu[p];
         var[j] = out;
@@ -231,9 +231,83 @@ __global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(cons
     carry += __shfl_sync(FULL, incl, 31);
     vcarry = __shfl_sync(FULL, v[TVT_P - 1], 31);
   }
-  // a window with a non-finite result is left to gp_var_kernel, which rewrites every entry
-  fin = __all_sync(FULL, fin);
-  if (lane == 0) taken[lw] = fin ? 1 : 0;
+  return fin;
+}
+
+// One window on one warp: slot lw of the phase-A buffers (factor, z, table, meta, integer stamps), window win of the
+// call (counts, test stamps, status), results to mean_row / var_row.  s_w: the warp's shared room (tvt_warp_doubles).
+// Returns (warp-uniform) whether the window was taken; a window not taken has had nothing written.
+__device__ __forceinline__ bool tvt_window(const VarArgs& a, long long lw, long long win, double* s_w, double* mean_row,
+                                           double* var_row, int lane) {
+  const unsigned FULL = 0xffffffffu;
+  const int nt = a.nt, R = 8 * nt, M = a.M;
+  const int cap = tvt_tab_cap(nt, M);
+  double* s_al = s_w;
+  double* s_a = s_al + R + TVT_P;
+  double* s_t = s_a + R + TVT_P;
+  double* s_tab = s_t + R + TVT_P;
+
+  // ---- the window's own qualification (no factor read yet) ----
+  const double* km = a.kmeta + lw * (long long)VAR_META;
+  const int* xi = a.kxi + lw * (long long)R;
+  const int n = a.n_win ? a.n_win[win] : a.N;
+  const int mc = a.m_win ? a.m_win[win] : M;
+  bool ok = km[3] != 0.0 && n >= 2 && mc >= 1 && !(a.status && a.status[win] != 0);
+  int d = 1, ms = 0;
+  if (ok) {
+    ok = toep_uniform(xi, n, lane, d);
+    const double* xs = a.xstar + (a.xstar_stride ? win * a.xstar_stride : 0);
+    ok = ok && tvt_lattice(xs, km[1], xi[0], d, mc, lane, ms);
+  }
+  const TvtShape sh(n, ms, mc);
+  ok = ok && sh.need <= cap;
+  if (!__all_sync(FULL, ok)) return false;
+
+  // ---- [alpha, w] = L^-T [z, e_{n-1} / L_{n-1,n-1}] ----
+  const double maxinv2 = tvt_backsub<true>(a.L + lw * (long long)tiles_in_lower(nt) * 64, a.z + lw * (long long)R, n, nt,
+                                           lane, s_al, s_t);
+
+  // ---- anchor, guard, a = J t, zero padding, the chain's lag table ----
+  const double kss = km[0], noise = km[2];
+  const double* ktab = a.ktab + lw * (long long)VAR_TAB_MAX;
+  const double t0 = kss + (noise + CNGP_JITTER);
+  const double s = t0 - ktab[0];
+  const double gam = s_t[n - 1];
+  const double q0 = t0 - 2.0 * s + s * s * gam;
+  // min_k L_kk^2 >= g t0  <=>  max_k inv(L)_kk^2 <= 1 / (g t0)
+  bool good = maxinv2 * (TOEP_MIN_PIVOT2 * t0) <= 1.0 && isfinite(q0) && gam > 0.0;
+  const int npad = (n + TVT_P - 1) / TVT_P * TVT_P;
+  for (int i = lane; i < npad; i += 32) {
+    if (i < n) {
+      good &= isfinite(s_al[i]) && isfinite(s_t[i]);
+      s_a[i] = s_t[n - 1 - i];
+    } else {
+      s_al[i] = 0.0; s_a[i] = 0.0; s_t[i] = 0.0;
+    }
+  }
+  tvt_table(s_tab, ktab, sh, n, d, lane, 32);
+  if (!__all_sync(FULL, good)) return false;
+  __syncwarp();
+
+  // ---- the chain; a window with a non-finite result is left to gp_var_kernel, which rewrites every entry ----
+  const bool fin = tvt_chain<true>(s_tab, s_al, s_a, s_t, n, sh, ms, mc, q0, 1.0 / gam, kss, noise, a.sigma_mode,
+                                   mean_row, var_row, lane);
+  return __all_sync(FULL, fin);
+}
+
+__global__ void __launch_bounds__(TVT_WARPS * 32, 3) gp_var_toeplitz_kernel(const VarArgs a, int* taken) {
+  extern __shared__ __align__(16) double tvt_smem[];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const long long lw = (long long)blockIdx.x * TVT_WARPS + w;   // window within this launch
+  if (lw >= a.n_windows_launch) return;
+  const long long win = a.window0 + lw;
+  if (a.skip && a.skip[win]) {   // a member of a shared covariance: gp_toep_member_kernel has its results
+    if (lane == 0) taken[lw] = 1;
+    return;
+  }
+  const bool ok = tvt_window(a, lw, win, tvt_smem + (size_t)w * tvt_warp_doubles(a.nt, a.M), a.mean + win * (long long)a.M,
+                             a.var + win * (long long)a.M, lane);
+  if (lane == 0) taken[lw] = ok ? 1 : 0;
 }
 
 // The windows of a launch that gp_var_toeplitz_kernel did not take, in increasing order (ballot + block scan, a fixed
