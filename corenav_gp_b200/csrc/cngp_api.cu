@@ -541,7 +541,7 @@ static int launch_var_toeplitz(cngp_ctx* ctx, VarArgs& va, long long nw, cudaStr
 
 // Shared covariance (gp_toep_group.cuh, DESIGN.md section 4.2d).  Under the gate of the Toeplitz kernels and with one
 // theta for the whole call, the chunk's largest group of windows with the same key is factored once: the key and group
-// kernels, the one-window Schur fit into a slot of its own (slot SLOT_TG_DATA: factor | z | L_jj | table | meta |
+// kernels, the group's Schur fit into a slot of its own (slot SLOT_TG_DATA: factor | z | L_jj | table | meta |
 // integer stamps | variance row | mean row | log det) and the member kernel, which clears flag (slot SLOT_TG_FLAG,
 // [n_windows]) for whatever goes back to the per-window kernels.  Those then run with flag as their skip list.
 enum { SLOT_TG_KEY = 29, SLOT_TG_FLAG = 30, SLOT_TG_LIST = 31, SLOT_TG_REC = 32, SLOT_TG_DATA = 33 };
@@ -579,7 +579,16 @@ static int launch_toep_group(cngp_ctx* ctx, const FitArgs& fa, const VarArgs& va
   g.y = nullptr; g.L = gL; g.z = gz; g.feat = nullptr; g.lml = nullptr; g.logdet = glogdet; g.quad = nullptr;
   g.status = nullptr; g.ktab = gtab; g.kmeta = gmeta; g.kxi = gxi; g.n_lazy = nullptr; g.done = tg.rec + TG_FIT;
   g.ldiag = gdiag; g.f32_factor = 0;
-  launch_fit_toeplitz<KID_GENERIC>(g, 1, s);
+#ifdef CNGP_TG_TIMING
+  {
+    unsigned long long z[16] = {};
+    z[10] = ~0ull;
+    cudaMemcpyToSymbolAsync(tg_stamp, z, sizeof z, 0, cudaMemcpyHostToDevice, s);
+  }
+#endif
+  const size_t fsmem = tgf_smem_bytes(nt);
+  cudaFuncSetAttribute(gp_toep_group_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem);
+  gp_toep_group_fit_kernel<<<1, TGF_THREADS, fsmem, s>>>(g);
   ctx->launches += 2;   // + the begin() below that re-opens the fit span
   ctx->end();
   ctx->begin(CNGP_PROF_VAR);
@@ -593,6 +602,17 @@ static int launch_toep_group(cngp_ctx* ctx, const FitArgs& fa, const VarArgs& va
   const size_t smem = tg_smem_bytes(nt, M);
   cudaFuncSetAttribute(gp_toep_member_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   gp_toep_member_kernel<<<(unsigned)(1 + (nw + TG_WARPS - 1) / TG_WARPS), TG_WARPS * 32, smem, s>>>(t);
+#ifdef CNGP_TG_TIMING
+  {
+    unsigned long long h[16];
+    cudaStreamSynchronize(s);
+    cudaMemcpyFromSymbol(h, tg_stamp, sizeof h);
+    auto us = [&](int i, int from) { return h[i] ? 1e-3 * (double)(long long)(h[i] - h[from]) : -1.0; };
+    fprintf(stderr, "tg_timing fit_us prologue %.1f generators %.1f recursion %.1f outputs %.1f end %.1f"
+            " | member_us var_row %.1f members_start %.1f z %.1f alpha %.1f members_end %.1f\n",
+            us(1, 0), us(2, 0), us(3, 0), us(4, 0), us(5, 0), us(9, 8), us(10, 8), us(12, 8), us(13, 8), us(11, 8));
+  }
+#endif
   ctx->end();
   ctx->begin(CNGP_PROF_FIT);
   return CNGP_OK;

@@ -64,69 +64,76 @@ struct TvtShape {
   }
 };
 
-// [alpha, w] = L^-T [z, e_{n-1} / L_{n-1,n-1}] by one back substitution over the stored factor Lp, tile column
+// [alpha, w] = L^-T [z, e_{n-1} / L_{n-1,n-1}] by one back substitution over the stored factor, tile column
 // J = nt-1 .. 0, into s_al (and, with W, s_t).  W also returns max_k inv(L)_kk^2 over k < n (the conditioning guard).
 // Without W the alpha half is the same arithmetic, so alpha has the same bits either way.
+// tvt_backsub_col is the step of tile column J: col holds its tiles I = J .. nt-1 (inv(L_JJ) first) as rows
+// 8 (I - J) + r of RS doubles each - RS = 8 in the packed factor, more where a shared-memory copy pads its rows.
+template <bool W, int RS>
+__device__ __forceinline__ void tvt_backsub_col(const double* col, int J, const double* zp, int n, int nt, int lane,
+                                                double* s_al, double* s_t, double& inv_last, double& maxinv2) {
+  const unsigned FULL = 0xffffffffu;
+  const int r = lane >> 2, q = lane & 3;
+  col += r * RS + 2 * q;
+  const double2 dg = *reinterpret_cast<const double2*>(col);   // inv(L_JJ), row r, columns 2q, 2q+1
+  double c0a = 0.0, c0b = 0.0, c1a = 0.0, c1b = 0.0;             // (L_IJ^T x_I) for columns 2q, 2q+1: alpha | w
+#pragma unroll 8
+  for (int I = J + 1; I < nt; ++I) {
+    const double2 l = *reinterpret_cast<const double2*>(col + (I - J) * 8 * RS);
+    const double xa = s_al[8 * I + r];
+    c0a = fma(l.x, xa, c0a); c0b = fma(l.y, xa, c0b);
+    if (W) {
+      const double xw = s_t[8 * I + r];
+      c1a = fma(l.x, xw, c1a); c1b = fma(l.y, xw, c1b);
+    }
+  }
+  // rows of the diagonal tile: pivots of the guard, 1 / L_{n-1,n-1}
+  const int row = 8 * J + r;
+  const double dv = (r == 2 * q) ? dg.x : (r == 2 * q + 1 ? dg.y : 0.0);
+  if (W) {
+    if ((r >> 1) == q && row < n) maxinv2 = fmax(maxinv2, dv * dv);
+    if (J == nt - 1) {
+      const int kl = (n - 1) & 7;   // n-1 lies in the last tile column
+      inv_last = __shfl_sync(FULL, dv, 4 * kl + (kl >> 1));
+    }
+  }
+  for (int o = 4; o < 32; o <<= 1) {
+    c0a += __shfl_xor_sync(FULL, c0a, o); c0b += __shfl_xor_sync(FULL, c0b, o);
+    if (W) { c1a += __shfl_xor_sync(FULL, c1a, o); c1b += __shfl_xor_sync(FULL, c1b, o); }
+  }
+  // right-hand sides of rows 8J + 2q (+1), then gathered to row r = lane >> 2
+  const int ca = 8 * J + 2 * q;
+  const double2 zz = *reinterpret_cast<const double2*>(zp + ca);
+  const double b0a = zz.x - c0a, b0b = zz.y - c0b;
+  const double g0a = __shfl_sync(FULL, b0a, r >> 1), g0b = __shfl_sync(FULL, b0b, r >> 1);
+  const double h0 = (r & 1) ? g0b : g0a;
+  double h1 = 0.0;
+  if (W) {
+    const double b1a = (ca == n - 1 ? inv_last : 0.0) - c1a, b1b = (ca + 1 == n - 1 ? inv_last : 0.0) - c1b;
+    const double g1a = __shfl_sync(FULL, b1a, r >> 1), g1b = __shfl_sync(FULL, b1b, r >> 1);
+    h1 = (r & 1) ? g1b : g1a;
+  }
+  // x_J[c] = sum_r inv(L_JJ)[r][c] rhs[r]  (lower triangle only)
+  const double la = r >= 2 * q ? dg.x : 0.0, lb = r >= 2 * q + 1 ? dg.y : 0.0;
+  double x0a = la * h0, x0b = lb * h0, x1a = 0.0, x1b = 0.0;
+  if (W) { x1a = la * h1; x1b = lb * h1; }
+  for (int o = 4; o < 32; o <<= 1) {
+    x0a += __shfl_xor_sync(FULL, x0a, o); x0b += __shfl_xor_sync(FULL, x0b, o);
+    if (W) { x1a += __shfl_xor_sync(FULL, x1a, o); x1b += __shfl_xor_sync(FULL, x1b, o); }
+  }
+  if (r == 0) {
+    s_al[ca] = x0a; s_al[ca + 1] = x0b;
+    if (W) { s_t[ca] = x1a; s_t[ca + 1] = x1b; }
+  }
+  __syncwarp();
+}
 template <bool W>
 __device__ __forceinline__ double tvt_backsub(const double* Lp, const double* zp, int n, int nt, int lane, double* s_al,
                                               double* s_t) {
   const unsigned FULL = 0xffffffffu;
-  const int r = lane >> 2, q = lane & 3;
   double inv_last = 0.0, maxinv2 = 0.0;
-  for (int J = nt - 1; J >= 0; --J) {
-    const double* col = Lp + (long long)tile_index(J, J, nt) * 64 + 2 * lane;
-    const double2 dg = *reinterpret_cast<const double2*>(col);   // inv(L_JJ), row r, columns 2q, 2q+1
-    double c0a = 0.0, c0b = 0.0, c1a = 0.0, c1b = 0.0;             // (L_IJ^T x_I) for columns 2q, 2q+1: alpha | w
-#pragma unroll 8
-    for (int I = J + 1; I < nt; ++I) {
-      const double2 l = *reinterpret_cast<const double2*>(col + (I - J) * 64);
-      const double xa = s_al[8 * I + r];
-      c0a = fma(l.x, xa, c0a); c0b = fma(l.y, xa, c0b);
-      if (W) {
-        const double xw = s_t[8 * I + r];
-        c1a = fma(l.x, xw, c1a); c1b = fma(l.y, xw, c1b);
-      }
-    }
-    // rows of the diagonal tile: pivots of the guard, 1 / L_{n-1,n-1}
-    const int row = 8 * J + r;
-    const double dv = (r == 2 * q) ? dg.x : (r == 2 * q + 1 ? dg.y : 0.0);
-    if (W) {
-      if ((r >> 1) == q && row < n) maxinv2 = fmax(maxinv2, dv * dv);
-      if (J == nt - 1) {
-        const int kl = (n - 1) & 7;   // n-1 lies in the last tile column
-        inv_last = __shfl_sync(FULL, dv, 4 * kl + (kl >> 1));
-      }
-    }
-    for (int o = 4; o < 32; o <<= 1) {
-      c0a += __shfl_xor_sync(FULL, c0a, o); c0b += __shfl_xor_sync(FULL, c0b, o);
-      if (W) { c1a += __shfl_xor_sync(FULL, c1a, o); c1b += __shfl_xor_sync(FULL, c1b, o); }
-    }
-    // right-hand sides of rows 8J + 2q (+1), then gathered to row r = lane >> 2
-    const int ca = 8 * J + 2 * q;
-    const double2 zz = *reinterpret_cast<const double2*>(zp + ca);
-    const double b0a = zz.x - c0a, b0b = zz.y - c0b;
-    const double g0a = __shfl_sync(FULL, b0a, r >> 1), g0b = __shfl_sync(FULL, b0b, r >> 1);
-    const double h0 = (r & 1) ? g0b : g0a;
-    double h1 = 0.0;
-    if (W) {
-      const double b1a = (ca == n - 1 ? inv_last : 0.0) - c1a, b1b = (ca + 1 == n - 1 ? inv_last : 0.0) - c1b;
-      const double g1a = __shfl_sync(FULL, b1a, r >> 1), g1b = __shfl_sync(FULL, b1b, r >> 1);
-      h1 = (r & 1) ? g1b : g1a;
-    }
-    // x_J[c] = sum_r inv(L_JJ)[r][c] rhs[r]  (lower triangle only)
-    const double la = r >= 2 * q ? dg.x : 0.0, lb = r >= 2 * q + 1 ? dg.y : 0.0;
-    double x0a = la * h0, x0b = lb * h0, x1a = 0.0, x1b = 0.0;
-    if (W) { x1a = la * h1; x1b = lb * h1; }
-    for (int o = 4; o < 32; o <<= 1) {
-      x0a += __shfl_xor_sync(FULL, x0a, o); x0b += __shfl_xor_sync(FULL, x0b, o);
-      if (W) { x1a += __shfl_xor_sync(FULL, x1a, o); x1b += __shfl_xor_sync(FULL, x1b, o); }
-    }
-    if (r == 0) {
-      s_al[ca] = x0a; s_al[ca + 1] = x0b;
-      if (W) { s_t[ca] = x1a; s_t[ca + 1] = x1b; }
-    }
-    __syncwarp();
-  }
+  for (int J = nt - 1; J >= 0; --J)
+    tvt_backsub_col<W, 8>(Lp + (long long)tile_index(J, J, nt) * 64, J, zp, n, nt, lane, s_al, s_t, inv_last, maxinv2);
   if (W)
     for (int o = 16; o; o >>= 1) maxinv2 = fmax(maxinv2, __shfl_xor_sync(FULL, maxinv2, o));
   return maxinv2;

@@ -6,8 +6,9 @@ not do; its `achieved` and `frac` are no longer a share of anything.  The two ho
   - FP64 pipe: 4 FMA per factor entry pair and right-hand side of the back substitution, 3 n FMA per chain point.
 With --grouped, the shared-covariance path (DESIGN.md section 4.2d) instead: one window's factor and recurrence for the
 whole batch, and per member the forward solve for z (one FMA per factor entry), the back substitution for alpha (one
-right-hand side) and n FMA per chain point for the mean, the factor read from L2; HBM carries y in and mean, variance,
-LML and status out.  --ms is then the step time (fit and variance phases together: the member kernel does both).
+right-hand side) and n FMA per chain point for the mean; HBM carries y in and mean, variance, LML and status out.  The
+members of a CTA (TG_WARPS of them) share one shared-memory copy of each tile column, so L2 delivers the factor twice
+(z, alpha) per member CTA, plus the L_jj tiles with the z pass.  --ms is then the step time (fit and variance phases together: the member kernel does both).
 Usage: python tools/var_toeplitz_roofline.py --ms <variance phase ms> [--B 4096 --N 256 --M 600] [--grouped]
        [--hbm-tbs 7.7] [--fp64-tflops 33.9]   (data-sheet HBM bandwidth; DFMA issue peak of profiles/fp64_peak_r01.json)"""
 import argparse
@@ -32,6 +33,9 @@ def figures(B, N, M, ms, hbm_tbs, fp64_tflops):
     }
 
 
+TG_WARPS = 8   # members per CTA of gp_toep_member_kernel
+
+
 def grouped_figures(B, N, M, ms, hbm_tbs, fp64_tflops):
     nt = (N + 7) // 8
     tiles = nt * (nt + 1) // 2
@@ -44,7 +48,7 @@ def grouped_figures(B, N, M, ms, hbm_tbs, fp64_tflops):
     return {
         "B": B, "N": N, "M": M, "step_ms": ms, "grouped": True,
         "hbm_bytes": hbm_bytes, "hbm_tb_per_s": hbm_bytes / t * 1e-12, "hbm_frac": hbm_bytes / t * 1e-12 / hbm_tbs,
-        "l2_factor_bytes": tiles * 512 * 2 * B,                 # each member reads the factor twice (z, alpha)
+        "l2_factor_bytes": (tiles * 2 + nt) * 512 * -(-B // TG_WARPS),   # twice per member CTA, L_jj once
         "fma": fma, "fp64_tflops": 2 * fma / t * 1e-12, "fp64_frac": 2 * fma / t * 1e-12 / fp64_tflops,
         "lower_bound_ms": 1e3 * max(hbm_bytes / (hbm_tbs * 1e12), 2 * fma / (fp64_tflops * 1e12)),
     }
