@@ -110,6 +110,15 @@ SIGNATURES = {
     "cngp_large_reduce": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_dp, c_ip, c_dp, c_dp]),
     "cngp_large_backsolve_step": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_dp, c_i64, c_dp, c_dp]),
     "cngp_large_matvec": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_dp, c_dp, c_i64, c_dp]),
+    "cngp_large_predict_sizes": (C.c_int, [C.POINTER(LargePlan), c_i64, c_i64, C.POINTER(c_i64), C.POINTER(c_i64),
+                                           C.POINTER(c_i64)]),
+    "cngp_large_predict_assemble": (C.c_int, [c_vp, C.POINTER(LargePlan), C.POINTER(Kernel), c_dp, c_dp, c_dp, c_i64, c_dp]),
+    "cngp_large_predict_panel": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_dp, c_dp, c_i64, c_i64, c_dp, c_dp]),
+    "cngp_large_predict_update": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_i64, c_i64, c_dp, c_i64, c_i64]),
+    "cngp_large_predict_finish": (C.c_int, [c_vp, C.POINTER(LargePlan), C.POINTER(Kernel), c_dp, c_dp, c_dp, c_dp, c_i64,
+                                            c_dp, c_dp, c_dp]),
+    "cngp_chol_large_predict": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_dp, c_dp, c_i64, c_dp, c_i64, c_dp, c_dp, c_dp,
+                                          c_dp, c_dp, c_i32]),
 }
 
 _lib = None

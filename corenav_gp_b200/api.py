@@ -543,6 +543,31 @@ class GpContext:
             res["alpha"] = alpha
         return res
 
+    def chol_large_predict(self, kernel, theta, x, y, xstar):
+        """chol_large, then the predictive mean and variance at xstar [M] from the factor (GPy m.predict with
+        include_likelihood=True).  x, y, xstar: host arrays or CUDA tensors, all alike.  Returns dict(mean, var, logdet,
+        quad, lml, pivot): pivot = 0, or the (1-based) pivot at which Ky was found not positive definite - then every
+        other value is NaN."""
+        k = parse_kernel(kernel)
+        dev = _is_cuda(x)
+        N = int(np.prod(tuple(x.shape)))
+        M = int(np.prod(tuple(xstar.shape)))
+        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
+        if th.size != k.n_params + 1:
+            raise CngpError(f"theta has {th.size} entries, kernel needs {k.n_params + 1} (noise last)")
+        outs = np.empty(3)
+        mean = self._empty((M,), np.float64, dev)
+        var = self._empty((M,), np.float64, dev)
+        a = [_Arg(x, np.float64, dev), _Arg(y, np.float64, dev), _Arg(xstar, np.float64, dev),
+             _Arg(mean, np.float64, dev, output=True), _Arg(var, np.float64, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_chol_large_predict(self.h, C.byref(k), th.ctypes.data, a[0].ptr, a[1].ptr, N, a[2].ptr, M,
+                                              a[3].ptr, a[4].ptr, outs.ctypes.data, outs.ctypes.data + 8,
+                                              outs.ctypes.data + 16, L.MEM_DEVICE if dev else L.MEM_HOST)
+        if rc < 0:
+            self._check(rc, "cngp_chol_large_predict")
+        return dict(mean=mean, var=var, logdet=float(outs[0]), quad=float(outs[1]), lml=float(outs[2]), pivot=int(rc))
+
     def large_matvec(self, kernel, theta, x, v):
         """r = (K(x,x) + (noise + 1e-8) I) v evaluated on the fly on the device; x, v CUDA tensors [N]."""
         k = parse_kernel(kernel)

@@ -17,6 +17,9 @@
 //    per CTA, 8 consumer warps x 32 accumulator tiles in registers (mma.sync m8n8k4 f64 - FP64 has no tcgen05 kind),
 //    operands streamed through a 4-stage shared-memory ring by a producer warp issuing cp.async.bulk (UBLKCP) with
 //    mbarrier completion; C is loaded straight into the accumulators before the main loop and stored once.
+//  * predict pass (after the factorisation, reading only A, winv and alpha): W = L^-1 K(x, x*) as a forward sweep over
+//    R = K(x*, x) in the same block-cyclic shape - the owner forms W_k with the panel product, every rank updates its
+//    block columns of R with the same CTA body as the trailing update (cngp.h, cngp_large_predict_*).
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -224,10 +227,15 @@ struct GemmArgs {
   PanelGeom pg;
 };
 
+// One 16 x 16-tile block of C, rows rt0.. and columns ct0..:  C = sum_{k < KT} X(k, rt0..) Y(k, n0..)^T, or with `sub`
+// C -= the same (C loaded into the accumulators first).  The CTA body of large_gemm_kernel and large_pred_update_kernel.
+__device__ __forceinline__ void gemm_block(const double* Xb, long long xks, const double* Yb, long long yks, double* Cb,
+                                           long long ccs, long long rt0, long long n0, long long ct0, int KT, bool sub,
+                                           double* ring, unsigned long long* bars);
+
 __global__ void __launch_bounds__(LG_THREADS, 1) large_gemm_kernel(const GemmArgs a) {
   extern __shared__ __align__(128) double ring[];
   __shared__ unsigned long long bars[2 * LG_STAGES];
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const long long rt0 = (long long)(a.rb0 + blockIdx.x) * LG_BLK;
   long long n0, ct0;
   int KT;
@@ -256,6 +264,13 @@ __global__ void __launch_bounds__(LG_THREADS, 1) large_gemm_kernel(const GemmArg
     Yb = a.panel + cy.base; yks = cy.kstride;
     Cb = a.C; ccs = a.c_cstride;
   }
+  gemm_block(Xb, xks, Yb, yks, Cb, ccs, rt0, n0, ct0, KT, a.mode == 1, ring, bars);
+}
+
+__device__ __forceinline__ void gemm_block(const double* Xb, long long xks, const double* Yb, long long yks, double* Cb,
+                                           long long ccs, long long rt0, long long n0, long long ct0, int KT, bool sub,
+                                           double* ring, unsigned long long* bars) {
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const uint32_t full_u32 = smem_u32(&bars[0]), empty_u32 = smem_u32(&bars[LG_STAGES]);
   if (tid == 0) {
     for (int s = 0; s < LG_STAGES; ++s) { mbar_init(full_u32 + 8 * s, 1); mbar_init(empty_u32 + 8 * s, LG_CONSUMERS); }
@@ -283,7 +298,7 @@ __global__ void __launch_bounds__(LG_THREADS, 1) large_gemm_kernel(const GemmArg
   const int wr = w >> 2, wc = w & 3;
   tile2 acc[8][4];
   double* cbase = Cb + (ct0 + wc * 4) * ccs + (rt0 + wr * 8) * 64 + 2 * lane;
-  if (a.mode == 1) {
+  if (sub) {
 #pragma unroll
     for (int j = 0; j < 4; ++j)
 #pragma unroll
@@ -297,7 +312,7 @@ __global__ void __launch_bounds__(LG_THREADS, 1) large_gemm_kernel(const GemmArg
 #pragma unroll
       for (int i = 0; i < 8; ++i) acc[i][j] = tile2{0.0, 0.0};
   }
-  const bool neg = a.mode == 1;
+  const bool neg = sub;
   for (int it = 0; it < n_it; ++it) {
     const int s = it % LG_STAGES;
     // refill duty rotates over the warps: the slot consumed at iteration it-1 gets iteration it + LG_STAGES - 1
@@ -495,6 +510,129 @@ __global__ void __launch_bounds__(256) large_matvec_kernel(KProg kp, const doubl
   }
   for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   if (lane == 0) out[row] = s;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// predict pass over the stored factor: W = L^-1 K(x, x*) as a forward sweep on R = K(x*, x), block column by block column
+// ------------------------------------------------------------------------------------------------------------
+// R is stored like A but with m_tiles row tiles (test points, 8 per tile, padded to a multiple of 128 so that every GEMM
+// block is whole): tile (mt, local column tile lct) at R[(lct * m_tiles + mt) * 64].  Rows m >= M and columns >= N are 0.
+struct PredAsmArgs {
+  KProg kp;
+  const double* theta;   // device [P]
+  const double* x;       // device [N]
+  const double* xstar;   // device [M]
+  long long N, M, m_tiles;
+  long long lct0;        // first local column tile of the launch (blockIdx.y counts from it)
+  int world, rank;
+  double* R;
+};
+
+// grid (ceil(m_tiles / 8), local column tiles); one warp per tile
+template <int KID>
+__global__ void __launch_bounds__(256) large_pred_assemble_kernel(const PredAsmArgs a) {
+  __shared__ LeafConst hc[CNGP_MAX_LEAVES];
+  __shared__ KProg kps;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, r = lane >> 2, q = lane & 3;
+  FastK<KID> fk;
+  if (KID == KID_GENERIC) {
+    if (threadIdx.x < a.kp.n_leaves)
+      hc[threadIdx.x] = leaf_prepare(a.kp.leaf_type[threadIdx.x], a.theta + a.kp.leaf_param[threadIdx.x]);
+    if (threadIdx.x == 0) kps = a.kp;
+    __syncthreads();
+  } else {
+    fk.init(a.theta);                                             // phase origin 0, as large_assemble_kernel
+  }
+  const long long mt = (long long)blockIdx.x * 8 + w;
+  if (mt >= a.m_tiles) return;
+  const long long lct = a.lct0 + blockIdx.y;
+  const long long gct = ((lct / LG_BT) * a.world + a.rank) * LG_BT + lct % LG_BT;
+  const long long m = 8 * mt + r, c0 = 8 * gct + 2 * q, c1 = c0 + 1;
+  tile2 v{0.0, 0.0};
+  if (m < a.M) {
+    const double xm = a.xstar[m];
+    if (KID == KID_GENERIC) {
+      if (c0 < a.N) v.a = keval_generic_cross(&kps, hc, a.x[c0], xm);
+      if (c1 < a.N) v.b = keval_generic_cross(&kps, hc, a.x[c1], xm);
+    } else {
+      const PointFeat fm = fk.point(xm);
+      if (c0 < a.N) v.a = fk.eval(fk.point(a.x[c0]), fm, false);
+      if (c1 < a.N) v.b = fk.eval(fk.point(a.x[c1]), fm, false);
+    }
+  }
+  tile_store(a.R + (lct * a.m_tiles + mt) * 64, lane, v);
+}
+
+// R(:, c) -= W_k L(c, k)^T for this rank's block columns c: grid (m_tiles / 16, local 16-tile column blocks).
+// W tile (k-tile kt, test tile mt) at W + kt * w_kstride + mt * 64; L tile (kt, global row tile n) at Lp + kt * l_kstride
+// + n * 64 (Lp is offset so that n counts from 0).
+struct PredUpdArgs {
+  const double* W; long long w_kstride;
+  const double* Lp; long long l_kstride;
+  double* R; long long r_cstride;
+  int lcb0, world, rank;
+};
+__global__ void __launch_bounds__(LG_THREADS, 1) large_pred_update_kernel(const PredUpdArgs a) {
+  extern __shared__ __align__(128) double ring[];
+  __shared__ unsigned long long bars[2 * LG_STAGES];
+  const long long lct0 = (long long)(a.lcb0 + blockIdx.y) * LG_BLK;
+  const long long n0 = ((lct0 / LG_BT) * a.world + a.rank) * LG_BT + lct0 % LG_BT;
+  gemm_block(a.W, a.w_kstride, a.Lp, a.l_kstride, a.R, a.r_cstride, (long long)blockIdx.x * LG_BLK, n0, lct0, LG_BT, true,
+             ring, bars);
+}
+
+// s[m] = sum over the 256 columns of W_k of W(m, i)^2, in a fixed order; one warp per test tile
+__global__ void __launch_bounds__(256) large_pred_sumsq_kernel(const double* W, long long m_tiles, long long M, double* s) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, r = lane >> 2, q = lane & 3;
+  const long long mt = (long long)blockIdx.x * 8 + w;
+  if (mt >= m_tiles) return;
+  double acc = 0.0;
+  for (int kt = 0; kt < LG_BT; ++kt) {
+    const tile2 v = tile_load(W + (kt * m_tiles + mt) * 64, lane);
+    acc = fma(v.a, v.a, acc);
+    acc = fma(v.b, v.b, acc);
+  }
+  acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+  acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+  if (q == 0 && 8 * mt + r < M) s[8 * mt + r] = acc;
+}
+
+// mean[m] = K(x*_m, x) alpha (one warp per test point, large_matvec_kernel's order); var[m] = max(k(x*_m, x*_m) -
+// sum_k s[k][m], 1e-15) + noise with the block sums added in increasing k
+template <int KID>
+__global__ void __launch_bounds__(256) large_pred_finish_kernel(KProg kp, const double* theta, const double* x,
+                                                                const double* alpha, long long N, const double* xstar,
+                                                                long long M, const double* s, long long n_blockcols,
+                                                                double* mean, double* var) {
+  __shared__ LeafConst hc[CNGP_MAX_LEAVES];
+  __shared__ KProg kps;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  FastK<KID> fk;
+  if (KID == KID_GENERIC) {
+    if (threadIdx.x < kp.n_leaves) hc[threadIdx.x] = leaf_prepare(kp.leaf_type[threadIdx.x], theta + kp.leaf_param[threadIdx.x]);
+    if (threadIdx.x == 0) kps = kp;
+    __syncthreads();
+  } else {
+    fk.init(theta);
+  }
+  const long long m = (long long)blockIdx.x * 8 + w;
+  if (m >= M) return;
+  const double xm = xstar[m];
+  PointFeat fm{xm, 0.0, 0.0, 0.0};
+  if (KID != KID_GENERIC) fm = fk.point(xm);
+  double acc = 0.0;
+  for (long long c = lane; c < N; c += 32) {
+    const double k = KID == KID_GENERIC ? keval_generic_cross(&kps, hc, x[c], xm) : fk.eval(fk.point(x[c]), fm, false);
+    acc = fma(k, alpha[c], acc);
+  }
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) {
+    double vs = 0.0;
+    for (long long k = 0; k < n_blockcols; ++k) vs += s[k * M + m];
+    const double kss = KID == KID_GENERIC ? kdiag_eval(kps, hc, xm) : fk.kdiag(xm);
+    mean[m] = acc;
+    var[m] = fmax(kss - vs, CNGP_VAR_FLOOR) + theta[kp.n_params];
+  }
 }
 
 template <typename F>
@@ -857,6 +995,147 @@ extern "C" int cngp_large_matvec(cngp_ctx* ctx, const cngp_kernel* kernel, const
   return CNGP_OK;
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// predict pass (see cngp.h): R = K(x*, x) swept forward through the stored factor
+// ------------------------------------------------------------------------------------------------------------
+namespace {
+inline long long pred_m_tiles(int64_t M) { return (M + 8 * LG_BLK - 1) / (8 * LG_BLK) * LG_BLK; }
+inline long long pred_payload_doubles(const cngp_large_plan* p, long long m_tiles, int64_t k) {
+  return (long long)LG_BT * 64 * (m_tiles + p->n_pad / 8 - (k + 1) * LG_BT);
+}
+int upload_theta(cngp_ctx* ctx, const KProg& kp, const double* theta, double** d_theta, const char* what) {
+  *d_theta = (double*)cngp_ctx_buf(ctx, SLOT_THETA, sizeof(double) * (CNGP_MAX_PARAMS + 1));
+  if (!*d_theta) return cngp_set_error(ctx, CNGP_ERR_NOMEM, what);
+  cudaStream_t s = cngp_ctx_stream(ctx);
+  LCU(ctx, cudaMemcpyAsync(*d_theta, theta, sizeof(double) * (kp.n_params + 1), cudaMemcpyHostToDevice, s));
+  LCU(ctx, cudaStreamSynchronize(s));   // theta is a host stack/array of the caller
+  return CNGP_OK;
+}
+}  // namespace
+
+extern "C" int cngp_large_predict_sizes(const cngp_large_plan* p, int64_t M, int64_t k, int64_t* r_doubles,
+                                        int64_t* payload_doubles, int64_t* s_doubles) {
+  if (!p || M <= 0 || k < 0 || k >= p->n_blockcols) return CNGP_ERR_INVALID;
+  const long long mt = pred_m_tiles(M);
+  if (r_doubles) *r_doubles = p->n_local_blockcols * LG_BT * mt * 64;
+  if (payload_doubles) *payload_doubles = pred_payload_doubles(p, mt, k);
+  if (s_doubles) *s_doubles = p->n_blockcols * M;
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_predict_assemble(cngp_ctx* ctx, const cngp_large_plan* p, const cngp_kernel* kernel,
+                                           const double* theta, const double* x, const double* xstar, int64_t M, double* R) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !kernel || !theta || !x || !xstar || !R || M <= 0)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_predict_assemble: bad argument");
+  KProg kp;
+  int rc = cngp_build_kprog(kernel, &kp);
+  if (rc) return cngp_set_error(ctx, rc, "large_predict_assemble: invalid kernel expression");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  double* d_theta;
+  if ((rc = upload_theta(ctx, kp, theta, &d_theta, "large_predict_assemble: theta buffer"))) return rc;
+  PredAsmArgs a;
+  a.kp = kp; a.theta = d_theta; a.x = x; a.xstar = xstar; a.N = p->N; a.M = M; a.m_tiles = pred_m_tiles(M);
+  a.world = p->world; a.rank = p->rank; a.R = R;
+  const long long n_local_ct = p->n_local_blockcols * LG_BT;
+  for (long long y0 = 0; y0 < n_local_ct; y0 += 65535) {      // grid.y is limited to 65535
+    a.lct0 = y0;
+    const dim3 grid((unsigned)((a.m_tiles + 7) / 8), (unsigned)std::min<long long>(65535, n_local_ct - y0));
+    cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+    dispatch_kid(match_fast_kernel(kp), [&](auto kid) {
+      large_pred_assemble_kernel<decltype(kid)::value><<<grid, 256, 0, cngp_ctx_stream(ctx)>>>(a);
+    });
+    cngp_ctx_end(ctx);
+  }
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_predict_panel(cngp_ctx* ctx, const cngp_large_plan* p, const double* A, const double* winv,
+                                        const double* R, int64_t M, int64_t k, double* payload, double* s) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !A || !winv || !R || !payload || !s || M <= 0 || k < 0 || k >= p->n_blockcols)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_predict_panel: bad argument");
+  if (k % p->world != p->rank) return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_predict_panel: not the owner of this block column");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t st = cngp_ctx_stream(ctx);
+  const long long l = k / p->world, mt = pred_m_tiles(M), NT = p->n_pad / 8, r0 = (k + 1) * LG_BT;
+  // W_k = R(:, k) inv(L_kk)^T: the panel product of large_gemm_kernel (mode 0) with the test rows as the panel rows
+  GemmArgs g;
+  memset(&g, 0, sizeof g);
+  g.X = R + l * LG_BT * mt * 64; g.x_kstride = mt * 64;
+  g.Y = winv + l * LG_BT * LG_BT * 64; g.y_kstride = (long long)LG_BT * 64;
+  g.panel = payload; g.pg.r0 = 0; g.pg.row_tiles = mt; g.pg.cs = 0;
+  g.mode = 0; g.world = p->world; g.rank = p->rank;
+  LCU(ctx, cudaFuncSetAttribute(large_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_SMEM));
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_gemm_kernel<<<dim3((unsigned)(mt / LG_BLK), LG_BT / LG_BLK), LG_THREADS, LG_SMEM, st>>>(g);
+  cngp_ctx_end(ctx);
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_pred_sumsq_kernel<<<(unsigned)((mt + 7) / 8), 256, 0, st>>>(payload, mt, M, s + k * M);
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  // L(rows below the diagonal block, k) from A behind W_k, without the y / z row tile: [k-tile][row tile - r0]
+  if (NT > r0) {
+    const long long cstride = p->row_tiles * 64;
+    LCU(ctx, cudaMemcpy2DAsync(payload + (long long)LG_BT * mt * 64, (size_t)(NT - r0) * 512, A + l * LG_BT * cstride + r0 * 64,
+                               (size_t)cstride * 8, (size_t)(NT - r0) * 512, LG_BT, cudaMemcpyDeviceToDevice, st));
+  }
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_predict_update(cngp_ctx* ctx, const cngp_large_plan* p, double* R, int64_t M, int64_t k,
+                                         const double* payload, int64_t c_lo, int64_t c_hi) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !R || !payload || M <= 0 || k < 0 || k >= p->n_blockcols)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_predict_update: bad argument");
+  c_lo = std::max<int64_t>(c_lo, k + 1);
+  c_hi = std::min<int64_t>(c_hi, p->n_blockcols);
+  if (c_lo >= c_hi) return CNGP_OK;
+  const long long l_lo = local_index_of(c_lo, p->world, p->rank), l_hi = local_index_of(c_hi, p->world, p->rank);
+  if (l_lo >= l_hi) return CNGP_OK;
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  const long long mt = pred_m_tiles(M), NT = p->n_pad / 8, r0 = (k + 1) * LG_BT;
+  PredUpdArgs a;
+  a.W = payload; a.w_kstride = mt * 64;
+  a.Lp = payload + (long long)LG_BT * mt * 64 - r0 * 64; a.l_kstride = (NT - r0) * 64;
+  a.R = R; a.r_cstride = mt * 64;
+  a.world = p->world; a.rank = p->rank;
+  LCU(ctx, cudaFuncSetAttribute(large_pred_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_SMEM));
+  const long long ncb = (l_hi - l_lo) * (LG_BT / LG_BLK);
+  for (long long y0 = 0; y0 < ncb; y0 += 65535) {
+    a.lcb0 = (int)(l_lo * (LG_BT / LG_BLK) + y0);
+    const unsigned ny = (unsigned)std::min<long long>(65535, ncb - y0);
+    cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+    large_pred_update_kernel<<<dim3((unsigned)(mt / LG_BLK), ny), LG_THREADS, LG_SMEM, cngp_ctx_stream(ctx)>>>(a);
+    cngp_ctx_end(ctx);
+  }
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_predict_finish(cngp_ctx* ctx, const cngp_large_plan* p, const cngp_kernel* kernel,
+                                         const double* theta, const double* x, const double* alpha, const double* xstar,
+                                         int64_t M, const double* s, double* mean, double* var) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !kernel || !theta || !x || !alpha || !xstar || !s || !mean || !var || M <= 0)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_predict_finish: bad argument");
+  KProg kp;
+  int rc = cngp_build_kprog(kernel, &kp);
+  if (rc) return cngp_set_error(ctx, rc, "large_predict_finish: invalid kernel expression");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  double* d_theta;
+  if ((rc = upload_theta(ctx, kp, theta, &d_theta, "large_predict_finish: theta buffer"))) return rc;
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  dispatch_kid(match_fast_kernel(kp), [&](auto kid) {
+    large_pred_finish_kernel<decltype(kid)::value><<<(unsigned)((M + 7) / 8), 256, 0, cngp_ctx_stream(ctx)>>>(
+        kp, d_theta, x, alpha, p->N, xstar, M, s, p->n_blockcols, mean, var);
+  });
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
 namespace {
 struct DevMem {
   void* p = nullptr;
@@ -914,4 +1193,90 @@ extern "C" int cngp_chol_large(cngp_ctx* ctx, const cngp_kernel* kernel, const d
   if (quad) *quad = bad ? nanv : sums[1];
   if (lml) *lml = bad ? nanv : 0.5 * (-(double)N * CNGP_LOG_2PI - sums[0] - sums[1]);
   return bad ? (int)sums[2] : CNGP_OK;
+}
+
+extern "C" int cngp_chol_large_predict(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, const double* x,
+                                       const double* y, int64_t N, const double* xstar, int64_t M, double* mean,
+                                       double* var, double* logdet, double* quad, double* lml, int32_t mem) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!kernel || !theta || !x || !y || !xstar || !mean || !var || N <= 0 || M <= 0)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "chol_large_predict: bad argument");
+  cngp_large_plan p;
+  cngp_large_make_plan(N, 1, 0, &p);
+  int64_t r_doubles, payload_doubles, s_doubles;
+  cngp_large_predict_sizes(&p, M, 0, &r_doubles, &payload_doubles, &s_doubles);
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t s = cngp_ctx_stream(ctx);
+  DevMem dA, dP, dW, dld, dst, dz, dal, dsum, dx, dy, dsa, dxs, dR, dpay, ds, dmean, dvar;
+  if (!dA.alloc(sizeof(double) * p.local_doubles) || !dP.alloc(sizeof(double) * p.panel_doubles) ||
+      !dW.alloc(sizeof(double) * p.winv_doubles) || !dld.alloc(sizeof(double) * p.n_blockcols) ||
+      !dst.alloc(sizeof(int) * p.n_blockcols) || !dz.alloc(sizeof(double) * p.n_pad) ||
+      !dal.alloc(sizeof(double) * p.n_pad) || !dsum.alloc(sizeof(double) * 4) || !dsa.alloc(sizeof(double) * p.n_pad) ||
+      !dR.alloc(sizeof(double) * r_doubles) || !dpay.alloc(sizeof(double) * payload_doubles) ||
+      !ds.alloc(sizeof(double) * s_doubles))
+    return cngp_set_error(ctx, CNGP_ERR_NOMEM, "chol_large_predict: device allocation failed");
+  const double *d_x = x, *d_y = y, *d_xs = xstar;
+  double *d_mean = mean, *d_var = var;
+  if (mem == CNGP_MEM_HOST) {
+    if (!dx.alloc(sizeof(double) * N) || !dy.alloc(sizeof(double) * N) || !dxs.alloc(sizeof(double) * M) ||
+        !dmean.alloc(sizeof(double) * M) || !dvar.alloc(sizeof(double) * M))
+      return cngp_set_error(ctx, CNGP_ERR_NOMEM, "chol_large_predict: device allocation failed");
+    LCU(ctx, cudaMemcpyAsync(dx.p, x, sizeof(double) * N, cudaMemcpyHostToDevice, s));
+    LCU(ctx, cudaMemcpyAsync(dy.p, y, sizeof(double) * N, cudaMemcpyHostToDevice, s));
+    LCU(ctx, cudaMemcpyAsync(dxs.p, xstar, sizeof(double) * M, cudaMemcpyHostToDevice, s));
+    d_x = (const double*)dx.p; d_y = (const double*)dy.p; d_xs = (const double*)dxs.p;
+    d_mean = (double*)dmean.p; d_var = (double*)dvar.p;
+  }
+  // the factorisation and the backward sweep of cngp_chol_large
+  int rc = cngp_large_assemble(ctx, &p, kernel, theta, d_x, d_y, (double*)dA.p);
+  if (rc) return rc;
+  LCU(ctx, cudaMemsetAsync(dP.p, 0, sizeof(double) * p.panel_doubles, s));
+  for (int64_t k = 0; k < p.n_blockcols; ++k) {
+    if ((rc = cngp_large_factor_panel(ctx, &p, (double*)dA.p, k, (double*)dP.p, (double*)dW.p, (double*)dld.p, (int*)dst.p))) return rc;
+    if ((rc = cngp_large_update(ctx, &p, (double*)dA.p, k, (const double*)dP.p, k + 1, p.n_blockcols))) return rc;
+  }
+  if ((rc = cngp_large_reduce(ctx, &p, (const double*)dA.p, (const double*)dld.p, (const int*)dst.p, (double*)dz.p, (double*)dsum.p))) return rc;
+  double sums[3];
+  LCU(ctx, cudaMemcpyAsync(sums, dsum.p, sizeof sums, cudaMemcpyDeviceToHost, s));
+  LCU(ctx, cudaStreamSynchronize(s));
+  const double nanv = std::nan("");
+  if (sums[2] != 0.0) {                      // not positive definite: nothing below reads the broken factor
+    if (logdet) *logdet = nanv;
+    if (quad) *quad = nanv;
+    if (lml) *lml = nanv;
+    if (mem == CNGP_MEM_HOST) {
+      std::fill(mean, mean + M, nanv);
+      std::fill(var, var + M, nanv);
+    } else {
+      std::vector<double> nans((size_t)M, nanv);
+      LCU(ctx, cudaMemcpyAsync(mean, nans.data(), sizeof(double) * M, cudaMemcpyHostToDevice, s));
+      LCU(ctx, cudaMemcpyAsync(var, nans.data(), sizeof(double) * M, cudaMemcpyHostToDevice, s));
+      LCU(ctx, cudaStreamSynchronize(s));
+    }
+    return (int)sums[2];
+  }
+  LCU(ctx, cudaMemsetAsync(dal.p, 0, sizeof(double) * p.n_pad, s));
+  LCU(ctx, cudaMemsetAsync(dsa.p, 0, sizeof(double) * p.n_pad, s));
+  for (int64_t j = p.n_blockcols - 1; j >= 0; --j) {
+    if ((rc = cngp_large_backsolve_finish(ctx, &p, (const double*)dW.p, j, (const double*)dz.p, (const double*)dsa.p, (double*)dal.p))) return rc;
+    if ((rc = cngp_large_backsolve_apply(ctx, &p, (const double*)dA.p, j, (const double*)dal.p, (double*)dsa.p))) return rc;
+  }
+  // the predict pass, block column by block column (one rank: no look-ahead needed)
+  if ((rc = cngp_large_predict_assemble(ctx, &p, kernel, theta, d_x, d_xs, M, (double*)dR.p))) return rc;
+  for (int64_t k = 0; k < p.n_blockcols; ++k) {
+    if ((rc = cngp_large_predict_panel(ctx, &p, (const double*)dA.p, (const double*)dW.p, (const double*)dR.p, M, k,
+                                       (double*)dpay.p, (double*)ds.p))) return rc;
+    if ((rc = cngp_large_predict_update(ctx, &p, (double*)dR.p, M, k, (const double*)dpay.p, k + 1, p.n_blockcols))) return rc;
+  }
+  if ((rc = cngp_large_predict_finish(ctx, &p, kernel, theta, d_x, (const double*)dal.p, d_xs, M, (const double*)ds.p,
+                                      d_mean, d_var))) return rc;
+  if (mem == CNGP_MEM_HOST) {
+    LCU(ctx, cudaMemcpyAsync(mean, d_mean, sizeof(double) * M, cudaMemcpyDeviceToHost, s));
+    LCU(ctx, cudaMemcpyAsync(var, d_var, sizeof(double) * M, cudaMemcpyDeviceToHost, s));
+  }
+  LCU(ctx, cudaStreamSynchronize(s));
+  if (logdet) *logdet = sums[0];
+  if (quad) *quad = sums[1];
+  if (lml) *lml = 0.5 * (-(double)N * CNGP_LOG_2PI - sums[0] - sums[1]);
+  return CNGP_OK;
 }

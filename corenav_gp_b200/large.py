@@ -189,6 +189,62 @@ class LargeWindow:
     def alpha_block(self, j: int):
         return self.alpha[j * self.nb:(j + 1) * self.nb]
 
+    # ---- the engine interface used by predict_large_distributed ----
+    def _pred_sizes(self, M: int, k: int):
+        r, pay, s = C.c_int64(), C.c_int64(), C.c_int64()
+        rc = self.lib.cngp_large_predict_sizes(C.byref(self.plan), M, k, C.byref(r), C.byref(pay), C.byref(s))
+        if rc != 0:
+            raise CngpError(f"cngp_large_predict_sizes(M={M}, k={k}) failed (rc={rc})")
+        return int(r.value), int(pay.value), int(s.value)
+
+    def predict_begin(self, xstar):
+        """R = K(x*, x) for this rank's block columns, s = 0.  R, the two payload buffers (payload k+1 is formed while
+        the update with payload k still reads it) and s are allocated on first use and kept while M does not grow."""
+        self._bind()
+        dev = self.x.device
+        self.xstar = torch.as_tensor(xstar, dtype=torch.float64).to(dev).contiguous().reshape(-1)
+        self.M = M = int(self.xstar.numel())
+        r, pay, s = self._pred_sizes(M, 0)
+        f64 = dict(dtype=torch.float64, device=dev)
+        if getattr(self, "R", None) is None or self.R.numel() < max(1, r) or self.payloads[0].numel() < pay:
+            self.R = torch.empty(max(1, r), **f64)
+            self.payloads = [torch.empty(pay, **f64) for _ in range(2)]
+        self.s = torch.zeros(s, **f64)
+        self._chk(self.lib.cngp_large_predict_assemble(self.ctx.h, C.byref(self.plan), C.byref(self.kernel),
+                                                       self.theta.ctypes.data, self.x.data_ptr(), self.xstar.data_ptr(),
+                                                       M, self.R.data_ptr()), "cngp_large_predict_assemble")
+
+    def predict_payload(self, k: int):
+        """[W_k ; L(rows below the diagonal block, k)]: what the owner of k broadcasts."""
+        return self.payloads[k % 2][: self._pred_sizes(self.M, k)[1]]
+
+    def predict_panel(self, k: int):
+        self._bind()
+        self._chk(self.lib.cngp_large_predict_panel(self.ctx.h, C.byref(self.plan), self.A.data_ptr(), self.winv.data_ptr(),
+                                                    self.R.data_ptr(), self.M, k, self.payloads[k % 2].data_ptr(),
+                                                    self.s.data_ptr()), "cngp_large_predict_panel")
+
+    def predict_update(self, k: int, c_lo: int, c_hi: int):
+        self._bind()
+        self._chk(self.lib.cngp_large_predict_update(self.ctx.h, C.byref(self.plan), self.R.data_ptr(), self.M, k,
+                                                     self.payloads[k % 2].data_ptr(), c_lo, c_hi),
+                  "cngp_large_predict_update")
+
+    def predict_sums(self):
+        """s [n_blockcols * M]: this rank's rows of the per-block-column sums of W^2, zero elsewhere."""
+        return self.s
+
+    def predict_finish(self):
+        """-> (mean [M], var [M]) from alpha and the rank-summed s."""
+        self._bind()
+        mean = torch.empty(self.M, dtype=torch.float64, device=self.x.device)
+        var = torch.empty_like(mean)
+        self._chk(self.lib.cngp_large_predict_finish(self.ctx.h, C.byref(self.plan), C.byref(self.kernel),
+                                                     self.theta.ctypes.data, self.x.data_ptr(), self.alpha.data_ptr(),
+                                                     self.xstar.data_ptr(), self.M, self.s.data_ptr(), mean.data_ptr(),
+                                                     var.data_ptr()), "cngp_large_predict_finish")
+        return mean, var
+
 
 class TorchCollectives:
     """broadcast / all-reduce through torch.distributed (NCCL for CUDA tensors, gloo for CPU tensors)."""
@@ -207,13 +263,27 @@ class TorchCollectives:
 
 
 class NoCollectives:
-    """world == 1."""
+    """world == 1.  A broadcast moves nothing, but its wait() still orders the stream that waits after the stream that
+    produced the payload, as NCCL's does: the two-stream schedule forms panel k+1 on the chain stream, and the trailing
+    update on the main stream must not read it earlier."""
 
     class _Done:
         def wait(self):
             return True
 
+    class _Ready:
+        def __init__(self, ev):
+            self.ev = ev
+
+        def wait(self):
+            torch.cuda.current_stream().wait_event(self.ev)
+            return True
+
     def broadcast_async(self, t, src: int):
+        if torch is not None and isinstance(t, torch.Tensor) and t.is_cuda:
+            ev = torch.cuda.Event()
+            ev.record()                                          # the payload is complete here on the current stream
+            return self._Ready(ev)
         return self._Done()
 
     def all_reduce_sum(self, t):
@@ -393,6 +463,7 @@ def chol_large_distributed(engine, rank: int, world: int, coll=None, want_alpha:
     logdet, quad = float(both[0]), float(both[1])
     pivot = int(round(BIG - float(piv[0]))) if float(piv[0]) > 0 else 0
     res: Dict[str, object] = dict(pivot=pivot)
+    engine.pivot, engine.have_alpha = pivot, False       # what predict_large_distributed may read
     if pivot:
         nan = float("nan")
         res.update(logdet=nan, quad=nan, lml=nan)
@@ -420,6 +491,7 @@ def chol_large_distributed(engine, rank: int, world: int, coll=None, want_alpha:
                     engine.backsolve_step(j)
                 coll.broadcast_async(engine.alpha_block(j), src=j % world).wait()
         res["alpha"] = engine.alpha[: engine.N]
+        engine.have_alpha = True
     pt.mark("end")
     if pt.on:
         res["phase_ms"] = pt.summary()
@@ -427,9 +499,55 @@ def chol_large_distributed(engine, rank: int, world: int, coll=None, want_alpha:
     return res
 
 
+def predict_large_distributed(engine, xstar, rank: int, world: int, coll=None,
+                              lookahead: bool = True) -> Dict[str, object]:
+    """Predictive mean and variance at xstar [M] from `engine`'s stored factor (SPMD: every rank calls this after
+    chol_large_distributed(engine, ..., want_alpha=True); any number of calls may follow one factorisation).
+
+    A forward sweep W = L^-1 K(x, x*) over the block columns, in the shape of the factorisation: the owner of k forms
+    W_k and broadcasts it with L(:, k), every rank updates its own block columns of R = K(x*, x).  With the look-ahead
+    the owner of k+1 brings its block column up to date first and starts the next broadcast before the rest of update k.
+    Returns dict(mean, var, pivot) - identical on every rank and on every world size; if the factorisation found Ky not
+    positive definite (pivot > 0), mean and var are NaN and the factor is not read."""
+    if coll is None:
+        coll = TorchCollectives() if world > 1 else NoCollectives()
+    pivot = getattr(engine, "pivot", None)
+    if pivot is None or not (pivot or getattr(engine, "have_alpha", False)):
+        raise CngpError("predict_large_distributed: the window has not been factored with want_alpha=True")
+    if pivot:
+        nan = torch.full((int(np.prod(np.shape(xstar))),), float("nan"), dtype=torch.float64, device=engine.alpha.device)
+        return dict(mean=nan, var=nan.clone(), pivot=pivot)
+    nblk = engine.n_blockcols
+    engine.predict_begin(xstar)
+    if rank == 0 % world:
+        engine.predict_panel(0)
+    pending = coll.broadcast_async(engine.predict_payload(0), src=0)
+    for k in range(nblk):
+        pending.wait()                                           # payload k is here
+        nxt = k + 1
+        if nxt >= nblk:
+            break
+        if lookahead:
+            if nxt % world == rank:
+                engine.predict_update(k, nxt, nxt + 1)
+                engine.predict_panel(nxt)
+            pending = coll.broadcast_async(engine.predict_payload(nxt), src=nxt % world)   # overlaps the update below
+            engine.predict_update(k, nxt + 1, nblk)
+        else:
+            engine.predict_update(k, nxt, nblk)
+            if nxt % world == rank:
+                engine.predict_panel(nxt)
+            pending = coll.broadcast_async(engine.predict_payload(nxt), src=nxt % world)
+    s = engine.predict_sums()
+    coll.all_reduce_sum(s)                                       # each row comes from one rank: x + 0, exact
+    mean, var = engine.predict_finish()
+    return dict(mean=mean, var=var, pivot=0)
+
+
 def chol_large(ctx: GpContext, kernel, theta, x, y, rank: int = 0, world: int = 1, coll=None, want_alpha: bool = True,
                lookahead: bool = True, chunk_rows: Optional[int] = None) -> Dict[str, object]:
-    """Convenience: build this rank's LargeWindow and run the distributed factorisation."""
+    """Convenience: build this rank's LargeWindow and run the distributed factorisation.  The window is returned as
+    out["window"]: predict_large_distributed(out["window"], xstar, rank, world, coll) predicts from its factor."""
     win = LargeWindow(ctx, kernel, theta, x, y, rank=rank, world=world, chunk_rows=chunk_rows)
     out = chol_large_distributed(win, rank, world, coll=coll, want_alpha=want_alpha, lookahead=lookahead)
     out["window"] = win

@@ -407,6 +407,41 @@ int cngp_large_matvec(cngp_ctx* ctx, const cngp_kernel* kernel, const double* th
 int cngp_chol_large(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, const double* x, const double* y,
                     int64_t N, double* logdet, double* quad, double* lml, double* alpha, int32_t mem);
 
+/* ---- predict on the large window from its stored factor ----
+ * After the factorisation and the backward sweep, A (block columns of L below their diagonal blocks), winv and alpha
+ * are all a predict pass reads, so any number of passes, at any test points x* [M], can follow one factorisation:
+ *   mean = K(x*, x) alpha,   var = max(k(x*, x*) - sum_i W_i^2, 1e-15) + noise,   W = L^-1 K(x, x*)
+ * (cngp_predict_batch's definition).  W is a forward sweep over R = K(x*, x), stored like A with the test points as rows
+ * (M rounded up to a multiple of 128, zero beyond M) and dealt out block-cyclically as A is.  Per block column k:
+ *   owner of k:  cngp_large_predict_panel    W_k = R(:, k) inv(L_kk)^T and L(rows below the diagonal block, k) into one
+ *                                            payload; s[k][m] = sum over the block's columns of W_k(m, .)^2
+ *   all ranks:   broadcast of the payload (by the caller; nothing with one rank)
+ *   all ranks:   cngp_large_predict_update   R(:, c) -= W_k L(c, k)^T for its block columns c in [max(c_lo, k+1), c_hi)
+ * then s is summed over the ranks (zero outside the owners' rows, so the sum is exact) and cngp_large_predict_finish
+ * gives mean and var from alpha (all of it on every rank) and s, adding the s[k] in increasing k.  Every R(:, c) is written
+ * by one rank in increasing k, so the results have the same bits on every world size.  Device pointers except theta. */
+/* Buffer sizes in doubles for M test points: R of this rank, the payload of block column k (k = 0 is the largest), s. */
+int cngp_large_predict_sizes(const cngp_large_plan* plan, int64_t M, int64_t k, int64_t* r_doubles,
+                             int64_t* payload_doubles, int64_t* s_doubles);
+/* R = K(x*, x) for this rank's block columns. */
+int cngp_large_predict_assemble(cngp_ctx* ctx, const cngp_large_plan* plan, const cngp_kernel* kernel, const double* theta,
+                                const double* x, const double* xstar, int64_t M, double* R);
+/* Owner of block column k: payload = [W_k ; L(rows > k, k)] ([k-tile][row tile] each), s[k][0 .. M). */
+int cngp_large_predict_panel(cngp_ctx* ctx, const cngp_large_plan* plan, const double* A, const double* winv,
+                             const double* R, int64_t M, int64_t k, double* payload, double* s);
+int cngp_large_predict_update(cngp_ctx* ctx, const cngp_large_plan* plan, double* R, int64_t M, int64_t k,
+                              const double* payload, int64_t c_lo, int64_t c_hi);
+/* mean, var [M] from alpha [n_pad] and the rank-summed s [n_blockcols][M]. */
+int cngp_large_predict_finish(cngp_ctx* ctx, const cngp_large_plan* plan, const cngp_kernel* kernel, const double* theta,
+                              const double* x, const double* alpha, const double* xstar, int64_t M, const double* s,
+                              double* mean, double* var);
+/* The whole single-GPU sequence: cngp_chol_large's factorisation, then the predict pass at xstar [M].  x, y, xstar,
+ * mean, var follow `mem`; logdet/quad/lml are HOST scalars (may be NULL).  Returns CNGP_OK, or the failing pivot as in
+ * cngp_chol_large - then mean, var, logdet, quad and lml are NaN. */
+int cngp_chol_large_predict(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, const double* x,
+                            const double* y, int64_t N, const double* xstar, int64_t M, double* mean, double* var,
+                            double* logdet, double* quad, double* lml, int32_t mem);
+
 #ifdef __cplusplus
 }
 #endif
