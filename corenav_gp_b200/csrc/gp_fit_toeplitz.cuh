@@ -26,11 +26,16 @@ namespace cngp {
 constexpr int TOEP_WARPS = 4;                 // windows per CTA
 constexpr int TOEP_SLOTS = CNGP_MAX_N / 32;   // row slots per lane
 static_assert(CNGP_MAX_N % 32 == 0, "rows are dealt over the 32 lanes");
-// Conditioning guard.  The Schur recursion is as accurate as the Cholesky factorisation only while Ky is well
-// conditioned; its error grows faster with cond(Ky).  min_k L_kk^2 / t0 tracks 1 / cond: 0.11 to 0.14 for rbf,
-// rbf+stdperiodic, mat32+bias and ratquad+stdperiodic*rbf at noise 1e-3 (the benchmark window: cond 750), 6.5e-3 for
-// mat52+white at noise 1e-3 (cond 1.6e4, where the Schur predictive mean is 1.1e-10 away from the tile Cholesky's -
-// measured on a B200), 1e-4 for stdperiodic at noise 1e-4 (cond 2e6).  Windows below the guard go to the tile Cholesky.
+// Conditioning guard.  min_k L_kk^2 / t0 tracks 1 / cond(Ky): 0.11 to 0.14 for rbf, rbf+stdperiodic, mat32+bias and
+// ratquad+stdperiodic*rbf at noise 1e-3 (the benchmark window: cond 750), 6.5e-3 for mat52+white at noise 1e-3
+// (cond 1.6e4), 1e-3 for stdperiodic at noise 1e-3.  Just above the guard (ratio 1.5e-2; lengthscales x1 to x100,
+// N = 100 and 256) the Schur fit, the variance recurrence and the shared-covariance group are within 1.4e-13 of a float80
+// exact GP in mean, 1.4e-14 in variance and 1.9e-13 in LML (max(1, |ref|) relative; the tile Cholesky: 1.1e-13, 1.4e-15,
+// 1.1e-12), and the gradients they feed are as close as the tile path's - measured on a B200 by
+// tests/test_gpu_toeplitz_conditioning.py.  (The 1e-10 gaps between the Schur and the tile mean seen with a metric
+// floored at 1e-3 max|mean| are both paths' rounding on a tail that decays to zero, not an error.)  Below the guard the
+// windows take the tile Cholesky; the guard keeps the ill-conditioned ones (cond 1e6 and beyond) on the path whose
+// jitter ladder and status codes handle them.
 constexpr double TOEP_MIN_PIVOT2 = 1e-2;
 
 // stage stride: one column of the staged half tile column, rows rounded up to the 32 lanes
