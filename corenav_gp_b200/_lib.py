@@ -119,7 +119,16 @@ SIGNATURES = {
                                             c_dp, c_dp, c_dp]),
     "cngp_chol_large_predict": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_dp, c_dp, c_i64, c_dp, c_i64, c_dp, c_dp, c_dp,
                                           c_dp, c_dp, c_i32]),
+    "cngp_large_grad_sizes": (C.c_int, [C.POINTER(LargePlan), C.POINTER(c_i64), C.POINTER(c_i64), C.POINTER(c_i64)]),
+    "cngp_large_grad_begin": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp]),
+    "cngp_large_grad_panel": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_dp, c_dp, c_i64, c_dp]),
+    "cngp_large_grad_update": (C.c_int, [c_vp, C.POINTER(LargePlan), c_dp, c_i64, c_dp, c_i64, c_i64]),
+    "cngp_large_grad_contract": (C.c_int, [c_vp, C.POINTER(LargePlan), C.POINTER(Kernel), c_dp, c_dp, c_dp, c_dp, c_dp]),
+    "cngp_large_grad_finish": (C.c_int, [c_vp, C.POINTER(LargePlan), C.POINTER(Kernel), c_dp, c_dp]),
+    "cngp_chol_large_grad": (C.c_int, [c_vp, C.POINTER(Kernel), c_dp, c_dp, c_dp, c_i64, c_dp, c_dp, c_dp, c_dp, c_i32]),
 }
+
+LARGE_GRAD_STRIDE = MAX_PARAMS + 1   # row length of the gradient parts (cngp_large_grad_sizes)
 
 _lib = None
 

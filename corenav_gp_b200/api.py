@@ -568,6 +568,28 @@ class GpContext:
             self._check(rc, "cngp_chol_large_predict")
         return dict(mean=mean, var=var, logdet=float(outs[0]), quad=float(outs[1]), lml=float(outs[2]), pivot=int(rc))
 
+    def chol_large_grad(self, kernel, theta, x, y):
+        """chol_large, then the gradient of the LML with respect to theta [P] (natural parameters, noise last) from the
+        factor: GPy's ExactGaussianInference dL_dK with kern.update_gradients_full, as lml_grad.  x, y: host arrays or
+        CUDA tensors, alike; grad follows them.  Returns dict(lml, grad, logdet, quad, pivot): pivot = 0, or the (1-based)
+        pivot at which Ky was found not positive definite - then every other value is NaN."""
+        k = parse_kernel(kernel)
+        dev = _is_cuda(x)
+        N = int(np.prod(tuple(x.shape)))
+        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
+        if th.size != k.n_params + 1:
+            raise CngpError(f"theta has {th.size} entries, kernel needs {k.n_params + 1} (noise last)")
+        outs = np.empty(3)
+        grad = self._empty((th.size,), np.float64, dev)
+        a = [_Arg(x, np.float64, dev), _Arg(y, np.float64, dev), _Arg(grad, np.float64, dev, output=True)]
+        self._bind_stream(dev)
+        rc = self.lib.cngp_chol_large_grad(self.h, C.byref(k), th.ctypes.data, a[0].ptr, a[1].ptr, N, outs.ctypes.data,
+                                           outs.ctypes.data + 8, outs.ctypes.data + 16, a[2].ptr,
+                                           L.MEM_DEVICE if dev else L.MEM_HOST)
+        if rc < 0:
+            self._check(rc, "cngp_chol_large_grad")
+        return dict(lml=float(outs[2]), grad=grad, logdet=float(outs[0]), quad=float(outs[1]), pivot=int(rc))
+
     def large_matvec(self, kernel, theta, x, v):
         """r = (K(x,x) + (noise + 1e-8) I) v evaluated on the fly on the device; x, v CUDA tensors [N]."""
         k = parse_kernel(kernel)

@@ -20,6 +20,9 @@
 //  * predict pass (after the factorisation, reading only A, winv and alpha): W = L^-1 K(x, x*) as a forward sweep over
 //    R = K(x*, x) in the same block-cyclic shape - the owner forms W_k with the panel product, every rank updates its
 //    block columns of R with the same CTA body as the trailing update (cngp.h, cngp_large_predict_*).
+//  * gradient pass (after the factorisation, reading the same A, winv and alpha): the predict sweep with R = I gives V = L^-T block column by block column,
+//    and every rank accumulates its block columns of Ky^-1 = sum_k V_k V_k^T with the trailing update's kernel, then
+//    contracts them against dK/dtheta evaluated in registers (cngp.h, cngp_large_grad_*).
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -31,6 +34,7 @@
 
 #include "cngp_internal.h"
 #include "gp_fit.cuh"
+#include "gp_grad.cuh"
 
 using namespace cngp;
 
@@ -635,6 +639,155 @@ __global__ void __launch_bounds__(256) large_pred_finish_kernel(KProg kp, const 
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// LML gradient pass over the stored factor: V = L^-T as the forward sweep of the predict pass with R = I
+// ------------------------------------------------------------------------------------------------------------
+// RG is stored like A but with NT = n_pad/8 row tiles per column tile: tile (rt, lct) at RG[(lct * NT + rt) * 64].  Block
+// column c holds R(:, c) until W_c = V_c is formed from it, and G(:, c) = -(sum_{k >= c} V_k V_k^T)(:, c) after that (kept
+// negated so that the accumulation is the subtracting CTA body of the trailing update): the two never live at once.
+constexpr int GRAD_STRIDE = CNGP_MAX_PARAMS + 1;    // one gradient row: kernel parameters, noise in the slot P - 1
+
+// R = I on this rank's block columns (the storage is zero-filled beforehand); one thread per local column tile
+__global__ void __launch_bounds__(256) large_grad_identity_kernel(double* RG, long long NT, long long n_lct, int world, int rank) {
+  const long long lct = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (lct >= n_lct) return;
+  const long long gct = ((lct / LG_BT) * world + rank) * LG_BT + lct % LG_BT;
+  double* t = RG + (lct * NT + gct) * 64;
+  for (int i = 0; i < 8; ++i) t[i * 9] = 1.0;
+}
+
+// One entry of dL/dK (weight wgt, mirrored entry included) against dK/dtheta at (xa, xb), gp_grad_kernel's sum and product
+// rules: each leaf's derivatives times the values of the other leaves of its product term.  Expressions of up to
+// GRAD_FAST_LEAVES leaves accumulate per leaf (gl), larger ones straight into the parameter slots (g).
+__device__ __forceinline__ void large_grad_entry(const KProg& kp, const double* thv, const GradConst* gcs, const int* lt0,
+                                                 const int* lt1, double wgt, double xa, double xb, double r2, bool same,
+                                                 double (&gl)[GRAD_FAST_LEAVES][3], double (&g)[GRAD_STRIDE]) {
+  if (kp.n_leaves <= GRAD_FAST_LEAVES) {
+#pragma unroll
+    for (int ul = 0; ul < GRAD_FAST_LEAVES; ++ul) {
+      if (ul < kp.n_leaves) {
+        double others = 1.0, dv[3];
+        for (int u2 = lt0[ul]; u2 < lt1[ul]; ++u2)
+          if (u2 != ul) others *= leaf_value_grad_c<true>(kp.leaf_type[u2], thv + kp.leaf_param[u2], gcs[u2], xa, xb, r2, same, dv);
+        leaf_value_grad_c<true>(kp.leaf_type[ul], thv + kp.leaf_param[ul], gcs[ul], xa, xb, r2, same, dv);
+        const double ww = wgt * others;
+        gl[ul][0] += ww * dv[0]; gl[ul][1] += ww * dv[1]; gl[ul][2] += ww * dv[2];
+      }
+    }
+  } else {
+    for (int u = 0; u < kp.n_leaves; ++u) {
+      double others = 1.0, dv[3];
+      for (int u2 = lt0[u]; u2 < lt1[u]; ++u2)
+        if (u2 != u) others *= leaf_value_grad_c<true>(kp.leaf_type[u2], thv + kp.leaf_param[u2], gcs[u2], xa, xb, r2, same, dv);
+      leaf_value_grad_c<true>(kp.leaf_type[u], thv + kp.leaf_param[u], gcs[u], xa, xb, r2, same, dv);
+      const int np = leaf_nparams(kp.leaf_type[u]), po = kp.leaf_param[u];
+      const double ww = wgt * others;
+#pragma unroll
+      for (int i = 0; i < CNGP_MAX_PARAMS; ++i) {
+        const int jj = i - po;
+        if (jj >= 0 && jj < np) g[i] += ww * (jj == 0 ? dv[0] : (jj == 1 ? dv[1] : dv[2]));
+      }
+    }
+  }
+}
+
+// partial[lct][p] = sum over the entries i >= j (i, j < N) of local column tile lct of  w_ij dK_ij/dtheta_p,
+// w_ij = alpha_i alpha_j + G_ij (G = -Ky^-1), doubled off the diagonal; the noise slot gets the diagonal weights.
+// One CTA per column tile, warp w takes row tiles gct + w, gct + w + 8, ...; the sums are reduced in a fixed order.
+constexpr int GC_WARPS = 8;
+__global__ void __launch_bounds__(GC_WARPS * 32) large_grad_contract_kernel(const KProg kp, const double* theta, const double* x,
+                                                                            const double* alpha, const double* RG, long long N,
+                                                                            long long NT, int world, int rank, double* partial) {
+  __shared__ double thv[GRAD_STRIDE];
+  __shared__ GradConst gcs[CNGP_MAX_LEAVES];
+  __shared__ int lt0[CNGP_MAX_LEAVES], lt1[CNGP_MAX_LEAVES];
+  __shared__ double gred[GC_WARPS][GRAD_STRIDE];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, r = lane >> 2, q = lane & 3;
+  const int P = kp.n_params + 1;
+  if (tid < P) thv[tid] = theta[tid];
+  if (tid < kp.n_leaves) gcs[tid] = grad_prepare(kp.leaf_type[tid], theta + kp.leaf_param[tid]);
+  if (tid < kp.n_terms)
+    for (int u = kp.term_start[tid]; u < kp.term_start[tid + 1]; ++u) { lt0[u] = kp.term_start[tid]; lt1[u] = kp.term_start[tid + 1]; }
+  __syncthreads();
+  const long long lct = blockIdx.x;
+  const long long gct = ((lct / LG_BT) * world + rank) * LG_BT + lct % LG_BT;
+  double g[GRAD_STRIDE];
+#pragma unroll
+  for (int i = 0; i < GRAD_STRIDE; ++i) g[i] = 0.0;
+  double gl[GRAD_FAST_LEAVES][3];
+#pragma unroll
+  for (int i = 0; i < GRAD_FAST_LEAVES; ++i) gl[i][0] = gl[i][1] = gl[i][2] = 0.0;
+  const long long j0 = 8 * gct + 2 * q;
+  const double xb0 = j0 < N ? x[j0] : 0.0, xb1 = j0 + 1 < N ? x[j0 + 1] : 0.0;
+  const double ab0 = j0 < N ? alpha[j0] : 0.0, ab1 = j0 + 1 < N ? alpha[j0 + 1] : 0.0;
+  const long long rt_end = min(NT, (N + 7) / 8);
+  for (long long rt = gct + w; rt < rt_end; rt += GC_WARPS) {
+    const double2 v = *reinterpret_cast<const double2*>(RG + (lct * NT + rt) * 64 + 2 * lane);
+    const long long i = 8 * rt + r;
+    if (i >= N) continue;
+    const double xa = x[i], ai = alpha[i];
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const long long j = j0 + e;
+      if (j > i || j >= N) continue;
+      const bool same = i == j;
+      double wgt = ai * (e ? ab1 : ab0) + (e ? v.y : v.x);
+      if (!same) wgt += wgt;
+      const double xb = e ? xb1 : xb0;
+      const double r2 = same ? 0.0 : r2_expanded(xa, xb);
+      if (same) g[CNGP_MAX_PARAMS] += wgt;                 // noise: trace(dL_dK)
+      large_grad_entry(kp, thv, gcs, lt0, lt1, wgt, xa, xb, r2, same, gl, g);
+    }
+  }
+  if (kp.n_leaves <= GRAD_FAST_LEAVES) {
+#pragma unroll
+    for (int ul = 0; ul < GRAD_FAST_LEAVES; ++ul) {
+      if (ul < kp.n_leaves) {
+        const int np = leaf_nparams(kp.leaf_type[ul]), po = kp.leaf_param[ul];
+#pragma unroll
+        for (int i = 0; i < CNGP_MAX_PARAMS; ++i) {
+          const int jj = i - po;
+          if (jj >= 0 && jj < np) g[i] += (jj == 0 ? gl[ul][0] : (jj == 1 ? gl[ul][1] : gl[ul][2]));
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < GRAD_STRIDE; ++i) {
+    double v = g[i];
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) gred[w][i] = v;
+  }
+  __syncthreads();
+  if (tid < GRAD_STRIDE) {
+    double v = 0.0;
+    if (tid < P) {
+      const int src = tid == P - 1 ? CNGP_MAX_PARAMS : tid;
+      for (int ww = 0; ww < GC_WARPS; ++ww) v += gred[ww][src];
+    }
+    partial[lct * GRAD_STRIDE + tid] = v;
+  }
+}
+
+// part[c][p] = sum over the 32 column tiles of this rank's block column c of partial, in increasing column tile
+__global__ void __launch_bounds__(32) large_grad_part_kernel(const double* partial, int world, int rank, double* part) {
+  const long long l = blockIdx.x, c = l * world + rank;
+  const int p = threadIdx.x;
+  if (p >= GRAD_STRIDE) return;
+  double s = 0.0;
+  for (int t = 0; t < LG_BT; ++t) s += partial[(l * LG_BT + t) * GRAD_STRIDE + p];
+  part[c * GRAD_STRIDE + p] = s;
+}
+
+// grad[p] = 1/2 sum_c part[c][p], c increasing
+__global__ void __launch_bounds__(32) large_grad_finish_kernel(const double* part, long long n_blockcols, int P, double* grad) {
+  const int p = threadIdx.x;
+  if (p >= P) return;
+  double s = 0.0;
+  for (long long c = 0; c < n_blockcols; ++c) s += part[c * GRAD_STRIDE + p];
+  grad[p] = 0.5 * s;
+}
+
 template <typename F>
 void dispatch_kid(int kid, F&& f) {
   switch (kid) {
@@ -657,7 +810,7 @@ int cuda_fail(cngp_ctx* ctx, const char* what, cudaError_t e) {
   } while (0)
 
 // scratch slots of the context used here
-enum { SLOT_THETA = 20, SLOT_LPACK = 21, SLOT_WT = 22, SLOT_Z33 = 23, SLOT_PARTIAL = 24 };
+enum { SLOT_THETA = 20, SLOT_LPACK = 21, SLOT_WT = 22, SLOT_Z33 = 23, SLOT_PARTIAL = 24, SLOT_GPART = 25 };
 
 inline PanelGeom panel_geom(const cngp_large_plan* p, long long k) {
   PanelGeom g;
@@ -1136,6 +1289,170 @@ extern "C" int cngp_large_predict_finish(cngp_ctx* ctx, const cngp_large_plan* p
   return CNGP_OK;
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// LML gradient pass (see cngp.h): the predict sweep with R = I, Ky^-1 accumulated block column by block column
+// ------------------------------------------------------------------------------------------------------------
+extern "C" int cngp_large_grad_sizes(const cngp_large_plan* p, int64_t* rg_doubles, int64_t* payload_doubles,
+                                     int64_t* part_doubles) {
+  if (!p || p->n_blockcols <= 0) return CNGP_ERR_INVALID;
+  if (rg_doubles) *rg_doubles = p->n_local_blockcols * LG_BT * (p->n_pad / 8) * 64;
+  if (payload_doubles) *payload_doubles = (long long)LG_BT * 64 * (p->n_pad / 8);     // [W_k ; L(rows > k, k)], any k
+  if (part_doubles) *part_doubles = p->n_blockcols * GRAD_STRIDE;
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_grad_begin(cngp_ctx* ctx, const cngp_large_plan* p, double* RG) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !RG) return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_begin: bad argument");
+  if (p->n_local_blockcols == 0) return CNGP_OK;
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t st = cngp_ctx_stream(ctx);
+  const long long NT = p->n_pad / 8, n_lct = p->n_local_blockcols * LG_BT;
+  LCU(ctx, cudaMemsetAsync(RG, 0, sizeof(double) * (size_t)(n_lct * NT * 64), st));
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_grad_identity_kernel<<<(unsigned)((n_lct + 255) / 256), 256, 0, st>>>(RG, NT, n_lct, p->world, p->rank);
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_grad_panel(cngp_ctx* ctx, const cngp_large_plan* p, const double* A, const double* winv, double* RG,
+                                     int64_t k, double* payload) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !A || !winv || !RG || !payload || k < 0 || k >= p->n_blockcols)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_panel: bad argument");
+  if (k % p->world != p->rank) return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_panel: not the owner of this block column");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t st = cngp_ctx_stream(ctx);
+  const long long l = k / p->world, NT = p->n_pad / 8, r0 = (k + 1) * LG_BT;
+  double* Rk = RG + l * LG_BT * NT * 64;
+  // W_k = R(rows < 256 (k+1), k) inv(L_kk)^T: the panel product (large_gemm_kernel mode 0), as in cngp_large_predict_panel
+  GemmArgs g;
+  memset(&g, 0, sizeof g);
+  g.X = Rk; g.x_kstride = NT * 64;
+  g.Y = winv + l * LG_BT * LG_BT * 64; g.y_kstride = (long long)LG_BT * 64;
+  g.panel = payload; g.pg.r0 = 0; g.pg.row_tiles = r0; g.pg.cs = 0;
+  g.mode = 0; g.world = p->world; g.rank = p->rank;
+  LCU(ctx, cudaFuncSetAttribute(large_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_SMEM));
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_gemm_kernel<<<dim3((unsigned)(r0 / LG_BLK), LG_BT / LG_BLK), LG_THREADS, LG_SMEM, st>>>(g);
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  // L(rows below the diagonal block, k) behind W_k: [k-tile][row tile - r0]
+  if (NT > r0) {
+    const long long cstride = p->row_tiles * 64;
+    LCU(ctx, cudaMemcpy2DAsync(payload + (long long)LG_BT * r0 * 64, (size_t)(NT - r0) * 512, A + l * LG_BT * cstride + r0 * 64,
+                               (size_t)cstride * 8, (size_t)(NT - r0) * 512, LG_BT, cudaMemcpyDeviceToDevice, st));
+  }
+  // R(:, k) is consumed: block column k becomes G(:, k).  Rows below its diagonal block are zero already (R(:, k) has
+  // none), the diagonal block held R(k, k)
+  LCU(ctx, cudaMemset2DAsync(Rk + k * LG_BT * 64, (size_t)NT * 512, 0, (size_t)LG_BT * 512, LG_BT, st));
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_grad_update(cngp_ctx* ctx, const cngp_large_plan* p, double* RG, int64_t k, const double* payload,
+                                      int64_t c_lo, int64_t c_hi) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !RG || !payload || k < 0 || k >= p->n_blockcols)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_update: bad argument");
+  c_lo = std::max<int64_t>(c_lo, 0);
+  c_hi = std::min<int64_t>(c_hi, p->n_blockcols);
+  if (c_lo >= c_hi) return CNGP_OK;
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t st = cngp_ctx_stream(ctx);
+  const long long NT = p->n_pad / 8, r0 = (k + 1) * LG_BT;
+  const int rbk = (int)(r0 / LG_BLK);                     // 16-tile row blocks of W_k
+  // sweep: R(rows < 256 (k+1), c) -= W_k L(c, k)^T for c > k - large_pred_update_kernel over W_k's rows only
+  {
+    const long long l_lo = local_index_of(std::max<int64_t>(c_lo, k + 1), p->world, p->rank);
+    const long long l_hi = local_index_of(c_hi, p->world, p->rank);
+    if (l_lo < l_hi) {
+      PredUpdArgs a;
+      a.W = payload; a.w_kstride = r0 * 64;
+      a.Lp = payload + (long long)LG_BT * r0 * 64 - r0 * 64; a.l_kstride = (NT - r0) * 64;
+      a.R = RG; a.r_cstride = NT * 64;
+      a.world = p->world; a.rank = p->rank;
+      LCU(ctx, cudaFuncSetAttribute(large_pred_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_SMEM));
+      const long long ncb = (l_hi - l_lo) * (LG_BT / LG_BLK);
+      for (long long y0 = 0; y0 < ncb; y0 += 65535) {
+        a.lcb0 = (int)(l_lo * (LG_BT / LG_BLK) + y0);
+        const unsigned ny = (unsigned)std::min<long long>(65535, ncb - y0);
+        cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+        large_pred_update_kernel<<<dim3((unsigned)rbk, ny), LG_THREADS, LG_SMEM, st>>>(a);
+        cngp_ctx_end(ctx);
+      }
+    }
+  }
+  // accumulation: G(I, J) -= W_k(I) W_k(J)^T for J <= k, J <= I <= k - the trailing update (large_gemm_kernel mode 1) with
+  // W_k as the panel; blocks above the diagonal return at once
+  {
+    const long long l_lo = local_index_of(c_lo, p->world, p->rank);
+    const long long l_hi = local_index_of(std::min<int64_t>(c_hi, k + 1), p->world, p->rank);
+    if (l_lo < l_hi) {
+      const long long c_first = l_lo * p->world + p->rank;
+      GemmArgs g;
+      memset(&g, 0, sizeof g);
+      g.panel = const_cast<double*>(payload); g.pg.r0 = 0; g.pg.row_tiles = r0; g.pg.cs = 0;
+      g.C = RG; g.c_cstride = NT * 64;
+      g.mode = 1; g.rb0 = (int)(c_first * LG_BT / LG_BLK); g.world = p->world; g.rank = p->rank;
+      LCU(ctx, cudaFuncSetAttribute(large_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG_SMEM));
+      const long long ncb = (l_hi - l_lo) * (LG_BT / LG_BLK);
+      for (long long y0 = 0; y0 < ncb; y0 += 65535) {
+        g.lcb0 = (int)(l_lo * (LG_BT / LG_BLK) + y0);
+        const unsigned ny = (unsigned)std::min<long long>(65535, ncb - y0);
+        cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+        large_gemm_kernel<<<dim3((unsigned)(rbk - g.rb0), ny), LG_THREADS, LG_SMEM, st>>>(g);
+        cngp_ctx_end(ctx);
+      }
+    }
+  }
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_grad_contract(cngp_ctx* ctx, const cngp_large_plan* p, const cngp_kernel* kernel, const double* theta,
+                                        const double* x, const double* alpha, const double* RG, double* part) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !kernel || !theta || !x || !alpha || !RG || !part)
+    return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_contract: bad argument");
+  KProg kp;
+  int rc = cngp_build_kprog(kernel, &kp);
+  if (rc) return cngp_set_error(ctx, rc, "large_grad_contract: invalid kernel expression");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  double* d_theta;
+  if ((rc = upload_theta(ctx, kp, theta, &d_theta, "large_grad_contract: theta buffer"))) return rc;
+  cudaStream_t st = cngp_ctx_stream(ctx);
+  LCU(ctx, cudaMemsetAsync(part, 0, sizeof(double) * (size_t)(p->n_blockcols * GRAD_STRIDE), st));
+  const long long n_lct = p->n_local_blockcols * LG_BT;
+  if (n_lct == 0) return CNGP_OK;
+  double* partial = (double*)cngp_ctx_buf(ctx, SLOT_GPART, sizeof(double) * (size_t)(n_lct * GRAD_STRIDE));
+  if (!partial) return cngp_set_error(ctx, CNGP_ERR_NOMEM, "large_grad_contract: scratch");
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_grad_contract_kernel<<<(unsigned)n_lct, GC_WARPS * 32, 0, st>>>(kp, d_theta, x, alpha, RG, p->N, p->n_pad / 8,
+                                                                          p->world, p->rank, partial);
+  cngp_ctx_end(ctx);
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_grad_part_kernel<<<(unsigned)p->n_local_blockcols, 32, 0, st>>>(partial, p->world, p->rank, part);
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
+extern "C" int cngp_large_grad_finish(cngp_ctx* ctx, const cngp_large_plan* p, const cngp_kernel* kernel, const double* part,
+                                      double* grad) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!p || !kernel || !part || !grad) return cngp_set_error(ctx, CNGP_ERR_INVALID, "large_grad_finish: bad argument");
+  KProg kp;
+  int rc = cngp_build_kprog(kernel, &kp);
+  if (rc) return cngp_set_error(ctx, rc, "large_grad_finish: invalid kernel expression");
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cngp_ctx_begin(ctx, CNGP_PROF_LARGE);
+  large_grad_finish_kernel<<<1, 32, 0, cngp_ctx_stream(ctx)>>>(part, p->n_blockcols, kp.n_params + 1, grad);
+  cngp_ctx_end(ctx);
+  LCU(ctx, cudaGetLastError());
+  return CNGP_OK;
+}
+
 namespace {
 struct DevMem {
   void* p = nullptr;
@@ -1274,6 +1591,85 @@ extern "C" int cngp_chol_large_predict(cngp_ctx* ctx, const cngp_kernel* kernel,
     LCU(ctx, cudaMemcpyAsync(mean, d_mean, sizeof(double) * M, cudaMemcpyDeviceToHost, s));
     LCU(ctx, cudaMemcpyAsync(var, d_var, sizeof(double) * M, cudaMemcpyDeviceToHost, s));
   }
+  LCU(ctx, cudaStreamSynchronize(s));
+  if (logdet) *logdet = sums[0];
+  if (quad) *quad = sums[1];
+  if (lml) *lml = 0.5 * (-(double)N * CNGP_LOG_2PI - sums[0] - sums[1]);
+  return CNGP_OK;
+}
+
+extern "C" int cngp_chol_large_grad(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, const double* x,
+                                    const double* y, int64_t N, double* logdet, double* quad, double* lml, double* grad,
+                                    int32_t mem) {
+  if (!ctx) return CNGP_ERR_INVALID;
+  if (!kernel || !theta || !x || !y || !grad || N <= 0) return cngp_set_error(ctx, CNGP_ERR_INVALID, "chol_large_grad: bad argument");
+  KProg kp;
+  int rc = cngp_build_kprog(kernel, &kp);
+  if (rc) return cngp_set_error(ctx, rc, "chol_large_grad: invalid kernel expression");
+  const int P = kp.n_params + 1;
+  cngp_large_plan p;
+  cngp_large_make_plan(N, 1, 0, &p);
+  int64_t rg_doubles, payload_doubles, part_doubles;
+  cngp_large_grad_sizes(&p, &rg_doubles, &payload_doubles, &part_doubles);
+  LCU(ctx, cudaSetDevice(cngp_ctx_device(ctx)));
+  cudaStream_t s = cngp_ctx_stream(ctx);
+  DevMem dA, dP, dW, dld, dst, dz, dal, dsum, dx, dy, dsa, dRG, dpay, dpart, dgrad;
+  if (!dA.alloc(sizeof(double) * p.local_doubles) || !dP.alloc(sizeof(double) * p.panel_doubles) ||
+      !dW.alloc(sizeof(double) * p.winv_doubles) || !dld.alloc(sizeof(double) * p.n_blockcols) ||
+      !dst.alloc(sizeof(int) * p.n_blockcols) || !dz.alloc(sizeof(double) * p.n_pad) ||
+      !dal.alloc(sizeof(double) * p.n_pad) || !dsum.alloc(sizeof(double) * 4) || !dsa.alloc(sizeof(double) * p.n_pad) ||
+      !dRG.alloc(sizeof(double) * rg_doubles) || !dpay.alloc(sizeof(double) * payload_doubles) ||
+      !dpart.alloc(sizeof(double) * part_doubles) || !dgrad.alloc(sizeof(double) * P))
+    return cngp_set_error(ctx, CNGP_ERR_NOMEM, "chol_large_grad: device allocation failed");
+  const double *d_x = x, *d_y = y;
+  if (mem == CNGP_MEM_HOST) {
+    if (!dx.alloc(sizeof(double) * N) || !dy.alloc(sizeof(double) * N))
+      return cngp_set_error(ctx, CNGP_ERR_NOMEM, "chol_large_grad: device allocation failed");
+    LCU(ctx, cudaMemcpyAsync(dx.p, x, sizeof(double) * N, cudaMemcpyHostToDevice, s));
+    LCU(ctx, cudaMemcpyAsync(dy.p, y, sizeof(double) * N, cudaMemcpyHostToDevice, s));
+    d_x = (const double*)dx.p; d_y = (const double*)dy.p;
+  }
+  // the factorisation and the backward sweep of cngp_chol_large
+  if ((rc = cngp_large_assemble(ctx, &p, kernel, theta, d_x, d_y, (double*)dA.p))) return rc;
+  LCU(ctx, cudaMemsetAsync(dP.p, 0, sizeof(double) * p.panel_doubles, s));
+  for (int64_t k = 0; k < p.n_blockcols; ++k) {
+    if ((rc = cngp_large_factor_panel(ctx, &p, (double*)dA.p, k, (double*)dP.p, (double*)dW.p, (double*)dld.p, (int*)dst.p))) return rc;
+    if ((rc = cngp_large_update(ctx, &p, (double*)dA.p, k, (const double*)dP.p, k + 1, p.n_blockcols))) return rc;
+  }
+  if ((rc = cngp_large_reduce(ctx, &p, (const double*)dA.p, (const double*)dld.p, (const int*)dst.p, (double*)dz.p, (double*)dsum.p))) return rc;
+  double sums[3];
+  LCU(ctx, cudaMemcpyAsync(sums, dsum.p, sizeof sums, cudaMemcpyDeviceToHost, s));
+  LCU(ctx, cudaStreamSynchronize(s));
+  const double nanv = std::nan("");
+  if (sums[2] != 0.0) {                      // not positive definite: nothing below reads the broken factor
+    if (logdet) *logdet = nanv;
+    if (quad) *quad = nanv;
+    if (lml) *lml = nanv;
+    std::vector<double> nans((size_t)P, nanv);
+    if (mem == CNGP_MEM_HOST) {
+      std::copy(nans.begin(), nans.end(), grad);
+    } else {
+      LCU(ctx, cudaMemcpyAsync(grad, nans.data(), sizeof(double) * P, cudaMemcpyHostToDevice, s));
+      LCU(ctx, cudaStreamSynchronize(s));
+    }
+    return (int)sums[2];
+  }
+  LCU(ctx, cudaMemsetAsync(dal.p, 0, sizeof(double) * p.n_pad, s));
+  LCU(ctx, cudaMemsetAsync(dsa.p, 0, sizeof(double) * p.n_pad, s));
+  for (int64_t j = p.n_blockcols - 1; j >= 0; --j) {
+    if ((rc = cngp_large_backsolve_finish(ctx, &p, (const double*)dW.p, j, (const double*)dz.p, (const double*)dsa.p, (double*)dal.p))) return rc;
+    if ((rc = cngp_large_backsolve_apply(ctx, &p, (const double*)dA.p, j, (const double*)dal.p, (double*)dsa.p))) return rc;
+  }
+  // the gradient pass, block column by block column (one rank: no look-ahead needed)
+  if ((rc = cngp_large_grad_begin(ctx, &p, (double*)dRG.p))) return rc;
+  for (int64_t k = 0; k < p.n_blockcols; ++k) {
+    if ((rc = cngp_large_grad_panel(ctx, &p, (const double*)dA.p, (const double*)dW.p, (double*)dRG.p, k, (double*)dpay.p))) return rc;
+    if ((rc = cngp_large_grad_update(ctx, &p, (double*)dRG.p, k, (const double*)dpay.p, 0, p.n_blockcols))) return rc;
+  }
+  if ((rc = cngp_large_grad_contract(ctx, &p, kernel, theta, d_x, (const double*)dal.p, (const double*)dRG.p, (double*)dpart.p))) return rc;
+  double* d_grad = mem == CNGP_MEM_HOST ? (double*)dgrad.p : grad;
+  if ((rc = cngp_large_grad_finish(ctx, &p, kernel, (const double*)dpart.p, d_grad))) return rc;
+  if (mem == CNGP_MEM_HOST) LCU(ctx, cudaMemcpyAsync(grad, d_grad, sizeof(double) * P, cudaMemcpyDeviceToHost, s));
   LCU(ctx, cudaStreamSynchronize(s));
   if (logdet) *logdet = sums[0];
   if (quad) *quad = sums[1];

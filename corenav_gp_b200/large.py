@@ -245,6 +245,55 @@ class LargeWindow:
                                                      var.data_ptr()), "cngp_large_predict_finish")
         return mean, var
 
+    # ---- the engine interface used by lml_grad_large_distributed ----
+    def grad_begin(self):
+        """RG = I for this rank's block columns.  RG (R, then G, like A), the two payload buffers and the parts are
+        allocated on first use and kept."""
+        self._bind()
+        if getattr(self, "RG", None) is None:
+            rg, pay, part = C.c_int64(), C.c_int64(), C.c_int64()
+            rc = self.lib.cngp_large_grad_sizes(C.byref(self.plan), C.byref(rg), C.byref(pay), C.byref(part))
+            if rc != 0:
+                raise CngpError(f"cngp_large_grad_sizes failed (rc={rc})")
+            f64 = dict(dtype=torch.float64, device=self.x.device)
+            self.RG = torch.empty(max(1, rg.value), **f64)
+            self.grad_payloads = [torch.empty(pay.value, **f64) for _ in range(2)]
+            self.part = torch.zeros(part.value, **f64)
+        self._chk(self.lib.cngp_large_grad_begin(self.ctx.h, C.byref(self.plan), self.RG.data_ptr()), "cngp_large_grad_begin")
+
+    def grad_payload(self, k: int):
+        """[W_k ; L(rows below the diagonal block, k)]: what the owner of k broadcasts (n_pad x NB doubles for every k)."""
+        return self.grad_payloads[k % 2]
+
+    def grad_panel(self, k: int):
+        self._bind()
+        self._chk(self.lib.cngp_large_grad_panel(self.ctx.h, C.byref(self.plan), self.A.data_ptr(), self.winv.data_ptr(),
+                                                 self.RG.data_ptr(), k, self.grad_payloads[k % 2].data_ptr()),
+                  "cngp_large_grad_panel")
+
+    def grad_update(self, k: int, c_lo: int, c_hi: int):
+        """This rank's block columns c in [c_lo, c_hi) with payload k: c > k swept, c <= k accumulated into G."""
+        self._bind()
+        self._chk(self.lib.cngp_large_grad_update(self.ctx.h, C.byref(self.plan), self.RG.data_ptr(), k,
+                                                  self.grad_payloads[k % 2].data_ptr(), c_lo, c_hi),
+                  "cngp_large_grad_update")
+
+    def grad_contract(self):
+        """-> part [n_blockcols * stride]: this rank's rows of the contraction, zero elsewhere."""
+        self._bind()
+        self._chk(self.lib.cngp_large_grad_contract(self.ctx.h, C.byref(self.plan), C.byref(self.kernel),
+                                                    self.theta.ctypes.data, self.x.data_ptr(), self.alpha.data_ptr(),
+                                                    self.RG.data_ptr(), self.part.data_ptr()), "cngp_large_grad_contract")
+        return self.part
+
+    def grad_finish(self):
+        """-> grad [P] from the rank-summed parts."""
+        self._bind()
+        grad = torch.empty(self.theta.size, dtype=torch.float64, device=self.x.device)
+        self._chk(self.lib.cngp_large_grad_finish(self.ctx.h, C.byref(self.plan), C.byref(self.kernel),
+                                                  self.part.data_ptr(), grad.data_ptr()), "cngp_large_grad_finish")
+        return grad
+
 
 class TorchCollectives:
     """broadcast / all-reduce through torch.distributed (NCCL for CUDA tensors, gloo for CPU tensors)."""
@@ -544,10 +593,54 @@ def predict_large_distributed(engine, xstar, rank: int, world: int, coll=None,
     return dict(mean=mean, var=var, pivot=0)
 
 
+def lml_grad_large_distributed(engine, rank: int, world: int, coll=None, lookahead: bool = True) -> Dict[str, object]:
+    """Gradient of the LML with respect to theta (natural parameters, noise last) from `engine`'s stored factor (SPMD:
+    every rank calls this after chol_large_distributed(engine, ..., want_alpha=True); any number of gradient and predict
+    passes may follow one factorisation).
+
+    The predict sweep with R = I: the owner of k forms W_k = (L^-T)(:, k) and broadcasts it with L(:, k); every rank
+    sweeps its block columns c > k and accumulates Ky^-1 = sum_k W_k W_k^T into its block columns c <= k; at the end each
+    rank contracts its block columns against dK/dtheta.  Returns dict(grad, pivot) - identical on every rank and on every
+    world size; if the factorisation found Ky not positive definite (pivot > 0), grad is NaN and the factor is not read."""
+    if coll is None:
+        coll = TorchCollectives() if world > 1 else NoCollectives()
+    pivot = getattr(engine, "pivot", None)
+    if pivot is None or not (pivot or getattr(engine, "have_alpha", False)):
+        raise CngpError("lml_grad_large_distributed: the window has not been factored with want_alpha=True")
+    if pivot:
+        nan = torch.full((int(np.size(engine.theta)),), float("nan"), dtype=torch.float64, device=engine.alpha.device)
+        return dict(grad=nan, pivot=pivot)
+    nblk = engine.n_blockcols
+    engine.grad_begin()
+    if rank == 0 % world:
+        engine.grad_panel(0)
+    pending = coll.broadcast_async(engine.grad_payload(0), src=0)
+    for k in range(nblk):
+        pending.wait()                                           # payload k is here
+        nxt = k + 1
+        if nxt < nblk:
+            if lookahead:
+                if nxt % world == rank:
+                    engine.grad_update(k, nxt, nxt + 1)
+                    engine.grad_panel(nxt)
+                pending = coll.broadcast_async(engine.grad_payload(nxt), src=nxt % world)   # overlaps the updates below
+                engine.grad_update(k, nxt + 1, nblk)
+            else:
+                engine.grad_update(k, nxt, nblk)
+                if nxt % world == rank:
+                    engine.grad_panel(nxt)
+                pending = coll.broadcast_async(engine.grad_payload(nxt), src=nxt % world)
+        engine.grad_update(k, 0, nxt)                            # G(:, c <= k) -= W_k W_k(c)^T
+    part = engine.grad_contract()
+    coll.all_reduce_sum(part)                                    # each row comes from one rank: x + 0, exact
+    return dict(grad=engine.grad_finish(), pivot=0)
+
+
 def chol_large(ctx: GpContext, kernel, theta, x, y, rank: int = 0, world: int = 1, coll=None, want_alpha: bool = True,
                lookahead: bool = True, chunk_rows: Optional[int] = None) -> Dict[str, object]:
     """Convenience: build this rank's LargeWindow and run the distributed factorisation.  The window is returned as
-    out["window"]: predict_large_distributed(out["window"], xstar, rank, world, coll) predicts from its factor."""
+    out["window"]: predict_large_distributed(out["window"], xstar, rank, world, coll) predicts from its factor, and
+    lml_grad_large_distributed(out["window"], rank, world, coll) gives the LML gradient from it."""
     win = LargeWindow(ctx, kernel, theta, x, y, rank=rank, world=world, chunk_rows=chunk_rows)
     out = chol_large_distributed(win, rank, world, coll=coll, want_alpha=want_alpha, lookahead=lookahead)
     out["window"] = win

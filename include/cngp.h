@@ -442,6 +442,44 @@ int cngp_chol_large_predict(cngp_ctx* ctx, const cngp_kernel* kernel, const doub
                             const double* y, int64_t N, const double* xstar, int64_t M, double* mean, double* var,
                             double* logdet, double* quad, double* lml, int32_t mem);
 
+/* ---- LML gradient on the large window from its stored factor ----
+ * The same definitions as cngp_lml_grad_batch (GPy ExactGaussianInference dL_dK + kern.update_gradients_full):
+ *   Ky = K + (noise + 1e-8) I,   dLML/dtheta_p = 1/2 sum_{i,j < N} (alpha_i alpha_j - (Ky^-1)_ij) dK_ij/dtheta_p,
+ *   noise (last entry): 1/2 (alpha' alpha - tr Ky^-1);  natural (not log) parameters, leaf parameters in program order.
+ * Like the predict pass it reads only A, winv and alpha, so any number of predict and gradient passes, in any order, can
+ * follow one factorisation.  With V = L^-T (upper triangular), Ky^-1 = V V^T = sum_k V_k V_k^T, and V is the predict
+ * sweep with R = I: W_k = V_k, non-zero in rows < NB (k+1) only.  RG stores R like A (n_pad/8 row tiles per column tile,
+ * block-cyclic); once block column k of R has given W_k it holds G(:, k) = -(Ky^-1)(:, k) (lower part) instead.
+ * Per block column k:
+ *   owner of k:  cngp_large_grad_panel    payload = [W_k (rows < NB (k+1)) ; L(rows > k, k)], n_pad x NB doubles for any k
+ *   all ranks:   broadcast of the payload (by the caller; nothing with one rank)
+ *   all ranks:   cngp_large_grad_update   its block columns c in [c_lo, c_hi): c > k  R(rows < NB (k+1), c) -= W_k L(c, k)^T
+ *                                                                           c <= k G(I, c) -= W_k(I) W_k(c)^T, c <= I <= k
+ * then cngp_large_grad_contract writes part[c][p] for this rank's block columns (zero elsewhere), the parts are summed
+ * over the ranks (each row comes from one rank, so the sum is exact) and cngp_large_grad_finish adds them in increasing c.
+ * Every R(:, c) and G(:, c) is written by one rank in increasing k: the same bits on every world size.  Device pointers
+ * except theta and the plan. */
+/* Buffer sizes in doubles: RG of this rank, one payload, part [n_blockcols][CNGP_MAX_PARAMS + 1]. */
+int cngp_large_grad_sizes(const cngp_large_plan* plan, int64_t* rg_doubles, int64_t* payload_doubles, int64_t* part_doubles);
+/* RG = I on this rank's block columns. */
+int cngp_large_grad_begin(cngp_ctx* ctx, const cngp_large_plan* plan, double* RG);
+int cngp_large_grad_panel(cngp_ctx* ctx, const cngp_large_plan* plan, const double* A, const double* winv, double* RG,
+                          int64_t k, double* payload);
+int cngp_large_grad_update(cngp_ctx* ctx, const cngp_large_plan* plan, double* RG, int64_t k, const double* payload,
+                           int64_t c_lo, int64_t c_hi);
+/* part[c][0 .. P) = sum over the entries i >= j of block column c of (alpha_i alpha_j - (Ky^-1)_ij) dK_ij/dtheta, the
+ * entries off the diagonal counted twice; alpha [n_pad] whole on every rank. */
+int cngp_large_grad_contract(cngp_ctx* ctx, const cngp_large_plan* plan, const cngp_kernel* kernel, const double* theta,
+                             const double* x, const double* alpha, const double* RG, double* part);
+/* grad [P] = 1/2 sum_c part[c] from the rank-summed part. */
+int cngp_large_grad_finish(cngp_ctx* ctx, const cngp_large_plan* plan, const cngp_kernel* kernel, const double* part,
+                           double* grad);
+/* The whole single-GPU sequence: cngp_chol_large's factorisation, then the gradient pass.  x, y, grad [P] follow `mem`;
+ * logdet/quad/lml are HOST scalars (may be NULL).  Returns CNGP_OK, or the failing pivot as in cngp_chol_large - then
+ * grad, logdet, quad and lml are NaN. */
+int cngp_chol_large_grad(cngp_ctx* ctx, const cngp_kernel* kernel, const double* theta, const double* x, const double* y,
+                         int64_t N, double* logdet, double* quad, double* lml, double* grad, int32_t mem);
+
 #ifdef __cplusplus
 }
 #endif

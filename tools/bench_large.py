@@ -10,7 +10,13 @@ Prints one JSON line: seconds per factorisation (CUDA events, max over ranks), F
     python tools/bench_large.py [N [reps [lookahead]]] --predict [M=600]
 
 adds the predict pass at M test points (the callback's horizon by default) from the same factor, timed apart from the
-factorisation: ms per pass, the update GEMM alone and its FP64 TFLOP/s, and the payload bytes each pass broadcasts."""
+factorisation: ms per pass, the update GEMM alone and its FP64 TFLOP/s, and the payload bytes each pass broadcasts.
+
+    python tools/bench_large.py [N [reps [lookahead]]] --grad
+
+times the LML gradient pass instead, alternated with the factorisation on the same GPU: ms per pass and per
+factorisation (best and median), the sweep GEMM and the SYRK launches alone with their FP64 TFLOP/s, the contraction,
+and the payload bytes per pass."""
 import json
 import os
 import sys
@@ -126,8 +132,70 @@ def run_predict(ctx, N, M, reps, rank, world, lookahead=True):
             "mean_finite": bool(torch.isfinite(mean).all())}
 
 
+def run_grad(ctx, N, reps, rank, world, lookahead=True):
+    """The LML gradient pass from the stored factor, alternated with the factorisation on the same GPU `reps` times
+    (after one untimed round of each), then the pass's sweep GEMM, its accumulation (SYRK) launches and the contraction
+    timed on their own; times are the max over ranks."""
+    if world > 1:
+        import torch.distributed as dist
+    kname = "rbf+stdperiodic"
+    th = np.array([0.01, 10.0, 0.0025, 37.0, 1.0, 1e-2])
+    x, y = syn.slip_windows(5, 1, N)
+    win = large.LargeWindow(ctx, kname, th, x[0], y[0], rank=rank, world=world)
+
+    def timed(fn):
+        torch.cuda.synchronize()
+        if world > 1:
+            dist.barrier()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        r = fn()
+        e1.record()
+        torch.cuda.synchronize()
+        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
+        if world > 1:
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        return float(t[0]), r
+
+    fac_ms, grad_ms, out, g = [], [], None, None
+    for it in range(reps + 1):
+        tf, out = timed(lambda: large.chol_large_distributed(win, rank, world, want_alpha=True, lookahead=lookahead))
+        tg, g = timed(lambda: large.lml_grad_large_distributed(win, rank, world, lookahead=lookahead))
+        if it > 0:
+            fac_ms.append(tf)
+            grad_ms.append(tg)
+    nblk = win.n_blockcols
+    # the pass's pieces on their own, on whatever RG and the payloads hold (their time does not depend on the values)
+    sweep, syrk, contract = [], [], []
+    for _ in range(reps):
+        sweep.append(timed(lambda: [win.grad_update(k, k + 1, nblk) for k in range(nblk)])[0])
+        syrk.append(timed(lambda: [win.grad_update(k, 0, k + 1) for k in range(nblk)])[0])
+        contract.append(timed(win.grad_contract)[0])
+    # executed flop (one rank's share is 1/world of it): sweep 2 x 256(k+1) x 256 x 256 per column c > k; SYRK one
+    # 128 x 128 x 256 block product per lower 128-block of the (k+1) x (k+1) block triangle
+    sweep_flop = sum(2.0 * 256 * (k + 1) * 256 * 256 * (nblk - k - 1) for k in range(nblk))
+    syrk_flop = sum(2.0 * 128 * 128 * 256 * (2 * (k + 1)) * (2 * (k + 1) + 1) / 2 for k in range(nblk))
+    payload_bytes = nblk * win.grad_payload(0).numel() * 8
+    best, fbest = min(grad_ms), min(fac_ms)
+    grad = g["grad"].cpu().numpy()
+    del win
+    return {"N": N, "n_gpus": world, "lookahead": lookahead, "kernel": kname, "theta": th.tolist(),
+            "grad_ms": grad_ms, "grad_best_ms": best, "grad_median_ms": float(np.median(grad_ms)),
+            "factor_ms_alternated": fac_ms, "factor_best_ms": fbest, "factor_median_ms": float(np.median(fac_ms)),
+            "grad_over_factor_best": best / fbest,
+            "grad_over_factor_median": float(np.median(grad_ms)) / float(np.median(fac_ms)),
+            "sweep_gemm_ms": sweep, "sweep_gemm_tflops": sweep_flop / world / (min(sweep) * 1e-3) * 1e-12,
+            "syrk_ms": syrk, "syrk_tflops": syrk_flop / world / (min(syrk) * 1e-3) * 1e-12,
+            "sweep_flop": sweep_flop, "syrk_flop": syrk_flop, "contract_ms": contract,
+            "payload_bytes_per_pass": payload_bytes, "lml": out["lml"], "grad": grad.tolist(),
+            "grad_finite": bool(np.all(np.isfinite(grad)))}
+
+
 def main():
     argv = list(sys.argv[1:])
+    grad = "--grad" in argv
+    if grad:
+        argv.remove("--grad")
     M = None
     if "--predict" in argv:
         i = argv.index("--predict")
@@ -146,6 +214,16 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device(f"cuda:{local}"))
     ctx = GpContext(device=local)
+    if grad:
+        line = run_grad(ctx, N, reps, rank, world, lookahead)
+        line["device"] = torch.cuda.get_device_properties(local).name
+        if rank == 0:
+            print(json.dumps(line))
+        if world > 1:
+            dist.barrier()
+            dist.destroy_process_group()
+        ctx.close()
+        return
     line = run(ctx, N, reps, rank, world, lookahead)
     if M is not None:
         line["predict"] = run_predict(ctx, N, M, reps, rank, world, lookahead)
